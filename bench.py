@@ -3,7 +3,7 @@
 (BASELINE.json config 4).  One JSON line on stdout; see DESIGN.md section "Measurement".
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows I --cols J --K K]
-                    [--workload sweep|cv|small|nmtf]
+                    [--workload sweep|cv|small|nmtf] [--dump-outputs DIR]
 
 A "step" is one Gibbs sweep plus one VB sweep (all U columns, all V columns, tau, train metrics each);
 value = sweeps per second over both.  N>1 (torchrun): rows of R / R^T are sharded across ranks
@@ -497,6 +497,50 @@ def checksum(models, engs):
     return out
 
 
+DUMP_BYTES = 64 * 10 ** 6        # 64 MB, decimal
+
+
+def dump_outputs(engs, steps, out_dir, rank):
+    """What the timed sweeps handed back, as run(steps) would give it to a caller, written to out_dir/<name>.npy (float64):
+    gibbs_U / gibbs_V, vb_{exp,var,mu,tau}{U,V} (the classes' attribute names) and <mode>_trace, one row per timed sweep
+    of tau, MSE, R^2, Rp (all_tau / all_exp_tau and all_performances).  The VB ELBO (all_elbo) is left out: from this
+    seeded random start it is -inf, as in the reference, while strongly truncated entries make log erfc underflow
+    (DESIGN.md section 5, parity; at the headline shape through at least the first 23 sweeps,
+    profiles/r04_dump_repeat.txt), so it holds nothing to compare.  Beyond DUMP_BYTES the factor arrays keep a fixed seeded
+    sample of their rows, the same rows for every array of a side; rows_U.npy / rows_V.npy then hold the row indices."""
+    import torch
+    if "vb" in engs:
+        engs["vb"].gather_params()          # mu / tau of the other ranks' rows (no-op on one GPU)
+    torch.cuda.synchronize()
+    if rank != 0:
+        return
+    sides = ([], [])                        # (name, device tensor [n, K]) per factor side
+    small = {}
+    for mode, e in engs.items():
+        for side, (f, s) in enumerate(((e.U, "U"), (e.V, "V"))):
+            fields = ((f.fac, "exp"), (f.var, "var"), (f.mu, "mu"), (f.tauf, "tau")) if e.vb else ((f.fac, ""),)
+            for t, attr in fields:
+                sides[side].append(("%s_%s%s" % (mode, attr, s), t[:f.n]))
+        last = e.sweeps_done - e.trace_base
+        small[mode + "_trace"] = e.trace[last - steps:last, :4].cpu().numpy()     # tau, MSE, R^2, Rp
+    n = [sides[i][0][1].shape[0] for i in (0, 1)]
+    row_bytes = [sum(t[0].numel() * 8 for _, t in sides[i]) for i in (0, 1)]
+    room = DUMP_BYTES - sum(a.nbytes for a in small.values()) - 4096
+    frac = min(1.0, room / float(sum(n[i] * (row_bytes[i] + 8) for i in (0, 1))))
+    out = dict(small)
+    for i, s in enumerate("UV"):
+        idx = None
+        if frac < 1.0:
+            idx = np.sort(np.random.RandomState(i).choice(n[i], int(n[i] * frac), replace=False))
+            out["rows_" + s] = idx.astype(np.float64)
+            idx = torch.from_numpy(idx).to(sides[i][0][1].device)
+        for name, t in sides[i]:
+            out[name] = (t if idx is None else t.index_select(0, idx)).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -511,7 +555,10 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--sustained-s", type=float, default=2.5)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state left by the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "sweep" or args.impl != "ours"):
+        ap.error("--dump-outputs needs --workload sweep --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.workload != "sweep":
@@ -584,6 +631,8 @@ def main():
     total_ms, g_ms, v_ms = (float(x) for x in times.cpu())
     value = 2.0 * args.steps / (total_ms / 1e3)
     state = checksum(models, engs)                     # after exactly warmup + steps sweeps, for every N
+    if args.dump_outputs:
+        dump_outputs(engs, args.steps, args.dump_outputs, rank)
 
     # ---- sustained figure: the same loop for >= sustained_s seconds (the board settles at its power cap) ----------
     sustained = None
