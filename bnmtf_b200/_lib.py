@@ -50,6 +50,9 @@ SIGNATURES = {
                            c_i, c_i, c_d, c_u64, c_p, c_u64, c_i64, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_p, c_p],
     "bnmtf_masked_metrics_f64": [c_p, c_p, c_i64, c_i64, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p],
     "bnmtf_mstat_reduce_f64": [c_p, c_i64, c_p, c_p, c_p],
+    "bnmtf_csr_stats_f64": [c_p, c_p, c_p, c_p, c_p, c_p, c_i64, c_i, c_p, c_p, c_i64, c_p, c_p, c_i, c_p, c_p, c_p, c_p, c_p,
+                            c_p, c_p],
+    "bnmtf_csr_metrics_f64": [c_p, c_p, c_p, c_i64, c_p, c_p, c_i, c_p, c_i, c_p, c_p, c_p],
     "bnmtf_metrics_from_sums_f64": [c_p, c_p, c_d, c_p, c_p, c_p],
     "bnmtf_select_metrics_f64": [c_p, c_p, c_p, c_p],
     "bnmtf_dense_metrics_f64": [c_p, c_p, c_p, c_i64, c_p, c_i, c_p, c_p],
@@ -87,7 +90,7 @@ KERNELS_PER_CALL = {"bnmtf_pack_dataset_f64": 1, "bnmtf_pack_mask_f64": 1, "bnmt
                     "bnmtf_pad_factor_f64": 1, "bnmtf_stats_rx_f64": 1, "bnmtf_stats_rx_umma_f64": 5,
                     "bnmtf_rx_planes_pack_f64": 2, "bnmtf_range_guard_f64": 1, "bnmtf_stats_gated_f64": 2, "bnmtf_stats_gram_f64": 1, "bnmtf_stats_gram_fixup_f64": 1, "bnmtf_kmeans_distances_f64": 1, "bnmtf_small_sweeps_f64": 1, "bnmtf_small_tri_sweeps_f64": 1, "bnmtf_stats_gram_umma_f64": 4, "bnmtf_mstat_reduce_f64": 2,
                     "bnmtf_metrics_from_sums_f64": 1, "bnmtf_select_metrics_f64": 1,
-                    "bnmtf_gram_full_f64": 2, "bnmf_row_solve_f64": 1, "bnmtf_masked_metrics_f64": 3,
+                    "bnmtf_gram_full_f64": 2, "bnmf_row_solve_f64": 1, "bnmtf_masked_metrics_f64": 3, "bnmtf_csr_stats_f64": 2, "bnmtf_csr_metrics_f64": 2,
                     "bnmtf_dense_metrics_f64": 2, "bnmtf_vb_factor_terms_f64": 1, "bnmtf_reduce8_f64": 1,
                     "bnmtf_reduce1_f64": 1, "bnmf_finish_sweep_f64": 1, "bnmtf_tn_moments_f64": 1, "bnmtf_np_build_pred_f64": 1,
                     "bnmtf_np_row_update_f64": 1, "bnmtf_np_s_update_f64": 2, "bnmtf_np_metrics_f64": 2,

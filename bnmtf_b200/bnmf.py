@@ -12,10 +12,12 @@ run(iterations) keeps the whole loop on the device (no host round trip per colum
 import math
 
 import numpy as np
+import scipy.sparse
 import torch
 
 from . import _lib
-from .engine import BNMFEngine, Dataset, S_BETA_S, S_ELBO, S_ESD, S_LOGTAU, S_TAU, _ptr, _stream, require_cuda
+from .data import validate_sparse
+from .engine import Dataset, SparseDataset, engine_for, S_BETA_S, S_ELBO, S_ESD, S_LOGTAU, S_TAU, _ptr, _stream, require_cuda
 
 def _elbo_alpha_s_correction(model):
     """The device evaluates the ELBO with alpha* = alpha + |Omega|/2, which is what update_tau() always yields.  The
@@ -141,18 +143,29 @@ class _TwoFactorBase(object):
     _mode = None
 
     def __init__(self, R, M, K, priors, device=None, seed=None, distributed=False):
-        self.R = np.array(R, dtype=float)
-        self.M = np.array(M, dtype=float)
-        self.K = K
+        self._sparse = scipy.sparse.issparse(R)
+        if self._sparse:
+            # sparse input: the stored entries of R are its known entries (explicit zeros included), M (or None: all of
+            # them) selects the training entries; self.R / self.M are canonical CSR matrices (data.validate_sparse)
+            if distributed:
+                raise ValueError("sparse R is not supported with distributed=True")
+            self.R, self.M, self._train = validate_sparse(R, M)
+            self.K = K
+            (self.I, self.J) = self.R.shape
+            self.size_Omega = float(self.M.nnz)
+        else:
+            self.R = np.array(R, dtype=float)
+            self.M = np.array(M, dtype=float)
+            self.K = K
 
-        assert len(self.R.shape) == 2, "Input matrix R is not a two-dimensional array, " \
-            "but instead %s-dimensional." % len(self.R.shape)
-        assert self.R.shape == self.M.shape, "Input matrix R is not of the same size as " \
-            "the indicator matrix M: %s and %s respectively." % (self.R.shape, self.M.shape)
+            assert len(self.R.shape) == 2, "Input matrix R is not a two-dimensional array, " \
+                "but instead %s-dimensional." % len(self.R.shape)
+            assert self.R.shape == self.M.shape, "Input matrix R is not of the same size as " \
+                "the indicator matrix M: %s and %s respectively." % (self.R.shape, self.M.shape)
 
-        (self.I, self.J) = self.R.shape
-        self.size_Omega = self.M.sum()
-        self.check_empty_rows_columns()
+            (self.I, self.J) = self.R.shape
+            self.size_Omega = self.M.sum()
+            self.check_empty_rows_columns()
 
         self.alpha, self.beta, self.lambdaU, self.lambdaV = \
             float(priors['alpha']), float(priors['beta']), np.array(priors['lambdaU']), np.array(priors['lambdaV'])
@@ -185,8 +198,7 @@ class _TwoFactorBase(object):
             self.lambdaV = self.lambdaV * np.ones((self.J, self.K))
         self._device_arg, self._seed, self.verbose = dataset.device, seed, False
         self._distributed = dataset.world > 1
-        self._eng = BNMFEngine(dataset, K, cls._mode, self.alpha, self.beta,
-                               seed=_shared_seed(seed, dataset.world > 1))
+        self._eng = engine_for(dataset, K, cls._mode, self.alpha, self.beta, seed=_shared_seed(seed, dataset.world > 1))
         return self
 
     def check_empty_rows_columns(self):
@@ -205,8 +217,11 @@ class _TwoFactorBase(object):
             if self._distributed:
                 import torch.distributed as dist
                 world, rank = dist.get_world_size(), dist.get_rank()
-            ds = Dataset.from_host(self.R, self.M, dev, world, rank)
-            self._eng = BNMFEngine(ds, self.K, self._mode, self.alpha, self.beta,
+            if self._sparse:
+                ds = SparseDataset(self.R, self._train, dev)
+            else:
+                ds = Dataset.from_host(self.R, self.M, dev, world, rank)
+            self._eng = engine_for(ds, self.K, self._mode, self.alpha, self.beta,
                                    seed=_shared_seed(self._seed, self._distributed))
         return self._eng
 

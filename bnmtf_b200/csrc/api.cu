@@ -46,6 +46,11 @@ int launch_stats_gram_umma(const uint32_t*, int, int, int, const double*, const 
 int launch_pad_factor(const double*, const double*, int, int, int, double*, double*, cudaStream_t);
 int launch_masked_metrics(const double*, const uint32_t*, int, int, const double*, const double*, int, int, const double*, double*, double*, const int*, cudaStream_t);
 int launch_mstat_reduce(const double*, int, double*, double*, cudaStream_t);
+int launch_csr_stats(const int64_t*, const int32_t*, const double*, const int64_t*, const int32_t*, const int32_t*, long long, int,
+                     const int32_t*, const int32_t*, long long, const double*, const double*, int, double*, double*, double*,
+                     double*, double*, double*, cudaStream_t);
+int launch_csr_metrics(const int64_t*, const int32_t*, const double*, long long, const double*, const double*, int, double*, int,
+                       double*, const int*, cudaStream_t);
 int launch_metrics_from_sums(const double*, const double*, double, double*, int*, cudaStream_t);
 int launch_select_metrics(const int*, const double*, double*, cudaStream_t);
 int launch_vb_factor_terms(const double*, const double*, const double*, const double*, const double*, long long, double*, int, cudaStream_t);
@@ -403,6 +408,22 @@ int bnmtf_masked_metrics_f64(const double* R, const uint32_t* bits, int64_t rows
                              const int* run_flag, void* stream) {
   if (check_k(K)) return -2;
   return launch_masked_metrics(R, bits, (int)rows, (int)ld, Ap, Bp, K, nseg, statics3, partials, out8, run_flag, ST(stream));
+}
+
+int bnmtf_csr_stats_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, const int64_t* item_begin,
+                        const int32_t* item_row, const int32_t* item_slot, int64_t n_items, int chunk, const int32_t* heavy_row,
+                        const int32_t* heavy_first, int64_t n_heavy, const double* Xp, const double* Vp, int K, double* RXpart,
+                        double* Gpart, double* SVpart, double* RXc, double* Gc, double* SVc, void* stream) {
+  if (check_k(K)) return -2;
+  if (Vp && !SVpart) { set_error("csr_stats: Vp given without SVpart"); return -2; }
+  return launch_csr_stats(rowptr, colidx, val, item_begin, item_row, item_slot, n_items, chunk, heavy_row, heavy_first, n_heavy,
+                          Xp, Vp, K, RXpart, Gpart, SVpart, RXc, Gc, SVc, ST(stream));
+}
+
+int bnmtf_csr_metrics_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t rows, const double* Ap,
+                          const double* Bp, int K, double* partials, int nparts, double* out8, const int* run_flag, void* stream) {
+  if (check_k(K)) return -2;
+  return launch_csr_metrics(rowptr, colidx, val, rows, Ap, Bp, K, partials, nparts, out8, run_flag, ST(stream));
 }
 
 int bnmtf_mstat_reduce_f64(const double* mstat, int64_t rows, double* partial, double* out4, void* stream) {

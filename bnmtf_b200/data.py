@@ -124,3 +124,95 @@ def upload(R, M, device=None, distributed=False):
         import torch.distributed as dist
         world, rank = dist.get_world_size(), dist.get_rank()
     return Dataset.from_host(np.array(R, dtype=float), np.array(M, dtype=float), dev, world, rank)
+
+
+# ---- sparse input ------------------------------------------------------------------------------------------------
+def _entries(A, name):
+    """(rows, cols, values) of every stored entry of a scipy.sparse matrix / array, explicit zeros and duplicates included."""
+    import scipy.sparse as sp
+    if not sp.issparse(A):
+        raise ValueError("%s must be a scipy.sparse matrix or array, not %s" % (name, type(A).__name__))
+    if A.ndim != 2:
+        raise ValueError("%s must be two-dimensional" % name)
+    C = A.tocoo()
+    return np.asarray(C.row, dtype=np.int64), np.asarray(C.col, dtype=np.int64), np.asarray(C.data, dtype=np.float64)
+
+
+def canonical_csr(R):
+    """The stored entries of a scipy.sparse R (any format) as a canonical CSR: float64 values, indices sorted within each
+    row, explicit zeros KEPT (a stored zero is a known entry).  Duplicate (i, j) entries raise ValueError: summing them
+    would change the data."""
+    import scipy.sparse as sp
+    if not sp.issparse(R):
+        raise ValueError("R must be a scipy.sparse matrix or array, not %s" % type(R).__name__)
+    I, J = R.shape
+    if R.format == "csr" and R.has_canonical_format:          # sorted and duplicate-free already: no sort needed
+        return sp.csr_matrix((np.array(R.data, dtype=np.float64), np.array(R.indices, dtype=np.int32),
+                              np.array(R.indptr, dtype=np.int64)), shape=(I, J))
+    rows, cols, vals = _entries(R, "R")
+    order = np.lexsort((cols, rows))
+    rows, cols, vals = rows[order], cols[order], vals[order]
+    if rows.size > 1:
+        dup = (rows[1:] == rows[:-1]) & (cols[1:] == cols[:-1])
+        if dup.any():
+            k = int(np.argmax(dup))
+            raise ValueError("R has more than one stored entry at (%d, %d)" % (rows[k], cols[k]))
+    indptr = np.concatenate([[0], np.cumsum(np.bincount(rows, minlength=I))]).astype(np.int64)
+    return sp.csr_matrix((vals, cols.astype(np.int32), indptr), shape=(I, J))
+
+
+def sparse_selection(Rc, M, name="M"):
+    """Boolean per stored entry of the canonical CSR Rc: True where the scipy.sparse M has a non-zero entry.  Every such
+    entry must be a stored entry of Rc (ValueError otherwise)."""
+    rows, cols, vals = _entries(M, name)
+    if tuple(M.shape) != tuple(Rc.shape):
+        raise ValueError("%s has shape %s, R has %s" % (name, tuple(M.shape), tuple(Rc.shape)))
+    nz = vals != 0
+    J = Rc.shape[1]
+    key = np.unique(rows[nz] * J + cols[nz])
+    rkey = np.repeat(np.arange(Rc.shape[0], dtype=np.int64), np.diff(Rc.indptr)) * J + Rc.indices.astype(np.int64)
+    pos = np.searchsorted(rkey, key)
+    inside = pos < rkey.size
+    inside[inside] = rkey[pos[inside]] == key[inside]
+    if not inside.all():
+        k = key[np.argmin(inside)]
+        raise ValueError("%s selects (%d, %d), which is not a stored entry of R" % (name, k // J, k % J))
+    sel = np.zeros(rkey.size, dtype=bool)
+    sel[pos] = True
+    return sel
+
+
+def validate_sparse(R, M=None):
+    """Host-side checks and canonical form of sparse input (no GPU call): -> (R as canonical CSR, M as CSR of ones on the
+    training entries, bool per stored entry of R: training or not).  M None: every stored entry of R is a training
+    entry.  Raises the reference's AssertionError texts for a shape mismatch and an unobserved row / column, ValueError
+    for duplicate entries in R and for an M entry outside R's pattern."""
+    import scipy.sparse as sp
+    if M is not None:
+        if not sp.issparse(M):
+            raise ValueError("with sparse R, M must be None or a scipy.sparse matrix, not %s" % type(M).__name__)
+        assert tuple(R.shape) == tuple(M.shape), "Input matrix R is not of the same size as " \
+            "the indicator matrix M: %s and %s respectively." % (tuple(R.shape), tuple(M.shape))
+    Rc = canonical_csr(R)
+    I, J = Rc.shape
+    train = np.ones(Rc.nnz, dtype=bool) if M is None else sparse_selection(Rc, M)
+    rows = np.repeat(np.arange(I, dtype=np.int64), np.diff(Rc.indptr))
+    sums_rows = np.bincount(rows[train], minlength=I)
+    sums_columns = np.bincount(Rc.indices[train], minlength=J)
+    for i, c in enumerate(sums_rows):
+        assert c != 0, "Fully unobserved row in R, row %s." % i
+    for j, c in enumerate(sums_columns):
+        assert c != 0, "Fully unobserved column in R, column %s." % j
+    indptr = np.concatenate([[0], np.cumsum(sums_rows)]).astype(np.int64)
+    Mc = sp.csr_matrix((np.ones(int(train.sum())), Rc.indices[train], indptr), shape=(I, J))
+    return Rc, Mc, train
+
+
+def upload_sparse(R, M=None, device=None):
+    """Sparse (R, M) -> engine.SparseDataset on `device` (default: the current CUDA device): the training entries in
+    CSR form for the row phase and for the column phase, with the static work plan of the statistics kernel.  R and M
+    as the model constructors take them (validate_sparse).  The result can be passed to `Model.from_dataset(ds, K,
+    priors)` of the two-factor models so that several models share one resident copy of the matrix."""
+    from .engine import SparseDataset, require_cuda
+    Rc, _, train = validate_sparse(R, M)
+    return SparseDataset(Rc, train, require_cuda(device))

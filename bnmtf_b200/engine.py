@@ -896,3 +896,219 @@ class BNMFEngine:
         if getattr(self, "trace_win", None) is None:
             self.trace_win = torch.zeros(2, dtype=torch.int64, device=self.ds.device)
         self.trace_win.copy_(torch.tensor([self.trace_base, self.trace_base + self.trace_cap], dtype=torch.int64))
+
+
+# ==== sparse input: the observed entries only, in CSR form (csrc/sparse.cu) ==========================================
+CSR_CHUNK = 1024        # entries per work item of the CSR statistics kernel: longer rows are split, their chunks added in order
+CSR_METRIC_CTAS = 1184  # CTAs (partial results) of bnmtf_csr_metrics_f64: 8 per SM
+
+
+def csr_work_plan(indptr, chunk=CSR_CHUNK):
+    """Static work plan of bnmtf_csr_stats_f64 for the row pointers `indptr` (include/bnmtf_b200.h): every row becomes
+    ceil(n_i / chunk) items (one for an empty row); the items of a row with more than one get consecutive chunk slots.
+    -> dict of numpy arrays item_begin (int64), item_row, item_slot, heavy_row, heavy_first (int32) and n_slots."""
+    indptr = np.asarray(indptr, dtype=np.int64)
+    rows = indptr.shape[0] - 1
+    lens = np.diff(indptr)
+    nch = np.maximum(1, -(-lens // chunk))
+    item_row = np.repeat(np.arange(rows, dtype=np.int64), nch)
+    first = np.cumsum(nch) - nch
+    c = np.arange(item_row.shape[0], dtype=np.int64) - np.repeat(first, nch)
+    heavy = nch > 1
+    item_slot = np.full(item_row.shape[0], -1, dtype=np.int64)
+    in_heavy = heavy[item_row]
+    item_slot[in_heavy] = np.arange(int(in_heavy.sum()), dtype=np.int64)
+    heavy_first = np.concatenate([[0], np.cumsum(nch[heavy])]).astype(np.int32)
+    return {"item_begin": indptr[item_row] + c * chunk, "item_row": item_row.astype(np.int32),
+            "item_slot": item_slot.astype(np.int32), "heavy_row": np.nonzero(heavy)[0].astype(np.int32),
+            "heavy_first": heavy_first, "n_slots": int(heavy_first[-1]), "chunk": int(chunk)}
+
+
+class DeviceCSR:
+    """One CSR orientation on the device: int64 row pointers, int32 column indices, fp64 values, and the static work
+    plan of the statistics kernel."""
+
+    def __init__(self, indptr, indices, data, device, plan=True):
+        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(device)
+        self.rows = int(len(indptr) - 1)
+        self.nnz = int(indptr[-1])
+        self.rowptr, self.colidx, self.val = t(indptr, np.int64), t(indices, np.int32), t(data, np.float64)
+        if self.nnz == 0:           # (a valid pointer for the kernels, never read)
+            self.colidx, self.val = torch.zeros(1, dtype=torch.int32, device=device), torch.zeros(1, dtype=torch.float64, device=device)
+        self.plan = None
+        if plan:
+            p = csr_work_plan(indptr)
+            self.chunk, self.n_items, self.n_slots = p["chunk"], int(p["item_row"].shape[0]), p["n_slots"]
+            self.n_heavy = int(p["heavy_row"].shape[0])
+            self.item_begin, self.item_row, self.item_slot = t(p["item_begin"], np.int64), t(p["item_row"], np.int32), t(p["item_slot"], np.int32)
+            self.heavy_row = t(p["heavy_row"], np.int32) if self.n_heavy else None
+            self.heavy_first = t(p["heavy_first"], np.int32)
+            self.plan = p
+
+    def nbytes(self):
+        ts = [self.rowptr, self.colidx, self.val] + ([self.item_begin, self.item_row, self.item_slot, self.heavy_first]
+                                                     + ([self.heavy_row] if self.n_heavy else []) if self.plan else [])
+        return sum(x.numel() * x.element_size() for x in ts)
+
+    def metrics(self, Ap, Bp, K, partials, out8, run_flag=None):
+        """bnmtf_csr_metrics_f64 over these entries -> out8."""
+        nparts = max(1, min(CSR_METRIC_CTAS, -(-self.rows // 8)))
+        _lib.call("bnmtf_csr_metrics_f64", _ptr(self.rowptr), _ptr(self.colidx), _ptr(self.val), self.rows, _ptr(Ap), _ptr(Bp),
+                  int(K), _ptr(partials), nparts, _ptr(out8), _ptr(run_flag), _stream())
+
+
+class SparseDataset:
+    """The training entries of R on the device, in both orientations: CSR of R for the row phase and CSR of R^T (i.e. the
+    CSC of R) for the column phase.  No I x J array exists at any point.  `host_R` keeps the canonical host CSR of every
+    stored entry of R (training or not), which predict(M_pred) evaluates on.  Single GPU only."""
+    world, rank = 1, 0
+    bits = None                 # the training entries (the dense engine's `bits` argument: None selects csr[0])
+
+    def __init__(self, host_R, train, device):
+        """host_R: canonical scipy.sparse CSR (sorted indices, no duplicates); train: bool per stored entry, or None (all)."""
+        import scipy.sparse as sp
+        self.I, self.J = host_R.shape
+        self.device = device
+        self.partI, self.partJ = Partition(self.I), Partition(self.J)
+        self.host_R = host_R
+        if train is None or bool(np.all(train)):
+            Rt = host_R
+        else:
+            rows = np.repeat(np.arange(self.I, dtype=np.int64), np.diff(host_R.indptr))[train]
+            indptr = np.concatenate([[0], np.cumsum(np.bincount(rows, minlength=self.I))]).astype(np.int64)
+            Rt = sp.csr_matrix((host_R.data[train], host_R.indices[train], indptr), shape=host_R.shape)
+        RtT = Rt.tocsc()            # scipy's counting sort: column-major with sorted row indices, explicit zeros kept
+        self.csr = {0: DeviceCSR(Rt.indptr, Rt.indices, Rt.data, device),
+                    1: DeviceCSR(RtT.indptr, RtT.indices, RtT.data, device)}
+        self.n_obs = float(Rt.indptr[-1])
+        # static sums {sum r, sum r^2, |Omega|} of the training entries: the metric kernel with a zero prediction
+        zeros = torch.zeros((max(self.I, self.J) + 8) * 8, dtype=torch.float64, device=device)
+        part = torch.zeros(CSR_METRIC_CTAS * 8, dtype=torch.float64, device=device)
+        out = torch.zeros(8, dtype=torch.float64, device=device)
+        self.csr[0].metrics(zeros, zeros, 1, part, out)
+        self.statics = out[4:7].clone()
+
+    def nbytes(self):
+        return self.csr[0].nbytes() + self.csr[1].nbytes()
+
+    def pack_mask(self, M_pred):
+        """The entries of R on the pattern of M_pred (which must lie inside R's stored entries) as a DeviceCSR, the
+        entry set bnmtf_csr_metrics_f64 evaluates predict(M_pred) on."""
+        from .data import sparse_selection
+        sel = sparse_selection(self.host_R, M_pred, "M_pred")
+        R = self.host_R
+        rows = np.repeat(np.arange(self.I, dtype=np.int64), np.diff(R.indptr))[sel]
+        indptr = np.concatenate([[0], np.cumsum(np.bincount(rows, minlength=self.I))]).astype(np.int64)
+        return DeviceCSR(indptr, R.indices[sel], R.data[sel], self.device, plan=False)
+
+
+class SparseBNMFEngine(BNMFEngine):
+    """BNMFEngine on a SparseDataset.  The format decision lives here: the statistics of a phase come from one
+    bnmtf_csr_stats_f64 call over the phase's CSR (fp64, polarity 1, one segment: no digit planes, no range guard, no
+    unmasked totals), the sweep's metrics from the column-phase statistics with bnmtf_csr_metrics_f64 as the gated direct
+    pass.  Everything else -- solver calls, factor handling, the end of the sweep, CUDA-graph replay -- is BNMFEngine's."""
+
+    def __init__(self, dataset, K, mode, alpha, beta, seed=0, comm=None):
+        if dataset.world != 1:
+            raise ValueError("sparse input runs on one GPU")
+        self.ds, self.K, self.mode = dataset, int(K), mode
+        self.gram = self.rx = "csr"
+        self.metrics_mode = "stats"
+        self.guard = 1e-5
+        self.polarity = 1
+        self.range_guard = False
+        self.split = self.overlap = 0
+        self.use_graph = int(os.environ.get("BNMTF_GRAPH", "1")) >= 1
+        self._graph = self._graph_key = self._graph_seen = None
+        self._small_c = 0               # never the single-kernel small path
+        self.m, self.vb = MODE[mode], mode == "vb"
+        self.alpha, self.beta, self.seed = float(alpha), float(beta), int(seed) & (2 ** 64 - 1)
+        self.comm = comm if comm is not None else Comm(1, 0)
+        dev = dataset.device
+        self.U = Factor(dataset.partI, K, dev, self.vb, self.comm)
+        self.V = Factor(dataset.partJ, K, dev, self.vb, self.comm)
+        self.scalars = torch.zeros(16, dtype=torch.float64, device=dev)
+        self.iter = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.iter_scratch = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.trace, self.trace_cap, self.trace_base, self.sweeps_done = None, 0, 0, 0
+        KP, GL = kp_for(K), gram_len(K)
+        self.loc = {0: (0, dataset.I), 1: (0, dataset.J)}
+        self.nseg = {0: (1, 1, 1), 1: (1, 1, 1)}
+        self.range_flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        rmax = max(dataset.I, dataset.J)
+        smax = max(1, dataset.csr[0].n_slots, dataset.csr[1].n_slots)
+        f64 = lambda *shape: torch.zeros(shape, dtype=torch.float64, device=dev)
+        self.RXpart, self.Gpart = f64(rmax, KP), f64(rmax, GL)
+        self.SVpart = f64(rmax, KP) if self.vb else None
+        self.RXc, self.Gc = f64(smax, KP), f64(smax, GL)          # chunk partials of the heavy rows
+        self.SVc = f64(smax, KP) if self.vb else None
+        self.Gfull = f64(GL + KP)                                    # (read by the solver only at polarity 0)
+        self.extra = f64(rmax) if self.vb else None
+        self.red = f64(24)
+        self.m8, self.el8, self.ex1, self.sums4 = self.red[0:8], self.red[8:16], self.red[16:17], self.red[17:21]
+        self.mpart = f64(CSR_METRIC_CTAS * 8)
+        self.nb_terms = 64 if rmax * self.K <= (1 << 17) else 296
+        self.elpart = f64(2 * self.nb_terms * 8) if self.vb else None
+        self.sterm = self.order_dev = None
+        self.statics = dataset.statics.clone()
+        self.statics_global = self.statics
+        self.mstat, self.mstat_part, self.m8d = f64(rmax, 4), f64(256), f64(8)
+        self.flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        self._set_omega(dataset.n_obs)
+
+    def _sides(self, side):
+        lo, cnt = self.loc[side]
+        me, other = (self.U, self.V) if side == 0 else (self.V, self.U)
+        return me, other, self.ds.csr[side], None, cnt, None, lo
+
+    def stats(self, side, need_rx=True, sums=False, timers=None):
+        """RXpart / Gpart / SVpart of one phase from its CSR (the column sums the statistics-based metrics need are in the
+        Gram record whatever `sums` says)."""
+        me, other, c, _, rows, _, lo = self._sides(side)
+        other.pad()
+        _lib.call("bnmtf_csr_stats_f64", _ptr(c.rowptr), _ptr(c.colidx), _ptr(c.val), _ptr(c.item_begin), _ptr(c.item_row),
+                  _ptr(c.item_slot), c.n_items, c.chunk, _ptr(c.heavy_row), _ptr(c.heavy_first), c.n_heavy, _ptr(other.Xp),
+                  _ptr(other.Vp), self.K, _ptr(self.RXpart) if need_rx else 0, _ptr(self.Gpart), _ptr(self.SVpart),
+                  _ptr(self.RXc), _ptr(self.Gc), _ptr(self.SVc), _stream())
+
+    def _metrics_padded(self, bits, gated=False):
+        """The seven sums over the entry set `bits` (None: the training entries; else a DeviceCSR from pack_mask)."""
+        entries = self.ds.csr[0] if bits is None else bits
+        entries.metrics(self.U.Xp, self.V.Xp, self.K, self.mpart, self.m8d if gated else self.m8,
+                        self.flag if gated else None)
+
+    def small_cluster(self):
+        return 0
+
+    def profile_sweep(self, reps=3):
+        """CUDA-event timings (ms per call, mean over reps and over the two phases) of the CSR statistics call and the
+        solver.  Runs real sweeps (the state advances; the trace is not written)."""
+        acc = {"stats_csr_row": 0.0, "stats_csr_col": 0.0, "row_solve": 0.0}
+        for _ in range(reps):
+            for side in (0, 1):
+                e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+                e[0].record()
+                self.stats(side, sums=side == 1)
+                e[1].record()
+                self.solve(side, want_extra=self.vb and side == 1, want_mstat=side == 1)
+                e[2].record()
+                e[2].synchronize()
+                acc["stats_csr_row" if side == 0 else "stats_csr_col"] += e[0].elapsed_time(e[1]) / reps
+                acc["row_solve"] += e[1].elapsed_time(e[2]) / (2 * reps)
+            self.V.pad()
+            _lib.call("bnmtf_mstat_reduce_f64", _ptr(self.mstat), self.loc[1][1], _ptr(self.mstat_part), _ptr(self.sums4), _stream())
+            if self.vb:
+                self._vb_extra()
+                self._vb_terms()
+            _lib.call("bnmtf_metrics_from_sums_f64", _ptr(self.sums4), _ptr(self.statics_global), self.guard,
+                      _ptr(self.m8), _ptr(self.flag), _stream())
+            self.finish(update_tau=True, record=False)
+        acc["stats_csr"] = 0.5 * (acc["stats_csr_row"] + acc["stats_csr_col"])
+        acc["_meta"] = {"gram": self.gram, "rx": self.rx, "metrics_mode": self.metrics_mode}
+        return acc
+
+
+def engine_for(dataset, K, mode, alpha, beta, seed=0):
+    """The engine that runs on `dataset`: SparseBNMFEngine for a SparseDataset, BNMFEngine otherwise."""
+    cls = SparseBNMFEngine if isinstance(dataset, SparseDataset) else BNMFEngine
+    return cls(dataset, K, mode, alpha, beta, seed=seed)

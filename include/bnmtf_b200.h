@@ -223,6 +223,28 @@ int bnmf_row_solve_f64(int mode, int64_t rows, int K, int nseg_rx, int nseg_g, i
 int bnmtf_masked_metrics_f64(const double* R, const uint32_t* bits, int64_t rows, int64_t ld, const double* Ap,
                              const double* Bp, int K, int nseg, const double* statics3, double* partials, double* out8,
                              const int* run_flag, void* stream);
+/* ---- sparse input: statistics and metric sums over the stored entries of a CSR matrix (csrc/sparse.cu) ----------
+ * CSR: rowptr (rows + 1 int64), colidx (int32, sorted within a row), val (double); the columns index the rows of the
+ * padded factor images.  No dense rows x cols array is read or written.
+ * bnmtf_csr_stats_f64 writes RXpart (rows x KP, or NULL to skip), Gpart (rows x NTP*64) and SVpart (rows x KP, VB: Vp !=
+ * NULL) with the layout and slots of bnmtf_stats_rx_f64 / bnmtf_stats_gram_f64 at polarity 1 and nseg 1, i.e. sums over
+ * the row's stored entries of r Xp_j, Xp_j Xp_j^T and Vp_j (the ones column of Xp puts the column sums in slot (k, K) and
+ * the count in (K, K)), all in fp64.  Work plan (static, built once per matrix): n_items items; item t covers the entries
+ * [item_begin[t], min(item_begin[t] + chunk, rowptr[row + 1])) of row item_row[t]; item_slot[t] = -1 writes the row's
+ * record directly (a row with one item), s >= 0 writes chunk partial s of RXc / Gc / SVc (same record layouts).  Heavy row
+ * h = heavy_row[h] owns the consecutive slots [heavy_first[h], heavy_first[h + 1]) in chunk order, and its record is
+ * their sum in that order.  Deterministic: no floating-point atomics. */
+int bnmtf_csr_stats_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, const int64_t* item_begin,
+                        const int32_t* item_row, const int32_t* item_slot, int64_t n_items, int chunk, const int32_t* heavy_row,
+                        const int32_t* heavy_first, int64_t n_heavy, const double* Xp, const double* Vp /*or NULL*/, int K,
+                        double* RXpart /*or NULL*/, double* Gpart, double* SVpart /*or NULL*/, double* RXc, double* Gc,
+                        double* SVc, void* stream);
+/* The seven sums of bnmtf_masked_metrics_f64 {e^2, p, p^2, r p, r, r^2, n} (out8[7] = 0) over the stored entries of a CSR,
+ * p = Ap_i . Bp_j over k < K (Ap: the row factor's padded image, offset to row 0 of this CSR).  partials: nparts x 8
+ * doubles of scratch (nparts CTAs; any count >= 1).  run_flag as in bnmtf_masked_metrics_f64. */
+int bnmtf_csr_metrics_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t rows, const double* Ap,
+                          const double* Bp, int K, double* partials, int nparts, double* out8, const int* run_flag,
+                          void* stream);
 /* Training metrics of a sweep from the statistics of its last phase instead of a third pass over R
  * (predict_while_running, bnmf_gibbs_optimised.py:199-223): mstat (rows x 4, bnmf_row_solve_f64) -> out4 = this
  * shard's {sum r p, sum p^2, sum p, 0}; partial: >= 256 doubles of scratch. */
