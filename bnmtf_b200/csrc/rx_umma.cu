@@ -10,14 +10,17 @@
 //       missing entries -- the mask is folded into the data.  Layout: [row block of 128][column tile of 64][plane]
 //       [128 rows x 64 B], each 8 KB plane tile already in the K-major 64-byte-swizzled order tcgen05 reads, so one
 //       stage of the A operand is ONE contiguous 56 KB bulk copy from HBM.
-//   X (per call): p_jk = llrint(X_jk 2^(56-f_k)) >= 0, digit t of column k is row t*KPAD + k of the B operand
-//       (rebuilt by a pre-pass every phase, 7 MB, L2 resident, TMA tiled loads).
+//   X (per call): p_jk = llrint(X_jk 2^(56-f_k)) >= 0, digit t of column k is row (6-t)*KS + k of the B operand, KS =
+//       K rounded up to a multiple of 4 (rebuilt by a pre-pass every phase, <= 7 MB, L2 resident, TMA tiled loads).
+//       The digits run from the top one down, so every plane's digit range t = tmin(s)..6 starts at row 0 of the
+//       staged tile: no MMA operand starts inside a swizzle atom, whatever KS is.
 //   sum_j q_ij p_jk = sum_{s,t} 256^(s+t) sum_j a_s(i,j) b_t(j,k): the MMA of plane s against digits t >= tmin(s) with
-//       its accumulator base shifted by s*KPAD columns lands every product of equal weight s+t = u in the same int32
-//       accumulator D_u -- one MMA per plane and k-step.  Pairs with s+t < 5 (below 2^-59 of the product scale) are
-//       dropped, leaving 8 accumulators = 8*KPAD tensor-memory columns, double buffered: a set is drained (tcgen05.ld,
-//       Horner in fp64, tcgen05.st zeros) every 4096 columns -- before 7 * 255^2 * 4096 < 2^31 can overflow -- while
-//       the MMAs continue into the other set.
+//       its accumulator base at column (6-s)*KS lands every product of equal weight s+t = u in the same int32
+//       accumulator D_u (column (12-u)*KS, highest weight first) -- one MMA per plane and k-step.  Pairs with s+t < 5
+//       (below 2^-59 of the product scale) are dropped, leaving 8 accumulators = 8*KS tensor-memory columns (+ scratch
+//       columns, rxu_set_cols), double buffered: a set is drained (tcgen05.ld, Horner in fp64, tcgen05.st
+//       zeros) every 4096 columns -- before 7 * 255^2 * 4096 < 2^31 can overflow -- while the MMAs continue into the
+//       other set.
 //
 // Factors with negative or non-finite entries (impossible for the models' own updates, possible through the white-box
 // API) raise a device flag in the pre-pass: this kernel then returns at once and the gated DMMA kernel does the work.
@@ -37,16 +40,32 @@ constexpr int RXU_UMIN = 2 * kDigits - 9;         // 7 digits: 5 (u = 5..12);  6
 constexpr int RXU_NU = RXU_PLANES + RXU_VDIG - 1 - RXU_UMIN;   // 8 accumulators
 constexpr int RXU_RBITS = 8 * RXU_PLANES - 1;     // R: signed, |q| < 2^RBITS
 constexpr int RXU_XBITS = 8 * RXU_VDIG;           // X: unsigned, q < 2^XBITS
-static_assert(2 * RXU_NU * 32 <= 512, "two accumulator sets must fit tensor memory");
 constexpr int RXU_KT = 64;                        // bytes (= columns) per pipeline stage
 constexpr int RXU_DRAIN = 64;                     // stages per accumulator period: 4096 columns
 constexpr int RXU_PLANE_TILE = 128 * RXU_KT;      // 8 KB
 constexpr int RXU_A_BYTES = RXU_PLANES * RXU_PLANE_TILE;
 constexpr int RXU_THREADS = 192;
-// Factor columns are padded to KPAD = 16, 24 or 32.  UMMA N must be a multiple of 16 at M = 128: with KPAD = 24 the MMAs of
-// an odd number of digits run 8 columns wide of their range, into digit rows past the last digit -- rows that exist in
-// the staged B operand and are zero (rxu_brows), so the extra columns add nothing.
-__host__ __device__ constexpr int rxu_brows(int kpad) { return (RXU_VDIG * kpad + (kpad % 16 ? 8 : 0) + 15) / 16 * 16; }
+// Digit blocks of the factor are KS = K rounded up to 4 rows apart.  UMMA N must be a multiple of 16 at M = 128, so the
+// MMA of plane s runs up to 12 columns past its nt*KS: into the B rows after its lowest digit and the tensor-memory
+// columns after its lowest-weight accumulator.  Below digit 0 the B rows exist and are zero (rxu_brows), so those
+// columns add nothing.  Below digit tmin > 0 they hold digit tmin - 1 -- dropped pairs of weight UMIN - 1 -- and land in
+// scratch columns past the 8 accumulators of the set (rxu_set_cols), which the drain zeroes and never reads.
+__host__ __device__ constexpr int rxu_r16(int n) { return (n + 15) / 16 * 16; }
+__host__ __device__ constexpr int rxu_tmin(int p) { return p < RXU_UMIN ? RXU_UMIN - p : 0; }
+__host__ __device__ constexpr int rxu_n(int p, int ks) { return rxu_r16((RXU_VDIG - rxu_tmin(p)) * ks); }   // UMMA N of plane p
+__host__ __device__ constexpr int rxu_brows(int ks) { return rxu_r16(RXU_VDIG * ks); }
+// tensor-memory columns of one accumulator set: plane p writes columns (PLANES-1-p)*KS ... + rxu_n(p)
+__host__ __device__ constexpr int rxu_set_cols(int ks) {
+  int m = 0;
+  for (int p = 0; p < RXU_PLANES; ++p) m = (RXU_PLANES - 1 - p) * ks + rxu_n(p, ks) > m ? (RXU_PLANES - 1 - p) * ks + rxu_n(p, ks) : m;
+  return rxu_r16(m);
+}
+constexpr bool rxu_sets_fit() {
+  for (int ks = 4; ks <= 32; ks += 4)
+    if (2 * rxu_set_cols(ks) > 512 || rxu_brows(ks) > 256) return false;
+  return true;
+}
+static_assert(rxu_sets_fit(), "two accumulator sets must fit tensor memory, the digit rows one TMA box");
 
 __host__ __device__ inline size_t rxu_tile_offset(int rb, int kt, int ktiles) {
   return ((size_t)rb * ktiles + kt) * RXU_A_BYTES;
@@ -186,14 +205,14 @@ __global__ void k_rxu_colscale(const unsigned long long* __restrict__ colmax, in
   cscale[k] = scalbn(1.0, e - RXU_XBITS);
 }
 
-// Bd[t*KPAD + k][j] = byte t of llrint(X_jk 2^(56-e_k)); zero for j >= n and for k >= K.  thread <-> (k, 4 columns)
-__global__ void __launch_bounds__(256) k_rxu_quantize(const double* __restrict__ Xp, int n, int K, int KP, int KPAD,
+// Bd[(VDIG-1-t)*KS + k][j] = byte t of llrint(X_jk 2^(56-e_k)); zero for j >= n and for k >= K.  thread <-> (k, 4 columns)
+__global__ void __launch_bounds__(256) k_rxu_quantize(const double* __restrict__ Xp, int n, int K, int KP, int KS,
                                                      long long ldb, const int* __restrict__ cexp, const int* __restrict__ flag,
                                                      uint8_t* __restrict__ Bd) {
   if (*flag) return;
   const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long groups = ldb >> 2;
-  if (gid >= groups * KPAD) return;
+  if (gid >= groups * KS) return;
   const int k = (int)(gid / groups);                  // column group fastest: coalesced 128-byte digit stores per warp
   const long long jg = (gid - (long long)k * groups) * 4;
   uint32_t w[RXU_VDIG];
@@ -212,7 +231,7 @@ __global__ void __launch_bounds__(256) k_rxu_quantize(const double* __restrict__
     }
   }
 #pragma unroll
-  for (int t = 0; t < RXU_VDIG; ++t) *reinterpret_cast<uint32_t*>(Bd + (size_t)(t * KPAD + k) * ldb + jg) = w[t];
+  for (int t = 0; t < RXU_VDIG; ++t) *reinterpret_cast<uint32_t*>(Bd + (size_t)((RXU_VDIG - 1 - t) * KS + k) * ldb + jg) = w[t];
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -220,6 +239,13 @@ __global__ void __launch_bounds__(256) k_rxu_quantize(const double* __restrict__
 // ---------------------------------------------------------------------------------------------------
 template <int N>
 __device__ __forceinline__ void tmem_ld_n(uint32_t addr, uint32_t (&r)[N]);
+template <>
+__device__ __forceinline__ void tmem_ld_n<4>(uint32_t addr, uint32_t (&r)[4]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(addr)
+               : "memory");
+}
 template <>
 __device__ __forceinline__ void tmem_ld_n<8>(uint32_t addr, uint32_t (&r)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
@@ -256,22 +282,40 @@ __device__ __forceinline__ void tmem_st_zero16(uint32_t addr) {
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+// Horner over the NU accumulators of one set (highest weight first) for factor columns k0 .. k0+W-1, added to c
+template <int W, int KS>
+__device__ __forceinline__ void rxu_drain_cols(uint32_t set_addr, int k0, double (&c)[KS]) {
+  double v[W];
+#pragma unroll
+  for (int k = 0; k < W; ++k) v[k] = 0.0;
+#pragma unroll
+  for (int a = 0; a < RXU_NU; ++a) {
+    uint32_t reg[W];
+    tmem_ld_n<W>(set_addr + (uint32_t)(a * KS + k0), reg);
+    tmem_ld_wait();
+#pragma unroll
+    for (int k = 0; k < W; ++k) v[k] = fma(v[k], 256.0, (double)(int)reg[k]);
+  }
+#pragma unroll
+  for (int k = 0; k < W; ++k) c[k0 + k] += v[k];
+}
+
 struct RxUmmaArgs {
   const uint8_t* planes; const double* rscale; const double* cscale; const int* flag;
   int rows, K, KP, ktiles, tiles_per_seg, stages, nseg;
   double* out;
 };
 
-template <int KPAD>
+template <int KS>
 __global__ void __launch_bounds__(RXU_THREADS, 1) k_rx_umma(const __grid_constant__ CUtensorMap tmap, RxUmmaArgs a) {
   if (*a.flag) return;                                  // negative / non-finite factor: the gated DMMA kernel runs instead
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  constexpr int B_BYTES = rxu_brows(KPAD) * RXU_KT;
+  constexpr int B_BYTES = rxu_brows(KS) * RXU_KT;
   static_assert(B_BYTES % 1024 == 0, "stages stay 1024-byte aligned");
   constexpr int STAGE = RXU_A_BYTES + B_BYTES;
-  constexpr int SET = RXU_NU * KPAD;                    // tensor-memory columns of one accumulator set
+  constexpr int SET = rxu_set_cols(KS);                 // tensor-memory columns of one accumulator set
   const int stages = a.stages;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)stages * STAGE);   // full[st], empty[st], acc_full[2], acc_empty[2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * stages + 4);
@@ -320,30 +364,19 @@ __global__ void __launch_bounds__(RXU_THREADS, 1) k_rx_umma(const __grid_constan
       const int ntile = min(a.ktiles, kt_begin + a.tiles_per_seg) - kt_begin;
       const int nper = (ntile + RXU_DRAIN - 1) / RXU_DRAIN;
       const int row = rb * 128 + tid;
-      double c[KPAD];
+      double c[KS];
 #pragma unroll
-      for (int k = 0; k < KPAD; ++k) c[k] = 0.0;
+      for (int k = 0; k < KS; ++k) c[k] = 0.0;
       for (int d = 0; d < nper; ++d, ++dg) {
         const uint32_t b = dg & 1u;
         mbar_wait(ACC_FULL(b), (dg >> 1) & 1u);
         tc_fence_after();
-        constexpr int HC = KPAD % 16 ? 8 : 16;           // factor columns at a time (keeps the register count down)
+        // 16 factor columns at a time (keeps the register count down), then the remaining 8 and / or 4
+        const uint32_t acc = tlane + b * SET;
 #pragma unroll
-        for (int h = 0; h < KPAD / HC; ++h) {
-          double v[HC];
-#pragma unroll
-          for (int k = 0; k < HC; ++k) v[k] = 0.0;
-#pragma unroll
-          for (int u = RXU_NU - 1; u >= 0; --u) {
-            uint32_t reg[HC];
-            tmem_ld_n<HC>(tlane + (uint32_t)(b * SET + u * KPAD + HC * h), reg);
-            tmem_ld_wait();
-#pragma unroll
-            for (int k = 0; k < HC; ++k) v[k] = fma(v[k], 256.0, (double)(int)reg[k]);
-          }
-#pragma unroll
-          for (int k = 0; k < HC; ++k) c[HC * h + k] += v[k];
-        }
+        for (int h = 0; h < KS / 16; ++h) rxu_drain_cols<16>(acc, 16 * h, c);
+        if (KS & 8) rxu_drain_cols<8>(acc, KS / 16 * 16, c);
+        if (KS & 4) rxu_drain_cols<4>(acc, KS / 8 * 8, c);
 #pragma unroll
         for (int c0 = 0; c0 < SET; c0 += 16) tmem_st_zero16(tlane + (uint32_t)(b * SET + c0));
         tmem_st_wait();
@@ -354,9 +387,9 @@ __global__ void __launch_bounds__(RXU_THREADS, 1) k_rx_umma(const __grid_constan
         const double rs = scalbn(a.rscale[row], 8 * RXU_UMIN);        // the lowest kept weight is 256^UMIN
         double* o = a.out + ((size_t)seg * a.rows + row) * a.KP;
 #pragma unroll
-        for (int k = 0; k < KPAD; ++k)
+        for (int k = 0; k < KS; ++k)
           if (k < a.KP) o[k] = (k < a.K) ? c[k] * rs * a.cscale[k] : 0.0;
-        for (int k = KPAD; k < a.KP; ++k) o[k] = 0.0;
+        for (int k = KS; k < a.KP; ++k) o[k] = 0.0;
       }
     }
     tc_fence_before();
@@ -403,16 +436,15 @@ __global__ void __launch_bounds__(RXU_THREADS, 1) k_rx_umma(const __grid_constan
             if (elect_one()) {
 #pragma unroll
               for (int kk = 0; kk < RXU_KT / 32; ++kk) {
+                // every plane reads its digits tmin..VDIG-1 from row 0 of the staged B tile
+                const uint64_t bd = umma_desc<RXU_KT>(sa + RXU_A_BYTES) + 2 * kk;
 #pragma unroll
                 for (int p = 0; p < RXU_PLANES; ++p) {
-                  const int tmin = p < RXU_UMIN ? RXU_UMIN - p : 0;
-                  const int nt = RXU_VDIG - tmin;
-                  // D = s32, A = u8 (top plane: s8), B = u8, K-major both, N = nt*KPAD (rounded up to 16: zero digit rows), M = 128
+                  // D = s32, A = u8 (top plane: s8), B = u8, K-major both, N = nt*KS rounded up to 16, M = 128
                   const uint32_t idesc = (2u << 4) | ((p == RXU_PLANES - 1 ? 1u : 0u) << 7) |
-                                         ((uint32_t)(((nt * KPAD + 15) / 16 * 16) >> 3) << 17) | (8u << 24);
+                                         ((uint32_t)(rxu_n(p, KS) >> 3) << 17) | (8u << 24);
                   const uint64_t ad = umma_desc<RXU_KT>(sa + (uint32_t)p * RXU_PLANE_TILE) + 2 * kk;
-                  const uint64_t bd = umma_desc<RXU_KT>(sa + RXU_A_BYTES + (uint32_t)(tmin * KPAD * RXU_KT)) + 2 * kk;
-                  umma_i8(tmem_base + b * SET + (uint32_t)((p + tmin - RXU_UMIN) * KPAD), ad, bd, idesc, 1u);
+                  umma_i8(tmem_base + b * SET + (uint32_t)((RXU_PLANES - 1 - p) * KS), ad, bd, idesc, 1u);
                 }
               }
               umma_commit(EMPTY_BAR(s));
@@ -458,10 +490,10 @@ int launch_rxu_pack(const double* R, const uint32_t* bits, int rows, int ld, uin
   return check_launch("rx_planes_pack");
 }
 
-static int rxu_kpad(int K) { return K <= 16 ? 16 : (K <= 24 ? 24 : 32); }
+static int rxu_stride(int K) { return (K + 3) & ~3; }
 
-// workspace: colmax (32 u64) | cscale (32 f64) | cexp (32 i32) | flag (i32, 16-byte slot) | digits (7*KPAD x ld, 1024-aligned)
-long long rxu_workspace_bytes(int K, long long ld) { return 1024 + (long long)rxu_brows(rxu_kpad(K)) * ld; }
+// workspace: colmax (32 u64) | cscale (32 f64) | cexp (32 i32) | flag (i32, 16-byte slot) | digits (brows x ld, 1024-aligned)
+long long rxu_workspace_bytes(int K, long long ld) { return 1024 + (long long)rxu_brows(rxu_stride(K)) * ld; }
 
 int launch_stats_rx(const double* R, const uint32_t* bits, int rows, int ld, const double* Xp, int K, int nseg, double* out,
                     const int* run_flag, cudaStream_t st);
@@ -470,11 +502,11 @@ int launch_stats_rx_umma(const uint8_t* planes, const double* rscale, const doub
                          int cols, const double* Xp, int K, int nseg, int max_ctas, double* out, void* workspace,
                          long long workspace_bytes, cudaStream_t st) {
   if (rows <= 0 || ld <= 0 || ld % 64 || nseg <= 0 || cols <= 0 || cols > ld) { set_error("stats_rx_umma: bad shape"); return -2; }
-  if (K > 32) { set_error("stats_rx_umma: K=%d > 32 (use the DMMA kernel)", K); return -2; }
+  if (K < 1 || K > 32) { set_error("stats_rx_umma: K=%d outside 1..32 (use the DMMA kernel)", K); return -2; }
   if (workspace_bytes < rxu_workspace_bytes(K, ld)) { set_error("stats_rx_umma: workspace too small"); return -2; }
   EncodeTiledFn encode = get_encode_fn();
   if (!encode) { set_error("stats_rx_umma: cuTensorMapEncodeTiled not available"); return -3; }
-  const int KPAD = rxu_kpad(K), KP = 8 * tiles_for(K);
+  const int KS = rxu_stride(K), KP = 8 * tiles_for(K);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   unsigned long long* colmax = reinterpret_cast<unsigned long long*>(ws);
   double* cscale = reinterpret_cast<double*>(ws + 256);
@@ -483,14 +515,14 @@ int launch_stats_rx_umma(const uint8_t* planes, const double* rscale, const doub
   uint8_t* Bd = ws + 1024;
 
   cudaMemsetAsync(ws, 0, 1024, st);
-  const int brows = rxu_brows(KPAD);
-  if (brows > RXU_VDIG * KPAD) cudaMemsetAsync(Bd + (size_t)RXU_VDIG * KPAD * ld, 0, (size_t)(brows - RXU_VDIG * KPAD) * ld, st);   // the zero digit rows
+  const int brows = rxu_brows(KS);
+  if (brows > RXU_VDIG * KS) cudaMemsetAsync(Bd + (size_t)RXU_VDIG * KS * ld, 0, (size_t)(brows - RXU_VDIG * KS) * ld, st);   // the zero digit rows
   int nb = (cols + 63) / 64;
   if (nb > 296) nb = 296;
   k_rxu_colmax<<<nb, 256, 0, st>>>(Xp, cols, K, KP, colmax, flag);
   k_rxu_colscale<<<1, 32, 0, st>>>(colmax, K, cexp, cscale);
-  const long long qthreads = (long long)(ld / 4) * KPAD;
-  k_rxu_quantize<<<(unsigned)((qthreads + 255) / 256), 256, 0, st>>>(Xp, cols, K, KP, KPAD, (long long)ld, cexp, flag, Bd);
+  const long long qthreads = (long long)(ld / 4) * KS;
+  k_rxu_quantize<<<(unsigned)((qthreads + 255) / 256), 256, 0, st>>>(Xp, cols, K, KP, KS, (long long)ld, cexp, flag, Bd);
   if (check_launch("stats_rx_umma prepass")) return -1;
 
   CUtensorMap tmap;
@@ -523,7 +555,9 @@ int launch_stats_rx_umma(const uint8_t* planes, const double* rscale, const doub
   int nctas = nitems;                                  // default: one item per CTA (the block scheduler balances the tail)
   int cluster = 1;
   if (max_ctas > 0 && max_ctas < nctas && max_ctas <= sm_count) { nctas = max_ctas; if (nctas >= 2) { nctas &= ~1; cluster = 2; } }
-  void (*kern)(const CUtensorMap, RxUmmaArgs) = KPAD == 32 ? k_rx_umma<32> : (KPAD == 24 ? k_rx_umma<24> : k_rx_umma<16>);
+  void (*const kerns[8])(const CUtensorMap, RxUmmaArgs) = {k_rx_umma<4>,  k_rx_umma<8>,  k_rx_umma<12>, k_rx_umma<16>,
+                                                            k_rx_umma<20>, k_rx_umma<24>, k_rx_umma<28>, k_rx_umma<32>};
+  void (*kern)(const CUtensorMap, RxUmmaArgs) = kerns[KS / 4 - 1];
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(nctas); cfg.blockDim = dim3(RXU_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;

@@ -364,7 +364,9 @@ class BNMFEngine:
         # SMs given to the R.X kernel when both statistics kernels run concurrently (0: one after the other).  The Gram
         # kernel's work grows with K(K+1)/2, the R.X kernel's with K and never below the time to stream the planes:
         # measured best 64 at K = 20 (127.3 / 129.6 / 127.6 sweeps/s at 72 / 64 / 60), 80 at K = 10 (208 vs 197 at 64),
-        # 96 at K = 5 (245 vs 228)
+        # 96 at K = 5 (245 vs 228).  Re-measured after the R.X MMAs shrank to N = 640 columns per k-step at K = 20
+        # (profiles/r06_split_sweep.txt, short runs): 64 still best at K = 20 (132.5 vs 131.8 / 131.8 / 130.1 at 56 / 72 /
+        # 80: with fewer SMs the R.X kernel outlasts the Gram), K = 10, 24 and 32 within 0.3 % of the values tried
         self.split = int(os.environ.get("BNMTF_SPLIT", "64" if self.K > 16 else ("80" if self.K > 8 else "96")))
         # Gram kernel form (bit 0: CTA pairs, cta_group::2; bit 1: 2:4-sparse MMAs + fp64 fix-up segment; bit 2: clusters of
         # two pairs with multicast digit tiles).  Measured at the headline shape (DESIGN.md section 4): the sparse kernel
