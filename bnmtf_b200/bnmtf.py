@@ -14,18 +14,59 @@ import os
 import random
 
 import numpy as np
+import scipy.sparse
 import torch
 
 from . import _lib
+from .data import training_csr, validate_sparse
 from .bnmf import METRICS, QUALITY, _TwoFactorBase, _elbo_alpha_s_correction, _metrics_from_sums
-from .engine import (MODE, Dataset, Factor, Partition, capture_graph, thread_flags, S_BETA_S, S_ELBO, S_ESD, S_LOGTAU, S_TAU, _ptr, _stream, gram_len,
-                     kp_for, require_cuda)
+from .engine import (CSR_METRIC_CTAS, MODE, Dataset, Factor, Partition, SparseDataset, capture_graph, thread_flags, S_BETA_S, S_ELBO,
+                     S_ESD, S_LOGTAU, S_TAU, _ptr, _stream, gram_len, kp_for, require_cuda)
 
 
 class BNMTFEngine:
     """Device state and sweep driver for one (R, M, K, L)."""
 
     def __init__(self, dataset, K, L, mode, alpha, beta, seed=0):
+        self._alloc(dataset, K, L, mode, alpha, beta, seed)
+        ds, dev = dataset, dataset.device
+        I, J = ds.I, ds.J
+        f64 = lambda *s: torch.zeros(s, dtype=torch.float64, device=dev)
+        self.nseg_m = max(1, min(ds.ldJ // 128, -(-1776 // ((I + 127) // 128))))
+        self.mpart = f64(((I + 127) // 128) * self.nseg_m * 8)
+        # Statistics kernels: the fp64 mma.sync ones at toy / GDSC sizes (latency-bound there, fewer launches), the tcgen05
+        # fixed-point ones of the two-factor engine for large matrices (BNMTF_NMTF_STATS=umma|dmma overrides).  A dataset
+        # with outlier rows (Dataset.wide) keeps fp64; the per-phase dynamic-range guard of the two-factor engine is not
+        # wired into the tri-factor kernels.
+        want = os.environ.get("BNMTF_NMTF_STATS", "umma" if I * J >= (1 << 22) else "dmma")
+        self.stats_impl = "dmma"
+        if want == "umma" and max(self.K, self.L) <= 32:
+            for side in (0, 1):
+                ds.ensure_planes(side)
+            if not any(ds.wide.values()):
+                self.stats_impl = "umma"
+                self.wsrx_bytes = max(_lib.call("bnmtf_rx_umma_workspace_bytes", d, ld) for d, ld in ((self.L, ds.ldJ), (self.K, ds.ldI)))
+                self.wsrx = torch.zeros(self.wsrx_bytes + 1024, dtype=torch.uint8, device=dev)
+                self.wsrx_ptr = (self.wsrx.data_ptr() + 1023) // 1024 * 1024
+                self.ws_bytes = max(_lib.call("bnmtf_gram_umma_workspace_bytes", d, int(self.vb), ld)
+                                    for d, ld in ((self.L, ds.ldJ), (self.K, ds.ldI)))
+                self.ws = torch.zeros(self.ws_bytes + 1024, dtype=torch.uint8, device=dev)
+                self.ws_ptr = (self.ws.data_ptr() + 1023) // 1024 * 1024
+        # training metrics of a sweep: "stats" = from the column statistics of the G phase (csrc/nmtf.cu::k_nmtf_mstat: no
+        # third pass over R; the direct pass runs only when the device-side cancellation guard trips, as in the two-factor
+        # engine), "direct" = always the pass over R
+        self.metrics_mode = os.environ.get("BNMTF_METRICS", "stats" if self.stats_impl == "umma" else "direct")
+        self.statics = f64(3)
+        _lib.call("bnmtf_masked_metrics_f64", _ptr(ds.R), _ptr(ds.bits), I, ds.ldJ, _ptr(self.FS.Xp), _ptr(self.G.Xp),
+                  self.L, self.nseg_m, 0, _ptr(self.mpart), _ptr(self.m8), 0, _stream())
+        self.statics.copy_(self.m8[4:7])
+        if ds.n_obs is None:
+            ds.n_obs = float(self.statics[2].item())
+        self.polarity = 0 if ds.n_obs >= 0.5 * I * J else 1
+        self._set_omega()
+
+    def _alloc(self, dataset, K, L, mode, alpha, beta, seed):
+        """Factors, S, the statistics records of both phases and the scratch of the sweep: what every format needs."""
         self.ds, self.K, self.L, self.mode = dataset, int(K), int(L), mode
         self.m, self.vb = MODE[mode], mode == "vb"
         self.alpha, self.beta, self.seed = float(alpha), float(beta), int(seed) & (2 ** 64 - 1)
@@ -63,49 +104,20 @@ class BNMTFEngine:
         self.extra = f64(J)
         self.red = f64(24)
         self.m8, self.el8, self.ex1 = self.red[0:8], self.red[8:16], self.red[16:17]
-        self.nseg_m = max(1, min(ds.ldJ // 128, -(-1776 // ((I + 127) // 128))))
-        self.mpart = f64(((I + 127) // 128) * self.nseg_m * 8)
         self.nb_terms = 32 if max(I * self.K, J * self.L) <= (1 << 16) else 296      # CTAs of the ELBO factor terms
         self.elpart = f64(3 * self.nb_terms * 8)
-        # Statistics kernels: the fp64 mma.sync ones at toy / GDSC sizes (latency-bound there, fewer launches), the tcgen05
-        # fixed-point ones of the two-factor engine for large matrices (BNMTF_NMTF_STATS=umma|dmma overrides).  A dataset
-        # with outlier rows (Dataset.wide) keeps fp64; the per-phase dynamic-range guard of the two-factor engine is not
-        # wired into the tri-factor kernels.
-        want = os.environ.get("BNMTF_NMTF_STATS", "umma" if I * J >= (1 << 22) else "dmma")
-        self.stats_impl = "dmma"
-        if want == "umma" and max(self.K, self.L) <= 32:
-            for side in (0, 1):
-                ds.ensure_planes(side)
-            if not any(ds.wide.values()):
-                self.stats_impl = "umma"
-                self.wsrx_bytes = max(_lib.call("bnmtf_rx_umma_workspace_bytes", d, ld) for d, ld in ((self.L, ds.ldJ), (self.K, ds.ldI)))
-                self.wsrx = torch.zeros(self.wsrx_bytes + 1024, dtype=torch.uint8, device=dev)
-                self.wsrx_ptr = (self.wsrx.data_ptr() + 1023) // 1024 * 1024
-                self.ws_bytes = max(_lib.call("bnmtf_gram_umma_workspace_bytes", d, int(self.vb), ld)
-                                    for d, ld in ((self.L, ds.ldJ), (self.K, ds.ldI)))
-                self.ws = torch.zeros(self.ws_bytes + 1024, dtype=torch.uint8, device=dev)
-                self.ws_ptr = (self.ws.data_ptr() + 1023) // 1024 * 1024
-        # training metrics of a sweep: "stats" = from the column statistics of the G phase (csrc/nmtf.cu::k_nmtf_mstat: no
-        # third pass over R; the direct pass runs only when the device-side cancellation guard trips, as in the two-factor
-        # engine), "direct" = always the pass over R
-        self.metrics_mode = os.environ.get("BNMTF_METRICS", "stats" if self.stats_impl == "umma" else "direct")
         self.guard = 1e-5
         self.mstat, self.mstat_part, self.sums4, self.m8d = f64(J, 4), f64(256), f64(4), f64(8)
         self.flag = torch.zeros(1, dtype=torch.int32, device=dev)
         self._side = self._ev = None
-        self.statics = f64(3)
-        _lib.call("bnmtf_masked_metrics_f64", _ptr(ds.R), _ptr(ds.bits), I, ds.ldJ, _ptr(self.FS.Xp), _ptr(self.G.Xp),
-                  self.L, self.nseg_m, 0, _ptr(self.mpart), _ptr(self.m8), 0, _stream())
-        self.statics.copy_(self.m8[4:7])
-        if ds.n_obs is None:
-            ds.n_obs = float(self.statics[2].item())
-        self.polarity = 0 if ds.n_obs >= 0.5 * I * J else 1
+        self.sterm = None
+
+    def _set_omega(self):
         from scipy.special import gammaln, psi
-        self.size_Omega = float(ds.n_obs)
+        self.size_Omega = float(self.ds.n_obs)
         self.alpha_s = self.alpha + self.size_Omega / 2.0
         self.digamma_alpha_s, self.lgamma_alpha = float(psi(self.alpha_s)), float(gammaln(self.alpha))
         self.lgamma_alpha_s = float(gammaln(self.alpha_s))
-        self.sterm = None
 
     # ---- small problems: the whole run as ONE kernel (csrc/small.cu::k_small_tri) -------------------------------
     def small_cluster(self):
@@ -383,6 +395,64 @@ class BNMTFEngine:
         self.trace_base = self.sweeps_done
 
 
+class SparseBNMTFEngine(BNMTFEngine):
+    """BNMTFEngine on a SparseDataset.  The format decision lives here: the statistics of a phase come from one
+    bnmtf_csr_stats_f64 call over the phase's CSR (rows of R against G, rows of R^T against F; fp64, polarity 1, one
+    record per row: no digit planes, no unmasked totals), the sweep's metrics from the column statistics with
+    bnmtf_csr_metrics_f64 as the gated direct pass.  Transform, S-phase reduction, solvers, end of the sweep and CUDA-graph
+    replay are BNMTFEngine's, which read the same records at polarity 1."""
+
+    def __init__(self, dataset, K, L, mode, alpha, beta, seed=0):
+        if dataset.world != 1:
+            raise ValueError("sparse input runs on one GPU")
+        self._alloc(dataset, K, L, mode, alpha, beta, seed)
+        f64 = lambda *s: torch.zeros(s, dtype=torch.float64, device=dataset.device)
+        KPm, GLm = max(kp_for(self.K), kp_for(self.L)), max(gram_len(self.K), gram_len(self.L))
+        smax = max(1, dataset.csr[0].n_slots, dataset.csr[1].n_slots)
+        # chunk partials of the long rows, for the wider of the two phases
+        self.RXc, self.Gc = f64(smax, KPm), f64(smax, GLm)
+        self.SVc = f64(smax, KPm) if self.vb else None
+        self.mpart = f64(CSR_METRIC_CTAS * 8)
+        self.stats_impl, self.metrics_mode, self.polarity = "csr", "stats", 1
+        self._small_c = 0               # never the single-kernel small path
+        self.statics = dataset.statics.clone()
+        self._set_omega()
+
+    def _csr_stats(self, side, st, other, need_rx):
+        c = self.ds.csr[side]
+        other.pad()
+        _lib.call("bnmtf_csr_stats_f64", _ptr(c.rowptr), _ptr(c.colidx), _ptr(c.val), _ptr(c.item_begin), _ptr(c.item_row),
+                  _ptr(c.item_slot), c.n_items, c.chunk, _ptr(c.heavy_row), _ptr(c.heavy_first), c.n_heavy, _ptr(other.Xp),
+                  _ptr(other.Vp), other.K, _ptr(st["RX"]) if need_rx else 0, _ptr(st["G"]), _ptr(st["SV"]) if self.vb else 0,
+                  _ptr(self.RXc), _ptr(self.Gc), _ptr(self.SVc), _stream())
+
+    def stats_rows(self, need_rx=True):
+        self._csr_stats(0, self.row, self.G, need_rx)
+
+    def stats_cols(self, need_rx=True):
+        self._csr_stats(1, self.col, self.F, need_rx)
+
+    def metrics(self, bits=None, gated=False):
+        """The seven sums over the entry set `bits` (None: the training entries; else a DeviceCSR from pack_mask) with the
+        prediction (F S) G^T -> self.m8 (gated: -> self.m8d, only if the device flag is raised)."""
+        _lib.call("bnmtf_small_matmul_f64", _ptr(self.F.fac), _ptr(self.S["fac"]), self.ds.I, self.K, self.L, 0,
+                  _ptr(self.FS.fac), _stream())
+        self.FS.pad()
+        self.G.pad()
+        entries = self.ds.csr[0] if bits is None else bits
+        entries.metrics(self.FS.Xp, self.G.Xp, self.L, self.mpart, self.m8d if gated else self.m8,
+                        self.flag if gated else None)
+
+    def small_cluster(self):
+        return 0
+
+
+def tri_engine_for(dataset, K, L, mode, alpha, beta, seed=0):
+    """The engine that runs on `dataset`: SparseBNMTFEngine for a SparseDataset, BNMTFEngine otherwise."""
+    cls = SparseBNMTFEngine if isinstance(dataset, SparseDataset) else BNMTFEngine
+    return cls(dataset, K, L, mode, alpha, beta, seed=seed)
+
+
 # =====================================================================================================
 class _ThreeFactorBase(object):
     _mode = None
@@ -395,19 +465,29 @@ class _ThreeFactorBase(object):
     check_empty_rows_columns = _TwoFactorBase.check_empty_rows_columns
 
     def __init__(self, R, M, K, L, priors, device=None, seed=None):
-        self.R = np.array(R, dtype=float)
-        self.M = np.array(M, dtype=float)
-        self.K = K
-        self.L = L
+        self._sparse = scipy.sparse.issparse(R)
+        if self._sparse:
+            # sparse input (as in the two-factor models): the stored entries of R are its known entries, explicit zeros
+            # included; M (or None: all of them) selects the training entries; self.R / self.M are canonical CSR matrices
+            self.R, self.M, self._train = validate_sparse(R, M)
+            self.K = K
+            self.L = L
+            (self.I, self.J) = self.R.shape
+            self.size_Omega = float(self.M.nnz)
+        else:
+            self.R = np.array(R, dtype=float)
+            self.M = np.array(M, dtype=float)
+            self.K = K
+            self.L = L
 
-        assert len(self.R.shape) == 2, "Input matrix R is not a two-dimensional array, " \
-            "but instead %s-dimensional." % len(self.R.shape)
-        assert self.R.shape == self.M.shape, "Input matrix R is not of the same size as " \
-            "the indicator matrix M: %s and %s respectively." % (self.R.shape, self.M.shape)
+            assert len(self.R.shape) == 2, "Input matrix R is not a two-dimensional array, " \
+                "but instead %s-dimensional." % len(self.R.shape)
+            assert self.R.shape == self.M.shape, "Input matrix R is not of the same size as " \
+                "the indicator matrix M: %s and %s respectively." % (self.R.shape, self.M.shape)
 
-        (self.I, self.J) = self.R.shape
-        self.size_Omega = self.M.sum()
-        self.check_empty_rows_columns()
+            (self.I, self.J) = self.R.shape
+            self.size_Omega = self.M.sum()
+            self.check_empty_rows_columns()
 
         self.alpha, self.beta, self.lambdaF, self.lambdaS, self.lambdaG = \
             float(priors['alpha']), float(priors['beta']), np.array(priors['lambdaF']), np.array(priors['lambdaS']), np.array(priors['lambdaG'])
@@ -426,10 +506,12 @@ class _ThreeFactorBase(object):
 
     @classmethod
     def from_dataset(cls, dataset, K, L, priors, seed=None):
-        """Build a model on an engine.Dataset that already lives on the GPU (matrices too large for, or never present in,
-        host memory).  R and M stay None on the host, so init_FG='kmeans' (a host algorithm on R) is not available."""
+        """Build a model on an engine.Dataset / engine.SparseDataset that already lives on the GPU (matrices too large for,
+        or never present in, host memory).  R and M stay None on the host.  init_FG='kmeans' works on a SparseDataset (it
+        clusters the dataset's host CSR of the training entries), not on a dense Dataset."""
         self = cls.__new__(cls)
         self.R = self.M = None
+        self._sparse = isinstance(dataset, SparseDataset)
         self.K, self.L = K, L
         (self.I, self.J) = (dataset.I, dataset.J)
         self.size_Omega = float(dataset.n_obs)
@@ -438,16 +520,19 @@ class _ThreeFactorBase(object):
             lam = np.array(priors[name], dtype=float)
             setattr(self, name, lam * np.ones(shape) if lam.shape == () else lam)
         self._device_arg, self._seed, self.verbose = dataset.device, seed, False
-        self._eng = BNMTFEngine(dataset, K, L, cls._mode, self.alpha, self.beta,
-                                seed=seed if seed is not None else _lib.derive_seed())
+        self._eng = tri_engine_for(dataset, K, L, cls._mode, self.alpha, self.beta,
+                                   seed=seed if seed is not None else _lib.derive_seed())
         return self
 
     def _engine(self):
         if self._eng is None:
             dev = require_cuda(self._device_arg)
-            ds = Dataset.from_host(self.R, self.M, dev)
+            if getattr(self, '_sparse', False):
+                ds = SparseDataset(self.R, self._train, dev)
+            else:
+                ds = Dataset.from_host(self.R, self.M, dev)
             seed = self._seed if self._seed is not None else _lib.derive_seed()
-            self._eng = BNMTFEngine(ds, self.K, self.L, self._mode, self.alpha, self.beta, seed=seed)
+            self._eng = tri_engine_for(ds, self.K, self.L, self._mode, self.alpha, self.beta, seed=seed)
         return self._eng
 
     def triple_dot(self, M1, M2, M3):
@@ -471,8 +556,21 @@ class _ThreeFactorBase(object):
         return eng.m8.cpu().numpy()
 
     def _kmeans_init(self, offset):
-        from .kmeans import KMeans
+        from .kmeans import KMeans, SparseKMeans
         dev = require_cuda(self._device_arg)            # the assignment step runs on the device (csrc/kmeans.cu)
+        if getattr(self, '_sparse', False):
+            # the observed entries only: the clusterings of KMeans on (R.toarray(), M.toarray()) and on their transposes
+            if self.R is None:                          # from_dataset(SparseDataset)
+                Xt, Xall = self._eng.ds.host_train, self._eng.ds.host_R
+            else:
+                Xt, Xall = training_csr(self.R, self._train), self.R
+            kmeans_F = SparseKMeans(Xt, self.K, X_all=Xall, device=dev)
+            kmeans_F.initialise()
+            kmeans_F.cluster()
+            kmeans_G = SparseKMeans(Xt.T.tocsr(), self.L, X_all=Xall.T.tocsr(), device=dev)
+            kmeans_G.initialise()
+            kmeans_G.cluster()
+            return kmeans_F.clustering_results + offset, kmeans_G.clustering_results + offset
         kmeans_F = KMeans(self.R, self.M, self.K, device=dev)
         kmeans_F.initialise()
         kmeans_F.cluster()

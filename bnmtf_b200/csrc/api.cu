@@ -94,6 +94,10 @@ int launch_small_tri(TriArgs, cudaStream_t);
 int small_cluster_size(int, int, int, int);
 int launch_small_sweeps(SmallArgs, cudaStream_t);
 int launch_kmeans_dist(const double*, const double*, int, int, const double*, const double*, int, double*, cudaStream_t);
+int launch_kmeans_csr_dist(const int64_t*, const int32_t*, const double*, long long, long long, const double*, const double*, int,
+                           double*, cudaStream_t);
+int launch_kmeans_csr_sums(const int64_t*, const int32_t*, const double*, long long, const int32_t*, int, int, double*, double*,
+                           cudaStream_t);
 int launch_row_solve(const RowSolveArgs&, cudaStream_t);
 int launch_np_build_pred(const double*, const double*, int, int, int, int, double*, cudaStream_t);
 int launch_np_row_update(const double*, const uint32_t*, double*, int, int, int, double*, const double*, int, cudaStream_t);
@@ -348,6 +352,16 @@ int bnmtf_small_tri_sweeps_f64(int mode, const double* R, const uint32_t* bits, 
 int bnmtf_kmeans_distances_f64(const double* X, const double* M, int64_t n, int64_t d, const double* centroids,
                                const double* mask_centroids, int K, double* dist, void* stream) {
   return launch_kmeans_dist(X, M, (int)n, (int)d, centroids, mask_centroids, K, dist, ST(stream));
+}
+
+int bnmtf_csr_kmeans_distances_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t n, int64_t d,
+                                   const double* centroids, const double* mask_centroids, int K, double* dist, void* stream) {
+  return launch_kmeans_csr_dist(rowptr, colidx, val, n, d, centroids, mask_centroids, K, dist, ST(stream));
+}
+
+int bnmtf_csr_kmeans_sums_f64(const int64_t* coordptr, const int32_t* point, const double* val, int64_t d,
+                              const int32_t* assign, int K, int only, double* sums, double* counts, void* stream) {
+  return launch_kmeans_csr_sums(coordptr, point, val, d, assign, K, only, sums, counts, ST(stream));
 }
 
 int bnmtf_stats_gram_fixup_f64(const uint32_t* bits, int64_t rows, int64_t ld, int64_t cols, const double* Xp, const double* Vp,

@@ -182,6 +182,17 @@ def sparse_selection(Rc, M, name="M"):
     return sel
 
 
+def training_csr(Rc, train):
+    """The training entries of the canonical CSR Rc as a canonical CSR (train: bool per stored entry, or None: all)."""
+    import scipy.sparse as sp
+    if train is None or bool(np.all(train)):
+        return Rc
+    I = Rc.shape[0]
+    rows = np.repeat(np.arange(I, dtype=np.int64), np.diff(Rc.indptr))[train]
+    indptr = np.concatenate([[0], np.cumsum(np.bincount(rows, minlength=I))]).astype(np.int64)
+    return sp.csr_matrix((Rc.data[train], Rc.indices[train], indptr), shape=Rc.shape)
+
+
 def validate_sparse(R, M=None):
     """Host-side checks and canonical form of sparse input (no GPU call): -> (R as canonical CSR, M as CSR of ones on the
     training entries, bool per stored entry of R: training or not).  M None: every stored entry of R is a training

@@ -968,17 +968,12 @@ class SparseDataset:
 
     def __init__(self, host_R, train, device):
         """host_R: canonical scipy.sparse CSR (sorted indices, no duplicates); train: bool per stored entry, or None (all)."""
-        import scipy.sparse as sp
         self.I, self.J = host_R.shape
         self.device = device
         self.partI, self.partJ = Partition(self.I), Partition(self.J)
+        from .data import training_csr
         self.host_R = host_R
-        if train is None or bool(np.all(train)):
-            Rt = host_R
-        else:
-            rows = np.repeat(np.arange(self.I, dtype=np.int64), np.diff(host_R.indptr))[train]
-            indptr = np.concatenate([[0], np.cumsum(np.bincount(rows, minlength=self.I))]).astype(np.int64)
-            Rt = sp.csr_matrix((host_R.data[train], host_R.indices[train], indptr), shape=host_R.shape)
+        self.host_train = Rt = training_csr(host_R, train)      # host CSR of the training entries (K-means initialisation)
         RtT = Rt.tocsc()            # scipy's counting sort: column-major with sorted row indices, explicit zeros kept
         self.csr = {0: DeviceCSR(Rt.indptr, Rt.indices, Rt.data, device),
                     1: DeviceCSR(RtT.indptr, RtT.indices, RtT.data, device)}

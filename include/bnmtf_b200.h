@@ -162,6 +162,18 @@ int bnmtf_small_tri_sweeps_f64(int mode, const double* R, const uint32_t* bits, 
  * cluster membership). */
 int bnmtf_kmeans_distances_f64(const double* X, const double* M, int64_t n, int64_t d, const double* centroids,
                                const double* mask_centroids, int K, double* dist, void* stream);
+/* The same distances for points held as a CSR of their observed entries (rowptr: n + 1 int64, colidx: int32 ascending within
+ * a row and < d, val: double; every stored entry has m = 1): equal, bit for bit, to bnmtf_kmeans_distances_f64 on the
+ * zero-filled dense X and the 0/1 dense M.  centroids, mask_centroids: K x d dense. */
+int bnmtf_csr_kmeans_distances_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t n, int64_t d,
+                                   const double* centroids, const double* mask_centroids, int K, double* dist, void* stream);
+/* Centroid update of K-means on the observed entries: from the coordinate-major CSR (coordptr: d + 1 int64; point: int32
+ * ascending within a coordinate; val: double), sums[c*d + j] = the values at coordinate j of the points assigned to c
+ * (assign: int32 per point), added one after the other in ascending point order, and counts[c*d + j] = their number --
+ * numpy's (Mc * Xc).sum(axis=0) and Mc.sum(axis=0) over the ascending members, bit for bit, for d >= 2.  only >= 0: cluster
+ * `only` alone (only its rows of sums / counts are written).  2 <= d, 1 <= K <= 64. */
+int bnmtf_csr_kmeans_sums_f64(const int64_t* coordptr, const int32_t* point, const double* val, int64_t d,
+                              const int32_t* assign, int K, int only, double* sums, double* counts, void* stream);
 /* The share the 2:4-sparse form leaves out (third and fourth selected column of every aligned group of four: 0.7 % of
  * the entries at 20 % missing), summed in fp64 (mma.sync.m8n8k4.f64 on gathered factor rows) into ONE segment: Gseg /
  * SVseg point at `rows` records laid out like a segment of Gpart / SVpart; pass nseg + 1 segments to the solver.  K <= 31. */
