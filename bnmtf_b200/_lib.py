@@ -73,6 +73,11 @@ SIGNATURES = {
     "bnmtf_np_row_update_f64": [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p, c_i, c_p],
     "bnmtf_np_s_update_f64": [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_i, c_i, c_p, c_i, c_i, c_p, c_p, c_i, c_p],
     "bnmtf_np_metrics_f64": [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_i, c_p, c_p],
+    "bnmtf_csr_np_row_update_f64": [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_i, c_i,
+                                    c_i, c_p, c_p],
+    "bnmtf_csr_np_s_update_f64": [c_p, c_p, c_p, c_p, c_p, c_i64, c_i, c_p, c_p, c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_p, c_i,
+                                  c_p],
+    "bnmtf_csr_np_metrics_f64": [c_p, c_p, c_p, c_i64, c_p, c_p, c_i, c_p, c_i, c_p, c_p],
     "bnmtf_small_matmul_f64": [c_p, c_p, c_i64, c_i, c_i, c_i, c_p, c_p],
     "bnmtf_tn_moments_f64": [c_p, c_p, c_i64, c_p, c_p, c_p],
     "bnmtf_tn_draw_f64": [c_p, c_p, c_i64, c_u64, c_u64, c_p, c_p],
@@ -96,7 +101,9 @@ KERNELS_PER_CALL = {"bnmtf_pack_dataset_f64": 1, "bnmtf_pack_mask_f64": 1, "bnmt
                     "bnmtf_dense_metrics_f64": 2, "bnmtf_vb_factor_terms_f64": 1, "bnmtf_reduce8_f64": 1,
                     "bnmtf_reduce1_f64": 1, "bnmf_finish_sweep_f64": 1, "bnmtf_tn_moments_f64": 1, "bnmtf_np_build_pred_f64": 1,
                     "bnmtf_np_row_update_f64": 1, "bnmtf_np_s_update_f64": 2, "bnmtf_np_metrics_f64": 2,
-                    "bnmtf_small_matmul_f64": 1, "bnmtf_nmtf_transform_f64": 1, "bnmtf_nmtf_sq_f64": 2,
+                    "bnmtf_small_matmul_f64": 1, "bnmtf_csr_np_metrics_f64": 2,
+                    # one launch per non-empty plan class / per pair plus one: the engine adds the rest
+                    "bnmtf_csr_np_row_update_f64": 0, "bnmtf_csr_np_s_update_f64": 1, "bnmtf_nmtf_transform_f64": 1, "bnmtf_nmtf_sq_f64": 2,
                     "bnmtf_coord_solve_f64": 1, "bnmtf_nmtf_extra_f64": 1, "bnmtf_nmtf_mstat_f64": 1,
                     "bnmtf_tn_draw_f64": 1, "bnmtf_gamma_draw_f64": 1, "bnmtf_exponential_draw_f64": 1}
 launch_count = [0]

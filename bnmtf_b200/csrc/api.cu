@@ -51,6 +51,13 @@ int launch_csr_stats(const int64_t*, const int32_t*, const double*, const int64_
                      double*, double*, double*, cudaStream_t);
 int launch_csr_metrics(const int64_t*, const int32_t*, const double*, long long, const double*, const double*, int, double*, int,
                        double*, const int*, cudaStream_t);
+int launch_csr_np_metrics(const int64_t*, const int32_t*, const double*, long long, const double*, const double*, int, double*, int,
+                          double*, cudaStream_t);
+int launch_csr_np_row_update(const int64_t*, const int64_t*, const int32_t*, const long long*, const int32_t*, const double*,
+                             double*, const double*, int, int, int, double*, cudaStream_t);
+int launch_csr_np_s_update(const int64_t*, const int32_t*, const double*, const int64_t*, const int32_t*, long long, int,
+                           const double*, const double*, int, const double*, int, const int32_t*, int, double*, double*,
+                           double*, int, cudaStream_t);
 int launch_metrics_from_sums(const double*, const double*, double, double*, int*, cudaStream_t);
 int launch_select_metrics(const int*, const double*, double*, cudaStream_t);
 int launch_vb_factor_terms(const double*, const double*, const double*, const double*, const double*, long long, double*, int, cudaStream_t);
@@ -504,6 +511,41 @@ int bnmtf_np_metrics_f64(const double* R, const uint32_t* bits, const double* P,
   int rc = launch_np_metrics(R, bits, P, (int)rows, (int)cols, (int)ld, partials, nparts, ST(stream));
   if (rc) return rc;
   return launch_reduce8(partials, nparts, out8, ST(stream));
+}
+
+int bnmtf_csr_np_row_update_f64(const int64_t* item_beg, const int64_t* item_end, const int32_t* item_row, int64_t n_warp,
+                                int64_t n_cta, int64_t n_c2, int64_t n_c4, int64_t n_c8, int64_t n_c16,
+                                const int32_t* colidx, const double* val, double* A, const double* B, int K, int k0, int k1,
+                                double* pw, void* stream) {
+  if (check_k(K)) return -2;
+  if (k0 < 0 || k1 <= k0 || k1 > K) { set_error("csr_np_row_update: column range [%d, %d) outside [0, %d)", k0, k1, K); return -2; }
+  const long long counts[6] = {n_warp, n_cta, n_c2, n_c4, n_c8, n_c16};
+  for (int c = 0; c < 6; ++c) {
+    if (counts[c] < 0 || counts[c] > 0x7fffffffLL || (c >= 2 && counts[c] % (1LL << (c - 1)) != 0)) {
+      set_error("csr_np_row_update: bad plan count %lld for class %d", counts[c], c);
+      return -2;
+    }
+  }
+  if (n_c2 + n_c4 + n_c8 + n_c16 > 0 && !pw) { set_error("csr_np_row_update: cluster items need the scratch pw"); return -2; }
+  return launch_csr_np_row_update(item_beg, item_end, item_row, counts, colidx, val, A, B, K, k0, k1, pw, ST(stream));
+}
+int bnmtf_csr_np_s_update_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, const int64_t* item_begin,
+                              const int32_t* item_row, int64_t n_items, int chunk, const double* FS, const double* F, int K,
+                              const double* G, int L, const int32_t* pairs, int n_pairs, double* S, double* pw,
+                              double* partials, int nparts, void* stream) {
+  if (check_k(K) || check_k(L)) return -2;
+  if (n_items <= 0 || chunk <= 0 || n_pairs < 1 || nparts < 1) {
+    set_error("csr_np_s_update: bad arguments (n_items=%lld chunk=%d n_pairs=%d nparts=%d)", (long long)n_items, chunk, n_pairs,
+              nparts);
+    return -2;
+  }
+  return launch_csr_np_s_update(rowptr, colidx, val, item_begin, item_row, n_items, chunk, FS, F, K, G, L, pairs, n_pairs, S, pw,
+                                partials, nparts, ST(stream));
+}
+int bnmtf_csr_np_metrics_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t rows, const double* A,
+                             const double* B, int K, double* partials, int nparts, double* out8, void* stream) {
+  if (check_k(K)) return -2;
+  return launch_csr_np_metrics(rowptr, colidx, val, rows, A, B, K, partials, nparts, out8, ST(stream));
 }
 int bnmtf_small_matmul_f64(const double* A, const double* B, int64_t n, int p, int q, int transB, double* C, void* stream) {
   return launch_small_matmul(A, B, (int)n, p, q, transB, C, ST(stream));

@@ -147,17 +147,20 @@ __global__ void __launch_bounds__(256) k_csr_combine(const int32_t* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------------
-// k_csr_metrics: partial sums over the stored entries of a CSR of {e^2, p, p^2, r p, r, r^2, 1}, p = A_i . B_j (k < K).
+// k_csr_metrics: partial sums over the stored entries of a CSR of {e^2, p, p^2, r p, r, r^2, 1}, p = A_i . B_j (k < K, rows
+// KP apart), and with IDIV the I-divergence term r log(r/p) - r + p of the non-probabilistic models as the eighth.
 // One warp per row (rows assigned round-robin over a fixed grid), lanes stride over the row's entries; per-lane sums in
 // entry order, then a fixed shuffle tree and a fixed per-CTA order -> one 8-vector per CTA.
 // ---------------------------------------------------------------------------------------------------
+template <bool IDIV>
 __global__ void __launch_bounds__(256) k_csr_metrics(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ colidx,
                                                      const double* __restrict__ val, int64_t rows,
                                                      const double* __restrict__ Ap, const double* __restrict__ Bp, int K,
                                                      int KP, double* __restrict__ partials, const int* __restrict__ run_flag) {
   if (run_flag && *run_flag == 0) return;      // gated fallback of the statistics-based metrics (uniform exit)
+  constexpr int NS = IDIV ? 8 : 7;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  double s[7] = {0, 0, 0, 0, 0, 0, 0};
+  double s[NS] = {};
   for (int64_t i = (int64_t)blockIdx.x * 8 + warp; i < rows; i += (int64_t)gridDim.x * 8) {
     const double* a = Ap + (size_t)i * KP;
     for (int64_t idx = rowptr[i] + lane; idx < rowptr[i + 1]; idx += 32) {
@@ -172,18 +175,19 @@ __global__ void __launch_bounds__(256) k_csr_metrics(const int64_t* __restrict__
       s[4] += r;
       s[5] = fma(r, r, s[5]);
       s[6] += 1.0;
+      if (IDIV) s[NS - 1] += r * log(r / p) - r + p;
     }
   }
   __shared__ double red[8][8];
 #pragma unroll
-  for (int q = 0; q < 7; ++q) {
+  for (int q = 0; q < NS; ++q) {
     const double v = warp_sum(s[q]);
     if (lane == 0) red[warp][q] = v;
   }
   __syncthreads();
   if (threadIdx.x < 8) {
     double v = 0.0;
-    if (threadIdx.x < 7) for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
+    if (threadIdx.x < NS) for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
     partials[(size_t)blockIdx.x * 8 + threadIdx.x] = v;
   }
 }
@@ -246,9 +250,17 @@ int launch_csr_metrics(const int64_t* rowptr, const int32_t* colidx, const doubl
                        const double* Bp, int K, double* partials, int nparts, double* out8, const int* run_flag,
                        cudaStream_t st) {
   if (rows <= 0 || nparts <= 0) { set_error("csr_metrics: bad shape rows=%lld nparts=%d", rows, nparts); return -2; }
-  k_csr_metrics<<<nparts, 256, 0, st>>>(rowptr, colidx, val, rows, Ap, Bp, K, 8 * tiles_for(K), partials, run_flag);
+  k_csr_metrics<false><<<nparts, 256, 0, st>>>(rowptr, colidx, val, rows, Ap, Bp, K, 8 * tiles_for(K), partials, run_flag);
   k_csr_metrics_final<<<1, 32, 0, st>>>(partials, nparts, out8, run_flag);
   return check_launch("csr_metrics");
+}
+
+int launch_csr_np_metrics(const int64_t* rowptr, const int32_t* colidx, const double* val, long long rows, const double* A,
+                          const double* B, int K, double* partials, int nparts, double* out8, cudaStream_t st) {
+  if (rows <= 0 || nparts <= 0) { set_error("csr_np_metrics: bad shape rows=%lld nparts=%d", rows, nparts); return -2; }
+  k_csr_metrics<true><<<nparts, 256, 0, st>>>(rowptr, colidx, val, rows, A, B, K, K, partials, nullptr);
+  k_csr_metrics_final<<<1, 32, 0, st>>>(partials, nparts, out8, nullptr);
+  return check_launch("csr_np_metrics");
 }
 
 }  // namespace bnmtf

@@ -222,8 +222,9 @@ def validate_sparse(R, M=None):
 def upload_sparse(R, M=None, device=None):
     """Sparse (R, M) -> engine.SparseDataset on `device` (default: the current CUDA device): the training entries in
     CSR form for the row phase and for the column phase, with the static work plan of the statistics kernel.  R and M
-    as the model constructors take them (validate_sparse).  The result can be passed to `Model.from_dataset(ds, K,
-    priors)` of the two-factor models so that several models share one resident copy of the matrix."""
+    as the model constructors take them (validate_sparse).  The result can be passed to `from_dataset` of every model
+    class -- `Model.from_dataset(ds, K, priors)` / `(ds, K, L, priors)` of the Bayesian models, `NMF.from_dataset(ds, K)`,
+    `NMTF.from_dataset(ds, K, L)` -- so that several models share one resident copy of the matrix."""
     from .engine import SparseDataset, require_cuda
     Rc, _, train = validate_sparse(R, M)
     return SparseDataset(Rc, train, require_cuda(device))

@@ -335,6 +335,32 @@ int bnmtf_np_s_update_f64(const double* R, const uint32_t* bits, double* P, int6
  * (predict / compute_I_div, nmf_np.py:122-148).  partials: >= 8*nparts doubles. */
 int bnmtf_np_metrics_f64(const double* R, const uint32_t* bits, const double* P, int64_t rows, int64_t cols, int64_t ld,
                          double* partials, int nparts, double* out8, void* stream);
+/* ---- the same updates on sparse input: the stored entries of a CSR only (csrc/sparse_np.cu) --------------------
+ * Each per-entry operation is the expression of the dense kernels above; no rows x cols array is read or written.
+ * bnmtf_csr_np_row_update_f64: for every row i of the CSR (colidx, val) and k = k0..k1-1 in order:
+ *   A_ik *= sum_j r_ij / p_ij B_jk / sum_j B_jk,  p_ij = A_i . B_j (k ascending, from 0.0), then p_ij += delta B_jk.
+ * A: rows x K, B: cols x K, plain row-major.  Work plan (static, built once per matrix): items in the order n_warp warp
+ * items, n_cta CTA items, then n_c2, n_c4, n_c8, n_c16 items of clusters of 2, 4, 8, 16 CTAs (nc consecutive items per
+ * row, the row's entries split into contiguous ranges in rank order); item t covers entries [item_beg[t], item_end[t]) of
+ * row item_row[t].  Warp items hold at most 256 entries, CTA items at most 2048.  pw: one double per entry of the CSR, the
+ * prediction of the cluster items' entries (scratch; may be NULL without cluster items). */
+int bnmtf_csr_np_row_update_f64(const int64_t* item_beg, const int64_t* item_end, const int32_t* item_row, int64_t n_warp,
+                                int64_t n_cta, int64_t n_c2, int64_t n_c4, int64_t n_c8, int64_t n_c16,
+                                const int32_t* colidx, const double* val, double* A, const double* B, int K, int k0, int k1,
+                                double* pw, void* stream);
+/* NMTF.update_S over the pairs (pairs[2t], pairs[2t+1]), t < n_pairs (device int32), in order, on the training CSR with the
+ * work plan of bnmtf_csr_stats_f64 (item_begin, item_row, chunk): p = FS_i . G_j into pw (nnz doubles), then per pair
+ * S_kl *= sum r F_ik G_jl / p / sum F_ik G_jl and p += (delta F_ik) G_jl.  n_pairs + 1 launches.  FS: rows x L (F S),
+ * F: rows x K, G: cols x L, S: K x L.  partials: >= 4 * nparts + 2 doubles of scratch. */
+int bnmtf_csr_np_s_update_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, const int64_t* item_begin,
+                              const int32_t* item_row, int64_t n_items, int chunk, const double* FS, const double* F, int K,
+                              const double* G, int L, const int32_t* pairs, int n_pairs, double* S, double* pw,
+                              double* partials, int nparts, void* stream);
+/* out8 = the eight sums of bnmtf_np_metrics_f64 over the stored entries of a CSR, p = A_i . B_j computed in place (A: rows
+ * x K, B: cols x K, plain row-major).  A stored zero r gives a NaN I-divergence term (0 log 0), as on dense input.
+ * partials: >= 8 * nparts doubles. */
+int bnmtf_csr_np_metrics_f64(const int64_t* rowptr, const int32_t* colidx, const double* val, int64_t rows, const double* A,
+                             const double* B, int K, double* partials, int nparts, double* out8, void* stream);
 /* C (n x q) = A (n x p) B (p x q), or A B^T with B (q x p) when transB: factor-sized products (S G^T, F S, ...). */
 int bnmtf_small_matmul_f64(const double* A, const double* B, int64_t n, int p, int q, int transB, double* C, void* stream);
 

@@ -45,3 +45,17 @@ m.tau = (m.alpha_s() - 1.0) / m.beta_s()
 m.run(int(g["its"]), minimum_TN=float(g["minimum_TN"]))
 print("toy_nmf_icm    its=%d  MSE %.1e  tau %.1e  U %.1e  V %.1e" % (int(g["its"]), rel(m.all_performances["MSE"], g["trace_MSE"]),
       rel(m.all_tau, g["trace_tau"]), rel(m.U, g["final_U"]), rel(m.V, g["final_V"])))
+g = G("toy_nmf_np")
+m = bnmtf_b200.NMF(g["R"], g["M"], int(g["K"]))
+m.initialise("ones")
+m.U, m.V = g["init_U"].copy(), g["init_V"].copy()
+m.run(int(g["its"]))
+print("toy_nmf_np     its=%d  MSE %.1e  Rp %.1e  U %.1e  V %.1e  Idiv %.1e" % (int(g["its"]), rel(m.all_performances["MSE"], g["trace_MSE"]),
+      rel(m.all_performances["Rp"], g["trace_Rp"]), rel(m.U, g["final_U"]), rel(m.V, g["final_V"]), rel(m.compute_I_div(), g["final_Idiv"])))
+g = G("toy_nmtf_np")
+m = bnmtf_b200.NMTF(g["R"], g["M"], int(g["K"]), int(g["L"]))
+m.initialise("ones", "ones")
+m.F, m.S, m.G = g["init_F"].copy(), g["init_S"].copy(), g["init_G"].copy()
+m.run(int(g["its"]))
+print("toy_nmtf_np    its=%d  MSE %.1e  F %.1e  S %.1e  G %.1e" % (int(g["its"]), rel(m.all_performances["MSE"], g["trace_MSE"]),
+      rel(m.F, g["final_F"]), rel(m.S, g["final_S"]), rel(m.G, g["final_G"])))
