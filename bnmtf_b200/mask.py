@@ -6,6 +6,7 @@ the row-major list of observed positions), so a seeded run produces the same mas
 those calls is vectorised numpy instead of python loops (the reference builds 65536 x 32768 masks entry by entry).
 Reference: code/cross_validation/mask.py:11-174.
 """
+import array
 import random
 
 import numpy as np
@@ -109,6 +110,130 @@ def compute_Ms(folds_M):
     folds = [np.asarray(f) for f in folds_M]
     total = sum(folds)
     return [total - f for f in folds]
+
+
+# ---- sparse input ------------------------------------------------------------------------------------------------
+# The same helpers for a scipy.sparse pattern (see DESIGN.md section 12).  The entries are the stored entries of a
+# canonical CSR (data.canonical_csr, or the CSR of ones data.validate_sparse returns), explicit zeros included; inside the
+# module a set of entries is a bool per stored entry, and the public functions return CSR masks of ones.  Nothing of
+# size I x J is built.  CSR order is row-major, the order of _observed_positions, and random.shuffle's swaps depend
+# only on the length of the list, so shuffling the entry numbers 0..n-1 with the calls the dense helpers make gives the
+# dense helpers' folds and splits on toarray(), bit for bit, and leaves `random` in the same state.
+def _pattern(P):
+    from .data import canonical_csr
+    return canonical_csr(P)
+
+
+def _entry_rows(P):
+    return np.repeat(np.arange(P.shape[0], dtype=np.int64), np.diff(P.indptr))
+
+
+def _entry_mask(P, sel):
+    """CSR of ones at the stored entries of the canonical CSR P where sel (bool per stored entry) is True."""
+    import scipy.sparse as sp
+    I = P.shape[0]
+    indptr = np.concatenate([[0], np.cumsum(np.bincount(_entry_rows(P)[sel], minlength=I))]).astype(np.int64)
+    return sp.csr_matrix((np.ones(int(np.count_nonzero(sel))), P.indices[sel], indptr), shape=P.shape)
+
+
+def _selection(P, M):
+    """Bool per stored entry of P: every entry (M None) or the non-zero entries of the scipy.sparse mask M."""
+    from .data import sparse_selection
+    return np.ones(P.nnz, dtype=bool) if M is None else sparse_selection(P, M)
+
+
+def _shuffled(n):
+    """The permutation random.shuffle applies to a list of length n, as int64 entry numbers.  An array.array of the
+    numbers is shuffled instead of a list: the same calls and swaps, at 8 bytes per entry instead of about 36."""
+    perm = array.array('q', np.arange(n, dtype=np.int64).tobytes())
+    random.shuffle(perm)
+    return np.frombuffer(perm, dtype=np.int64)
+
+
+def _no_empty_lines(P, sel):
+    """check_empty_rows_columns of the entries sel of P: every row and column of P's shape keeps one."""
+    return bool(np.bincount(_entry_rows(P)[sel], minlength=P.shape[0]).all()
+                and np.bincount(P.indices[sel], minlength=P.shape[1]).all())
+
+
+def _fold_selections(P, no_folds, sel):
+    """compute_folds on the entries sel of P: the test entries of each fold, as bool per stored entry of P."""
+    idx = np.flatnonzero(sel)
+    n = idx.size
+    perm = idx[_shuffled(n)]
+    cuts = [int(i * n / no_folds) for i in range(no_folds + 1)]
+    out = []
+    for i in range(no_folds):
+        test = np.zeros(P.nnz, dtype=bool)
+        test[perm[cuts[i]:cuts[i + 1]]] = True
+        out.append(test)
+    return out
+
+
+def _fold_selections_attempts(P, no_folds, attempts, sel):
+    """compute_folds_attempts on the entries sel of P (bool per stored entry of P per fold).  A row or column with
+    fewer than two of those entries can never pass the check, since its entry lands in some fold: the AssertionError is
+    then raised at once, without the attempts (and without drawing from `random`)."""
+    (I, J), rows = P.shape, _entry_rows(P)
+    n_rows, n_cols = np.bincount(rows[sel], minlength=I), np.bincount(P.indices[sel], minlength=J)
+    message = "Failed to generate folds for training and test data, %s attempts." % attempts
+    assert (n_rows >= 2).all() and (n_cols >= 2).all(), message
+    for _ in range(attempts):
+        folds = _fold_selections(P, no_folds, sel)
+        # the training entries of a fold (sel minus the fold) keep every row and column
+        if all((n_rows > np.bincount(rows[test], minlength=I)).all() and
+               (n_cols > np.bincount(P.indices[test], minlength=J)).all() for test in folds):
+            return folds
+    assert False, message
+
+
+def compute_folds_sparse(R, no_folds, M=None):
+    """compute_folds(I, J, no_folds, M) for sparse input: the entries of M (a scipy.sparse mask inside R's pattern; None:
+    every stored entry of R), shuffled and cut into no_folds test masks (CSR of ones)."""
+    P = _pattern(R)
+    return [_entry_mask(P, t) for t in _fold_selections(P, no_folds, _selection(P, M))]
+
+
+def compute_folds_attempts_sparse(R, no_folds, attempts, M=None):
+    """compute_folds_attempts(I, J, no_folds, attempts, M) for sparse input (CSR test masks).  Unlike the dense helper it
+    fails at once, with the same AssertionError, when a row or column of M has fewer than two entries: such a row can
+    never keep an entry in every training mask, and at 10^8 entries each of the 1000 attempts costs a python shuffle."""
+    P = _pattern(R)
+    return [_entry_mask(P, t) for t in _fold_selections_attempts(P, no_folds, attempts, _selection(P, M))]
+
+
+def compute_Ms_sparse(folds_M):
+    """compute_Ms for scipy.sparse folds: the training mask of each fold, the sum of the other folds (CSR)."""
+    import scipy.sparse as sp
+    folds = [sp.csr_matrix(f, dtype=float) for f in folds_M]
+    total = folds[0]
+    for f in folds[1:]:
+        total = total + f
+    return [(total - f).tocsr() for f in folds]
+
+
+def generate_M_from_M_sparse(M, fraction):
+    """generate_M_from_M for a sparse pattern M (every stored entry observed): (M_train, M_test) as CSR masks, so that
+    `fraction` of ALL I x J entries is missing from M_train."""
+    P = _pattern(M)
+    I, J = P.shape
+    missing = I * J - P.nnz
+    assert missing < I * J * fraction, \
+        "Specified %s fraction missing, so %s entries missing, but there are already %s missing by default!" % \
+        (fraction, I * J * fraction, missing)
+    perm = _shuffled(P.nnz)
+    train = np.zeros(P.nnz, dtype=bool)
+    train[perm[:int(I * J * (1 - fraction))]] = True
+    return _entry_mask(P, train), _entry_mask(P, ~train)
+
+
+def try_generate_M_from_M_sparse(M, fraction, attempts):
+    """try_generate_M_from_M for a sparse pattern M (CSR masks)."""
+    for _ in range(attempts):
+        M_train, M_test = generate_M_from_M_sparse(M, fraction)
+        if _no_empty_lines(M_train, np.ones(M_train.nnz, dtype=bool)):
+            return M_train, M_test
+    assert False, "Failed to generate folds for training and test data, %s attempts, fraction %s." % (attempts, fraction)
 
 
 def calc_inverse_M(M):

@@ -143,16 +143,117 @@ def _quality_args(burn_in, thinning):
     return (burn_in, thinning) if burn_in is not None and thinning is not None else ()
 
 
+# ---- sparse input (DESIGN.md section 12) ------------------------------------------------------------------------
+class _Entries:
+    """A training set of sparse input: R's canonical CSR `Rc` and a bool per stored entry of it (`train`).  The fits of
+    this package's model classes on it are built with from_dataset on one shared engine.SparseDataset per CUDA device,
+    made on first use and dropped by release(); any other classifier gets its constructor with (Rc, a CSR mask)."""
+
+    def __init__(self, Rc, train):
+        self.Rc, self.train = Rc, train
+        self._ds, self._mask = {}, None
+
+    def mask(self):
+        if self._mask is None:
+            self._mask = mask._entry_mask(self.Rc, self.train)
+        return self._mask
+
+    def dataset(self):
+        """The SparseDataset of these entries on the calling thread's current device."""
+        from .engine import SparseDataset, require_cuda
+        dev = require_cuda()
+        if dev.index not in self._ds:
+            self._ds[dev.index] = SparseDataset(self.Rc, self.train, dev)
+        return self._ds[dev.index]
+
+    def release(self):
+        self._ds.clear()
+
+    def construct(self, classifier, *args, **kwargs):
+        """classifier(R, M, *args, **kwargs) on these entries."""
+        from .bnmf import _TwoFactorBase
+        from .bnmtf import _ThreeFactorBase
+        from .np_models import _NPBase
+        if isinstance(classifier, type) and issubclass(classifier, _NPBase):
+            return classifier.from_dataset(self.dataset(), *args, **kwargs)
+        if isinstance(classifier, type) and issubclass(classifier, (_TwoFactorBase, _ThreeFactorBase)):
+            model = classifier.from_dataset(self.dataset(), *args, seed=0, **kwargs)
+            model._seed_after_initialise = True          # see _seeded
+            return model
+        return classifier(self.Rc, self.mask(), *args, **kwargs)
+
+
+def _seeded(model):
+    """from_dataset() fixes a model's Philox seed when it is called, while a model built by its constructor derives the
+    seed from numpy's state when initialise() first reaches the device, after its host draws.  For a model from
+    _Entries.construct, derive it now, after initialise(): a seeded Gibbs fit then draws what it draws on dense input."""
+    if model.__dict__.pop('_seed_after_initialise', False):
+        from . import _lib
+        model._seed = model._eng.seed = _lib.derive_seed()
+    return model
+
+
+def _sparse_entries(R, M, validate):
+    """The training set of (R, M) as an _Entries (M may be one already: a fold handed down by a cross-validation driver),
+    or None for dense input.  validate: the model classes' checks (data.validate_sparse), which dense input meets in the
+    constructor of every fit."""
+    import scipy.sparse as sp
+    from . import data
+    if isinstance(M, _Entries):
+        return M
+    if not sp.issparse(R):
+        if sp.issparse(M):
+            raise ValueError("with dense R, M must be a dense array, not %s" % type(M).__name__)
+        return None
+    if validate:
+        Rc, _, train = data.validate_sparse(R, M)
+        return _Entries(Rc, train)
+    if M is not None and not sp.issparse(M):
+        raise ValueError("with sparse R, M must be None or a scipy.sparse matrix, not %s" % type(M).__name__)
+    Rc = data.canonical_csr(R)
+    return _Entries(Rc, mask._selection(Rc, M))
+
+
+def _as_entries(entries, train):
+    """A training set given to a run_model() method: a dense mask as it is, a sparse one as an _Entries."""
+    if entries is None or isinstance(train, _Entries):
+        return train
+    return _Entries(entries.Rc, mask._selection(entries.Rc, train))
+
+
+def _cv_folds(entries, I, J, no_folds, M):
+    """[(training set, test mask)] of the cross-validation drivers: the reference's compute_folds_attempts and
+    compute_Ms for dense input; for sparse input an _Entries per fold and a CSR test mask, the same folds."""
+    if entries is None:
+        folds_test = mask.compute_folds_attempts(I=I, J=J, no_folds=no_folds, attempts=attempts_generate_M, M=M)
+        return list(zip(mask.compute_Ms(folds_test), folds_test))
+    tests = mask._fold_selections_attempts(entries.Rc, no_folds, attempts_generate_M, entries.train)
+    return [(_Entries(entries.Rc, entries.train & ~t), mask._entry_mask(entries.Rc, t)) for t in tests]
+
+
 class _Search:
     """Shared machinery of the three searches: fit `restarts` models per point, keep the one with the highest
-    log-likelihood, record every metric of that one."""
+    log-likelihood, record every metric of that one.  Sparse R: every fit shares one resident dataset of M's entries."""
 
     def __init__(self, classifier, R, M, priors, iterations, restarts, devices):
+        self.entries = _sparse_entries(R, M, validate=True)
+        self._own_entries = not isinstance(M, _Entries)
+        if self.entries is not None:
+            R = self.entries.Rc
         self.classifier, self.R, self.M, self.priors = classifier, R, M, priors
         (self.I, self.J) = self.R.shape
         self.iterations, self.restarts = iterations, restarts
         assert self.restarts > 0, "Need at least 1 restart."
         self.pool = DevicePool(devices)
+
+    def _new(self, *args):
+        if self.entries is None:
+            return self.classifier(self.R, self.M, *args)
+        return self.entries.construct(self.classifier, *args)
+
+    def _done(self):
+        if self.entries is not None and self._own_entries:
+            self.entries.release()
 
     def _build(self, point):       # -> model, constructed and initialised
         raise NotImplementedError
@@ -221,14 +322,15 @@ class LineSearch(_Search):
         self.all_performances = {metric: [] for metric in metrics}
 
     def _build(self, K):
-        model = self.classifier(self.R, self.M, K, self.priors)
+        model = self._new(K, self.priors)
         model.initialise(init=self.initUV)
-        return model
+        return _seeded(model)
 
     def search(self, burn_in=None, thinning=None, minimum_TN=None):
         for res in self._evaluate(self.values_K, burn_in, thinning, minimum_TN):
             for metric in metrics:
                 self.all_performances[metric].append(res[metric])
+        self._done()
 
     def best_value(self, metric):
         values = self.all_values(metric)
@@ -250,9 +352,9 @@ class GridSearch(_Search):
         priors['lambdaF'] = self.priors['lambdaF'] * np.ones((self.I, K))
         priors['lambdaS'] = self.priors['lambdaS'] * np.ones((K, L))
         priors['lambdaG'] = self.priors['lambdaG'] * np.ones((self.J, L))
-        model = self.classifier(self.R, self.M, K, L, priors)
+        model = self._new(K, L, priors)
         model.initialise(init_S=self.initS, init_FG=self.initFG)
-        return model
+        return _seeded(model)
 
     def search(self, burn_in=None, thinning=None):
         points = [(K, L) for K in self.values_K for L in self.values_L]
@@ -261,6 +363,7 @@ class GridSearch(_Search):
             ik, il = divmod(idx, len(self.values_L))
             for metric in metrics:
                 self.all_performances[metric][ik, il] = res[metric]
+        self._done()
 
     def best_value(self, metric):
         index = int(np.argmin(self.all_values(metric)))
@@ -280,9 +383,9 @@ class GreedySearch(_Search):
         self.all_performances = {metric: [] for metric in metrics}
 
     def _build(self, KL):
-        model = self.classifier(self.R, self.M, KL[0], KL[1], self.priors)
+        model = self._new(KL[0], KL[1], self.priors)
         model.initialise(init_S=self.initS, init_FG=self.initFG)
-        return model
+        return _seeded(model)
 
     def find_KL(self, metric, K, L):
         return [x for x in self.all_values(metric) if (x[0], x[1]) == (K, L)]
@@ -331,6 +434,7 @@ class GreedySearch(_Search):
                 # LAST L-direction score of the main loop, not the score just accepted.  Kept, so that the walk visits
                 # the same points; where the reference would hit an unbound name (main loop never ran) use p_K.
                 so_far = p_K if p_L is None else p_L
+        self._done()
 
     def best_value(self, metric):
         (best_K, best_L, _) = min(self.all_values(metric), key=lambda x: x[2])
@@ -344,13 +448,18 @@ class _SearchCrossValidation:
 
     def __init__(self, classifier, R, M, folds, priors, iterations, restarts, quality_metric, file_performance, devices):
         self.classifier = classifier
-        self.R = np.array(R, dtype=float)
-        self.M = np.array(M)
+        self.entries = _sparse_entries(R, M, validate=False)
+        if self.entries is None:
+            self.R = np.array(R, dtype=float)
+            self.M = np.array(M)
+        else:
+            self.R, self.M = self.entries.Rc, M
         self.folds, self.priors, self.iterations, self.restarts = folds, priors, iterations, restarts
         self.quality_metric = quality_metric
         self.fout = open(file_performance, 'w')
         (self.I, self.J) = self.R.shape
-        assert (self.R.shape == self.M.shape), "R and M are of different shapes: %s and %s respectively." % (self.R.shape, self.M.shape)
+        if self.entries is None:
+            assert (self.R.shape == self.M.shape), "R and M are of different shapes: %s and %s respectively." % (self.R.shape, self.M.shape)
         assert self.quality_metric in metrics
         self.performances = {}
         self.devices = devices
@@ -366,10 +475,8 @@ class _SearchCrossValidation:
     _best_label = "K"
 
     def run(self, burn_in=None, thinning=None, minimum_TN=None):
-        folds_test = mask.compute_folds_attempts(I=self.I, J=self.J, no_folds=self.folds, attempts=attempts_generate_M, M=self.M)
-        folds_training = mask.compute_Ms(folds_test)
         performances_test = {measure: [] for measure in measures}
-        for i, (train, test) in enumerate(zip(folds_training, folds_test)):
+        for i, (train, test) in enumerate(_cv_folds(self.entries, self.I, self.J, self.folds, self.M)):
             all_performances, best = self._select(train, burn_in, thinning, minimum_TN)
             self.fout.write("All model fits for fold %s, metric %s: %s.\n" % (i + 1, self.quality_metric, all_performances))
             self.fout.flush()
@@ -379,6 +486,10 @@ class _SearchCrossValidation:
             self.fout.flush()
             for measure in measures:
                 performances_test[measure].append(performance[measure])
+            if self.entries is not None:
+                train.release()
+        if self.entries is not None:
+            self.entries.release()
         self.average_performance_test = self.compute_average_performance(performances_test)
         self.performances = performances_test
         self.fout.write("Average performance: %s. \nPerformances test: %s." % (self.average_performance_test, performances_test))
@@ -389,6 +500,7 @@ class _SearchCrossValidation:
 
     def _run_final(self, train, test, point, burn_in, thinning, minimum_TN):
         qa = _quality_args(burn_in, thinning)
+        train = _as_entries(self.entries, train)
 
         def fit(model):
             if minimum_TN is None:
@@ -427,9 +539,12 @@ class LineSearchCrossValidation(_SearchCrossValidation):
         return ls.all_values(metric=self.quality_metric), ls.best_value(metric=self.quality_metric)
 
     def _final_model(self, train, K):
-        model = self.classifier(R=self.R, M=train, K=K, priors=self.priors)
+        if isinstance(train, _Entries):
+            model = train.construct(self.classifier, K=K, priors=self.priors)
+        else:
+            model = self.classifier(R=self.R, M=train, K=K, priors=self.priors)
         model.initialise(self.init_UV)
-        return model
+        return _seeded(model)
 
     def run_model(self, train, test, K, burn_in=None, thinning=None, minimum_TN=None):
         return self._run_final(train, test, K, burn_in, thinning, minimum_TN)
@@ -446,16 +561,20 @@ class GreedySearchCrossValidation(_SearchCrossValidation):
 
     def _select(self, train, burn_in, thinning, minimum_TN):
         # the reference passes M=self.M (the full mask), not the training fold (greedy_search_cross_validation.py:72): kept
-        gs = GreedySearch(classifier=self.classifier, values_K=self.values_K, values_L=self.values_L, R=self.R, M=self.M,
+        gs = GreedySearch(classifier=self.classifier, values_K=self.values_K, values_L=self.values_L, R=self.R,
+                          M=self.M if self.entries is None else self.entries,
                           priors=self.priors, initS=self.init_S, initFG=self.init_FG, iterations=self.iterations,
                           restarts=self.restarts, devices=self.devices)
         gs.search(self.quality_metric, burn_in=burn_in, thinning=thinning, minimum_TN=minimum_TN)
         return gs.all_values(metric=self.quality_metric), gs.best_value(metric=self.quality_metric)
 
     def _final_model(self, train, KL):
-        model = self.classifier(R=self.R, M=train, K=KL[0], L=KL[1], priors=self.priors)
+        if isinstance(train, _Entries):
+            model = train.construct(self.classifier, K=KL[0], L=KL[1], priors=self.priors)
+        else:
+            model = self.classifier(R=self.R, M=train, K=KL[0], L=KL[1], priors=self.priors)
         model.initialise(self.init_S, self.init_FG)
-        return model
+        return _seeded(model)
 
     def run_model(self, train, test, K, L, burn_in=None, thinning=None, minimum_TN=None):
         return self._run_final(train, test, (K, L), burn_in, thinning, minimum_TN)
@@ -464,6 +583,13 @@ class GreedySearchCrossValidation(_SearchCrossValidation):
 # ---------------------------------------------------------------------------------------------------------------
 def _fit_fold(job):
     method, X, train, test, parameters, train_config = job
+    if isinstance(train, _Entries):          # sparse input: the fold's own dataset, released when its fit is done
+        try:
+            model = _seeded(train.construct(method, **parameters))     # (counts the seed as dense input does)
+            model.train(**train_config)
+            return model.predict(test)
+        finally:
+            train.release()
     model = method(X, train, **parameters)
     model.train(**train_config)
     return model.predict(test)
@@ -476,12 +602,17 @@ class MatrixCrossValidation:
 
     def __init__(self, method, X, M, K, parameter_search, train_config, file_performance, devices=1):
         self.method = method
-        self.X = np.array(X, dtype=float)
-        self.M = np.array(M)
+        self.entries = _sparse_entries(X, M, validate=False)
+        if self.entries is None:
+            self.X = np.array(X, dtype=float)
+            self.M = np.array(M)
+        else:
+            self.X, self.M = self.entries.Rc, M
         self.K, self.train_config, self.parameter_search = K, train_config, parameter_search
         self.fout = open(file_performance, 'w')
         (self.I, self.J) = self.X.shape
-        assert (self.X.shape == self.M.shape), "X and M are of different shapes: %s and %s respectively." % (self.X.shape, self.M.shape)
+        if self.entries is None:
+            assert (self.X.shape == self.M.shape), "X and M are of different shapes: %s and %s respectively." % (self.X.shape, self.M.shape)
         self.all_performances = {}        # JSON(parameters) -> {criterion: [per fold]}
         self.average_performances = {}    # JSON(parameters) -> {criterion: average}
         self.performances = {}            # criterion -> [average per parameter setting]
@@ -490,11 +621,9 @@ class MatrixCrossValidation:
     def run(self):
         for parameters in self.parameter_search:
             try:
-                folds_test = mask.compute_folds_attempts(I=self.I, J=self.J, no_folds=self.K, attempts=attempts_generate_M, M=self.M)
-                folds_training = mask.compute_Ms(folds_test)
+                folds = _cv_folds(self.entries, self.I, self.J, self.K, self.M)
                 self.all_performances[self.JSON(parameters)] = {}
-                jobs = [(self.method, self.X, train, test, parameters, self.train_config)
-                        for train, test in zip(folds_training, folds_test)]
+                jobs = [(self.method, self.X, train, test, parameters, self.train_config) for train, test in folds]
                 for performance_dict in self.pool.map(_fit_fold, jobs):
                     self.store_performances(performance_dict, parameters)
                 self.log(parameters)
@@ -503,7 +632,7 @@ class MatrixCrossValidation:
                 self.fout.flush()
 
     def run_model(self, train, test, parameters):
-        return _fit_fold((self.method, self.X, train, test, parameters, self.train_config))
+        return _fit_fold((self.method, self.X, _as_entries(self.entries, train), test, parameters, self.train_config))
 
     def JSON(self, d):
         return json.dumps({k: (v.tolist() if isinstance(v, np.ndarray) else v) for k, v in d.items()}, sort_keys=True)
@@ -557,20 +686,23 @@ class MatrixNestedCrossValidation:
 
     def __init__(self, method, X, M, K, P, parameter_search, train_config, file_performance, files_nested_performances):
         self.method = method
-        self.X = np.array(X, dtype=float)
-        self.M = np.array(M)
+        self.entries = _sparse_entries(X, M, validate=False)
+        if self.entries is None:
+            self.X = np.array(X, dtype=float)
+            self.M = np.array(M)
+        else:
+            self.X, self.M = self.entries.Rc, M
         self.K, self.P, self.train_config, self.parameter_search = K, P, train_config, parameter_search
         self.files_nested_performances = files_nested_performances
         self.fout = open(file_performance, 'w')
         (self.I, self.J) = self.X.shape
-        assert (self.X.shape == self.M.shape), "X and M are of different shapes: %s and %s respectively." % (self.X.shape, self.M.shape)
+        if self.entries is None:
+            assert (self.X.shape == self.M.shape), "X and M are of different shapes: %s and %s respectively." % (self.X.shape, self.M.shape)
         self.all_performances = {}
         self.average_performances = {}
 
     def run(self):
-        folds_test = mask.compute_folds_attempts(I=self.I, J=self.J, no_folds=self.K, attempts=attempts_generate_M, M=self.M)
-        folds_training = mask.compute_Ms(folds_test)
-        for i, (train, test) in enumerate(zip(folds_training, folds_test)):
+        for i, (train, test) in enumerate(_cv_folds(self.entries, self.I, self.J, self.K, self.M)):
             crossval = ParallelMatrixCrossValidation(method=self.method, X=self.X, M=train, K=self.K,
                                                      parameter_search=self.parameter_search, train_config=self.train_config,
                                                      file_performance=self.files_nested_performances[i], P=self.P)
@@ -584,7 +716,7 @@ class MatrixNestedCrossValidation:
         self.log()
 
     def run_model(self, train, test, parameters):
-        return _fit_fold((self.method, self.X, train, test, parameters, self.train_config))
+        return _fit_fold((self.method, self.X, _as_entries(self.entries, train), test, parameters, self.train_config))
 
     def store_performances(self, performance_dict):
         for name, value in performance_dict.items():
