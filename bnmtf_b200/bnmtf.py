@@ -180,7 +180,7 @@ class BNMTFEngine:
 
             def gram():
                 _lib.call("bnmtf_stats_gram_umma_f64", _ptr(bits), rows, ld, other.n, _ptr(other.Xp), _ptr(other.Vp), dim,
-                          self.polarity, 1, 128 if ld >= 256 else 64, 1, sums, 0, _ptr(st["G"]), _ptr(st["SV"]) if self.vb else 0,
+                          self.polarity, 1, 128 if ld >= 256 else 64, sums, _ptr(st["G"]), _ptr(st["SV"]) if self.vb else 0,
                           self.ws_ptr, self.ws_bytes, _stream())
             split = self.split(dim)
             if need_rx and split > 0:

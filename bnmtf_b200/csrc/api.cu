@@ -40,9 +40,8 @@ int launch_stats_rx_umma(const uint8_t*, const double*, const double*, const uin
 int launch_stats_gram(const uint32_t*, int, int, const double*, const double*, int, int, int, double*, double*, const int*, cudaStream_t);
 int launch_gram_full(const double*, const double*, int, int, int, double*, double*, cudaStream_t);
 long long umma_workspace_bytes(int, int, long long);
-int launch_stats_gram_fixup(const uint32_t*, int, int, int, const double*, const double*, int, int, double*, double*, cudaStream_t);
-int launch_stats_gram_umma(const uint32_t*, int, int, int, const double*, const double*, int, int, int, int, int, int, int,
-                           double*, double*, void*, long long, cudaStream_t);
+int launch_stats_gram_umma(const uint32_t*, int, int, int, const double*, const double*, int, int, int, int, int, double*,
+                           double*, void*, long long, cudaStream_t);
 int launch_pad_factor(const double*, const double*, int, int, int, double*, double*, cudaStream_t);
 int launch_masked_metrics(const double*, const uint32_t*, int, int, const double*, const double*, int, int, const double*, double*, double*, const int*, cudaStream_t);
 int launch_mstat_reduce(const double*, int, double*, double*, cudaStream_t);
@@ -177,7 +176,7 @@ using namespace bnmtf;
 
 extern "C" {
 
-int bnmtf_version(void) { return 100; }
+int bnmtf_version(void) { return 101; }
 const char* bnmtf_last_error(void) { return g_err; }
 int64_t bnmtf_ld_for(int64_t cols) { return round_up64(cols, 64); }
 int bnmtf_kp_for(int K) { return 8 * tiles_for(K); }
@@ -371,26 +370,18 @@ int bnmtf_csr_kmeans_sums_f64(const int64_t* coordptr, const int32_t* point, con
   return launch_kmeans_csr_sums(coordptr, point, val, d, assign, K, only, sums, counts, ST(stream));
 }
 
-int bnmtf_stats_gram_fixup_f64(const uint32_t* bits, int64_t rows, int64_t ld, int64_t cols, const double* Xp, const double* Vp,
-                               int K, int polarity, double* Gseg, double* SVseg, void* stream) {
-  if (check_k(K)) return -2;
-  if ((Vp == nullptr) != (SVseg == nullptr)) { set_error("stats_gram_fixup: Vp and SVseg must be given together"); return -2; }
-  return launch_stats_gram_fixup(bits, (int)rows, (int)ld, (int)cols, Xp, Vp, K, polarity, Gseg, SVseg, ST(stream));
-}
-
 int64_t bnmtf_gram_umma_workspace_bytes(int K, int vb, int64_t ld) {
   if (K < 1 || K > 63 || ld <= 0) return -1;
   return umma_workspace_bytes(K, vb, ld);
 }
 
 int bnmtf_stats_gram_umma_f64(const uint32_t* bits, int64_t rows, int64_t ld, int64_t cols, const double* Xp,
-                              const double* Vp, int K, int polarity, int nseg, int tile, int pair, int sums,
-                              int max_stages, double* Gpart, double* SVpart, void* workspace, int64_t workspace_bytes,
-                              void* stream) {
+                              const double* Vp, int K, int polarity, int nseg, int tile, int sums, double* Gpart,
+                              double* SVpart, void* workspace, int64_t workspace_bytes, void* stream) {
   if (check_k(K)) return -2;
   if ((Vp == nullptr) != (SVpart == nullptr)) { set_error("stats_gram_umma: Vp and SVpart must be given together"); return -2; }
-  return launch_stats_gram_umma(bits, (int)rows, (int)ld, (int)cols, Xp, Vp, K, polarity, nseg, tile, pair, sums,
-                                max_stages, Gpart, SVpart, workspace, workspace_bytes, ST(stream));
+  return launch_stats_gram_umma(bits, (int)rows, (int)ld, (int)cols, Xp, Vp, K, polarity, nseg, tile, sums, Gpart, SVpart,
+                                workspace, workspace_bytes, ST(stream));
 }
 
 int bnmtf_gram_full_f64(const double* Xp, const double* Vp, int64_t n, int K, int64_t dummy_row, double* Gfull,

@@ -224,21 +224,4 @@ __device__ __forceinline__ double tn_draw(double mu, double tau, Philox& rng) {
 }
 #endif  // __CUDACC__
 
-// 2:4 split of 32 selection bits = eight groups of four columns (one nibble each, computed for all eight at once).
-// Per group: idx0 < idx1 are the positions of the first two selected columns (idx1 = 3 / idx0 = 0 when there are
-// fewer), v0 / v1 (bit 4g) say whether the column at idx0 / idx1 is selected, meta holds idx0 | idx1 << 2 in nibble g.
-// Returns the selected columns that do NOT fit (the third and fourth of a group): the fix-up kernel's share.
-__host__ __device__ __forceinline__ uint32_t sparse_split(uint32_t v, uint32_t& v0, uint32_t& v1, uint32_t& meta) {
-  const uint32_t m = 0x11111111u;
-  const uint32_t b0 = v & m, b1 = (v >> 1) & m, b2 = (v >> 2) & m, b3 = (v >> 3) & m;
-  const uint32_t c1 = b0 & b1;              // second selected column at position 1
-  const uint32_t c2 = (b0 ^ b1) & b2;       // ... at position 2
-  const uint32_t i0b0 = b1 & ~b0, i0b1 = b2 & ~(b0 | b1);
-  meta = i0b0 | (i0b1 << 1) | ((m & ~c2) << 2) | ((m & ~c1) << 3);
-  v0 = b0 | b1 | b2;
-  v1 = c1 | c2 | (b3 & ~(c1 | c2));
-  return ((c1 & b2) << 2) | ((b3 & (c1 | c2)) << 3);
-}
-
-
 }  // namespace bnmtf

@@ -38,34 +38,31 @@ constexpr int UG_THREADS = (UG_EXP_WARPS + 3) * 32;   // + TMA producer of the d
 constexpr int UG_MASK_BUFS = 3;      // mask windows in flight
 
 struct UmmaPlan {
-  int K, vb, sums, sp;
-  int nh_full;  // UMMA N of each accumulator of a full chunk (256; 240 in the 2:4-sparse form, which keeps 32 columns for the metadata)
+  int K, vb, sums;
+  int nh_full;  // UMMA N of each accumulator of a full chunk (256)
   int ng;       // K(K+1)/2 Gram columns
   int nc;       // ng (+K variance columns) (+K plain columns X_jk: masked column sums, for the metrics)
   int nch;      // chunks: all but the last hold cpc P-columns in two accumulators of 256 tensor-memory columns
   int cpc;      // P-columns per full chunk: 512 / kDigits (85 with six digits)
   int cpc_last; // P-columns of the last chunk
-  int nh_last;  // UMMA N of each accumulator of the last chunk (multiple of 32 for CTA pairs, else 16; <= 256)
-  int gran;
+  int nh_last;  // UMMA N of each accumulator of the last chunk (multiple of 32: each CTA of the pair holds n_half/2 digit rows; <= 256)
 };
 constexpr int UG_CHUNK_ROWS = 512;   // digit rows reserved per chunk in the staged B matrix
-constexpr int UG_SP_ACC_COLS = 480;  // 2:4-sparse form: tensor-memory columns of the accumulators; [480, 512) hold the metadata
 
 // Chunks are UNEVEN: 210 products x 6 digits = 1260 digit columns run as 512 + 512 + 256 tensor-memory columns (three
 // equal chunks of 70 products would need 3 x 448; with the K column sums / VB variances 3 x 512 instead of 512 + 512 +
 // 384): the MMA work follows the columns actually needed.
-__host__ __device__ inline UmmaPlan make_umma_plan(int K, int vb, int sums, int pair, int sp = 0) {
+__host__ __device__ inline UmmaPlan make_umma_plan(int K, int vb, int sums) {
   UmmaPlan p;
-  p.K = K; p.vb = vb; p.sums = sums; p.sp = sp;
+  p.K = K; p.vb = vb; p.sums = sums;
   p.ng = K * (K + 1) / 2;
   p.nc = p.ng + (vb ? K : 0) + (sums ? K : 0);
-  p.cpc = (sp ? UG_SP_ACC_COLS : 512) / UG_SLICES;      // 85 (73 with seven digits); sparse: 80 (68)
+  p.cpc = 512 / UG_SLICES;                   // 85 (73 with seven digits)
   p.nh_full = ((p.cpc * UG_SLICES + 1) / 2 + 15) / 16 * 16;
   p.nch = (p.nc + p.cpc - 1) / p.cpc;
   p.cpc_last = p.nc - (p.nch - 1) * p.cpc;
-  p.gran = (pair && !sp) ? 32 : 16;          // UMMA N granularity (CTA pair: each CTA holds n_half/2 digit rows)
   const int nd = p.cpc_last * UG_SLICES;
-  p.nh_last = ((nd + 1) / 2 + p.gran - 1) / p.gran * p.gran;
+  p.nh_last = ((nd + 1) / 2 + 31) / 32 * 32;
   return p;
 }
 __host__ __device__ inline int umma_cols_of(const UmmaPlan& p, int ch) { return ch == p.nch - 1 ? p.cpc_last : p.cpc; }
@@ -222,28 +219,13 @@ struct UmmaGramArgs {
   int KP, gl;       // padded factor width, doubles per Gram record (NTP*64)
   int mask_tma;     // mask words arrive through TMA windows (needs ld % 128 == 0: a 16-byte row pitch); else direct loads
   int stages_of[2]; // pipeline depth of the full chunks / of the last chunk (its stages are smaller)
-  int dbg;   // timing experiments only: 1 = skip TMA loads after the first fill, 2 = skip the A-tile stores
 };
 
-// PAIR: two CTAs of a cluster (adjacent row blocks, same chunk and segment) run every MMA as one cta_group::2
-// instruction of M = 256: each CTA expands its own 128 mask rows and loads only HALF of the digit rows of each
-// accumulator (the hardware reads the other half from the partner's shared memory), which halves the shared-memory
-// and L2 traffic per MMA -- the limit of the single-CTA form.
-//
-// SP: the 2:4-sparse form (tcgen05.mma.sp).  W is the 0/1 indicator of a set that holds ~20 % of the entries, so in
-// most groups of four consecutive columns at most two are selected: the A operand is stored compressed (two value
-// bytes per group of four columns, 64 bytes per row and 128-column stage) with its metadata (two 2-bit column indices
-// per group, idx0 < idx1) in tensor memory -- lane = row, one 32-bit column per 32 logical columns, written by the
-// expander threads with tcgen05.st -- and one MMA covers K = 64 logical columns in the time of a dense K = 32.  The
-// third and fourth selected entries of a group (0.7 % of the entries at 20 %) are left out here (sparse_overflow()
-// is the rule) and added by k_gram_fixup as one more segment of the partial statistics.
-//
-// MC: clusters of FOUR CTAs = two CTA pairs (four adjacent row blocks, same chunk and segment) share every digit tile:
-// each CTA fetches ONE of the two boxes its position in the pair needs and multicasts it into the shared memory of
-// the CTA with the same position in the other pair, which halves the L2 -> SM traffic of the digit rows (12 GB per
-// launch at the headline shape; measured: that traffic, not the tensor pipe, bounds the kernel).  A stage is free
-// when BOTH pairs have consumed it (their commits arrive at all four CTAs).
-template <int KT, bool PAIR, bool SP, bool MC>
+// Every MMA runs on a CTA pair: the two CTAs of a cluster (adjacent row blocks, same chunk and segment) issue it as one
+// cta_group::2 instruction of M = 256.  Each CTA expands its own 128 mask rows and loads only HALF of the digit rows of
+// each accumulator (the hardware reads the other half from the partner's shared memory), which halves the shared-memory
+// and L2 traffic per MMA -- the limit of a single-CTA form.
+template <int KT>
 __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_constant__ CUtensorMap tmap_full,
                                                             const __grid_constant__ CUtensorMap tmap_last,
                                                             const __grid_constant__ CUtensorMap tmap_bits, UmmaGramArgs a) {
@@ -251,16 +233,11 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const UmmaPlan& pl = a.pl;
-  static_assert(!MC || PAIR, "the multicast form is built on CTA pairs");
-  const uint32_t crank = PAIR ? cluster_ctarank() : 0u;     // rank in the cluster (0..3 with MC)
-  const uint32_t rank = crank & 1u;                         // position in the CTA pair (0: leader, issues the MMAs)
-  const uint32_t lead = crank & ~1u;                        // cluster rank of this pair's leader
+  const uint32_t rank = cluster_ctarank();                  // position in the CTA pair (0: leader, issues the MMAs)
   const int rb = blockIdx.x, ch = blockIdx.y, seg = blockIdx.z;
   const int n_half = umma_nhalf_of(pl, ch), cpc = umma_cols_of(pl, ch);       // this chunk: UMMA N per accumulator, P-columns
   const CUtensorMap& tmap = ch == pl.nch - 1 ? tmap_last : tmap_full;           // box height = this chunk's digit rows per load
-  constexpr int AKT = SP ? KT / 2 : KT;                 // bytes per row of an A tile
-  static_assert(!SP || KT == 128, "the sparse form runs 128-column stages");
-  const int A_BYTES = UG_ROWS * AKT, B_BYTES = (PAIR ? n_half : 2 * n_half) * KT, STAGE = A_BYTES + B_BYTES;
+  const int A_BYTES = UG_ROWS * KT, B_BYTES = n_half * KT, STAGE = A_BYTES + B_BYTES;
   const int stages = ch == pl.nch - 1 ? a.stages_of[1] : a.stages_of[0];    // (no dynamic index into the parameter struct)
   // mask windows: the bit words of the CTA's 128 rows x 512 columns (16 words = 64 bytes per row, 64-byte swizzle) arrive
   // through TMA (a warp of its own, UG_MASK_BUFS windows in flight: never in the way of the digit tiles).  (A thread per row reading its own words from global memory costs one L1
@@ -285,23 +262,18 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
   const int ntile = kt_end - kt_begin;                 // >= 1 by construction of the grid
 
   if (warp == UG_EXP_WARPS && lane == 0) {
-    // full: every local expander thread + the TMA thread (+, CTA pair, leader: the partner's relay thread; the
-    // partner's own full barrier only collects its expanders)
-    const uint32_t nfull = 4u + (PAIR ? (rank == 0 ? 2u : 0u) : 1u);     // the four warps of the group that expands the stage
-    for (int s = 0; s < stages; ++s) { mbar_init(FULL_BAR(s), nfull); mbar_init(EMPTY_BAR(s), MC ? 2 : 1); }
+    // full: the four warps of the group that expands the stage (+, leader: the TMA thread and the partner's relay
+    // thread; the partner's own full barrier only collects its expanders)
+    const uint32_t nfull = 4u + (rank == 0 ? 2u : 0u);
+    for (int s = 0; s < stages; ++s) { mbar_init(FULL_BAR(s), nfull); mbar_init(EMPTY_BAR(s), 1); }
     mbar_init(ACCUM_BAR, 1);
     for (int b = 0; b < UG_MASK_BUFS; ++b) { mbar_init(MASK_FULL(b), 1); mbar_init(MASK_EMPTY(b), 4 * (stages < UG_GROUPS ? stages : UG_GROUPS)); }
     fence_barrier_init();
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap) : "memory");
   }
   if (warp == UG_EXP_WARPS + 1) {
-    if (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
   for (int cl = tid; cl < cpc; cl += UG_THREADS) {
     const int c = ch * pl.cpc + cl;
@@ -310,7 +282,7 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
     pair_tab[cl] = (uint16_t)((pa << 8) | pb);
   }
   tc_fence_before();
-  if (PAIR) cluster_sync_all(); else __syncthreads();      // barriers of BOTH CTAs are initialised before any remote arrive
+  cluster_sync_all();                                      // barriers of BOTH CTAs are initialised before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -318,7 +290,7 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
     // ================= mask expanders, then epilogue =================
     // UG_GROUPS groups of 128 threads (thread <-> row) take the pipeline stages in turn: the per-stage chain of one group
     // (barrier wake-up, stores, proxy fence, arrive) overlaps the bit expansion of the others, and every scheduler has
-    // several expander warps to pick from (with two groups the expanders' own issue rate bounded the sparse form)
+    // several expander warps to pick from
     const int r = tid & (UG_ROWS - 1), half = tid >> 7;
     const int row = rb * UG_ROWS + r;
     const bool live = row < a.rows;
@@ -330,9 +302,8 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
     const int NG = stages < UG_GROUPS ? stages : UG_GROUPS;
     const uint32_t flip = a.polarity ? 0u : 0xffffffffu;
     // byte offset of this row inside an A tile, and its swizzle key (16-byte chunk index XOR)
-    const uint32_t row_off = (uint32_t)(r >> 3) * (8 * AKT) + (uint32_t)(r & 7) * AKT;
-    const uint32_t key = AKT == 128 ? (uint32_t)(r & 7) : (uint32_t)((r >> 1) & 3);
-    const uint32_t tlane_e = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)UG_SP_ACC_COLS;
+    const uint32_t row_off = (uint32_t)(r >> 3) * (8 * KT) + (uint32_t)(r & 7) * KT;
+    const uint32_t key = KT == 128 ? (uint32_t)(r & 7) : (uint32_t)((r >> 1) & 3);
     int cnt = 0;
     constexpr int WIN = 16 / WPT;                      // stages per mask window
     const bool mask_tma = a.mask_tma != 0;
@@ -365,7 +336,6 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
       }
       const bool edge = (wbase + WPT) * 32 > a.cols;     // the stage reaches past the last column
       uint32_t y[CPT][4];
-      uint32_t meta[WPT];
 #pragma unroll
       for (int i = 0; i < WPT; ++i) {
         uint32_t v = w[i] ^ flip;
@@ -374,40 +344,17 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
           if (jb + 32 > a.cols) v = jb >= a.cols ? 0u : (v & ((1u << (a.cols - jb)) - 1u));
         }
         v = live ? v : 0u;
-        if constexpr (SP) {
-          // eight groups of four columns at once (one nibble each): positions of the first two selected columns ->
-          // metadata nibble idx0 | idx1 << 2, their values (0/1) -> two bytes per group = one 16-byte chunk per word
-          uint32_t v0, v1;
-          const uint32_t ovf = sparse_split(v, v0, v1, meta[i]);
-          cnt += __popc(v) - __popc(ovf);
-          // z: bits 4g / 4g+1 = value at idx0 / idx1 of group g; the bits 0, 1, 4, 5 of each byte of z go to bits 0, 8, 16,
-          // 24 of one word (x 0x81081 puts them there; the cross terms never carry into those positions)
-          const uint32_t z = v0 | (v1 << 1);
+        cnt += __popc(v);
+        // 4 mask bits -> 4 bytes: bit k of the nibble lands on bit 8k of (nibble * 0x00204081)
 #pragma unroll
-          for (int q = 0; q < 4; ++q) y[i][q] = (((z >> (8 * q)) & 0x33u) * 0x00081081u) & 0x01010101u;
-        } else {
-          cnt += __popc(v);
-          // 4 mask bits -> 4 bytes: bit k of the nibble lands on bit 8k of (nibble * 0x00204081)
-#pragma unroll
-          for (int q = 0; q < 8; ++q) y[2 * i + (q >> 2)][q & 3] = (((v >> (4 * q)) & 0xfu) * 0x00204081u) & 0x01010101u;
-        }
+        for (int q = 0; q < 8; ++q) y[2 * i + (q >> 2)][q & 3] = (((v >> (4 * q)) & 0xfu) * 0x00204081u) & 0x01010101u;
       }
       mbar_wait(EMPTY_BAR(s), ph ^ 1u);                // the expansion above is done while the stage is still busy
       const uint32_t abase = smem_base + (uint32_t)s * STAGE + row_off;
-      if constexpr (SP) {
-        static_assert(WPT == 4, "four metadata columns per stage");
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
-                     ::"r"(tlane_e + 4u * (uint32_t)s), "r"(meta[0]), "r"(meta[1]), "r"(meta[2]), "r"(meta[3]) : "memory");
-      }
-      if (!((a.dbg & 2) && it >= stages))
 #pragma unroll
-      for (int cc = 0; cc < (SP ? WPT : CPT); ++cc) {
+      for (int cc = 0; cc < CPT; ++cc) {
         const uint32_t addr = abase + ((((uint32_t)cc) ^ key) << 4);
         asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(y[cc][0]), "r"(y[cc][1]), "r"(y[cc][2]), "r"(y[cc][3]) : "memory");
-      }
-      if constexpr (SP) {
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-        tc_fence_before();
       }
       fence_proxy_async();
       __syncwarp();
@@ -495,29 +442,12 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
         mbar_wait(EMPTY_BAR(s), ph ^ 1u);
         const uint32_t bdst = smem_base + (uint32_t)s * STAGE + A_BYTES;
         const int x = (kt_begin + it) * KT;
-        if (PAIR) {
-          // this CTA's half of the digit rows of each accumulator; the bytes of both CTAs are expected by the leader
-          if ((a.dbg & 1) && it >= stages) { if (rank == 0) mbar_arrive(FULL_BAR(s)); continue; }     // timing experiments
-          if (rank == 0) mbar_expect_tx(FULL_BAR(s), 2u * (uint32_t)B_BYTES);
-          const int hh = n_half >> 1;
-          if (MC) {
-            // box `crank >> 1` (accumulator 0 / 1) of this position's half, delivered to this CTA and to the CTA at the
-            // same position of the other pair; completion bytes go to the pair leader's barrier of each destination
-            // (barrier given as this CTA's own address with the peer bit cleared)
-            const uint32_t which = crank >> 1;
-            tma_load_2d_pair_mc(bdst + which * (uint32_t)hh * KT, &tmap, x, ch * UG_CHUNK_ROWS + (int)which * n_half + (int)rank * hh,
-                                FULL_BAR(s) & 0xFEFFFFFFu, (uint16_t)((1u << crank) | (1u << (crank ^ 2u))));
-            continue;
-          }
-          const uint32_t lead_full = mapa_u32(FULL_BAR(s), lead);
-          tma_load_2d_pair(bdst, &tmap, x, ch * UG_CHUNK_ROWS + (int)rank * hh, lead_full);
-          tma_load_2d_pair(bdst + (uint32_t)hh * KT, &tmap, x, ch * UG_CHUNK_ROWS + n_half + (int)rank * hh, lead_full);
-          continue;
-        }
-        if ((a.dbg & 1) && it >= stages) { mbar_arrive(FULL_BAR(s)); continue; }
-        mbar_expect_tx(FULL_BAR(s), (uint32_t)B_BYTES);
-        tma_load_2d(bdst, &tmap, x, ch * UG_CHUNK_ROWS, FULL_BAR(s));
-        tma_load_2d(bdst + (uint32_t)n_half * KT, &tmap, x, ch * UG_CHUNK_ROWS + n_half, FULL_BAR(s));
+        // this CTA's half of the digit rows of each accumulator; the bytes of both CTAs are expected by the leader
+        if (rank == 0) mbar_expect_tx(FULL_BAR(s), 2u * (uint32_t)B_BYTES);
+        const int hh = n_half >> 1;
+        const uint32_t lead_full = mapa_u32(FULL_BAR(s), 0u);
+        tma_load_2d_pair(bdst, &tmap, x, ch * UG_CHUNK_ROWS + (int)rank * hh, lead_full);
+        tma_load_2d_pair(bdst + (uint32_t)hh * KT, &tmap, x, ch * UG_CHUNK_ROWS + n_half + (int)rank * hh, lead_full);
       }
     }
     __syncwarp();
@@ -537,7 +467,7 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
     __syncwarp();
   } else {
     // ================= MMA issuer =================
-    if (PAIR && lane == 0 && rank != 0) {
+    if (lane == 0 && rank != 0) {
       // partner CTA: relay "my A tile is complete" to the leader's full barrier, one cluster-scope arrive per stage
       // (a release at cluster scope flushes L1: kept off the expander threads)
       int s = -1;
@@ -546,22 +476,20 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
         if (++s == stages) s = 0;
         if (s == 0) ph ^= 1u;
         mbar_wait(FULL_BAR(s), ph);
-        mbar_arrive_remote(mapa_u32(FULL_BAR(s), lead));
+        mbar_arrive_remote(mapa_u32(FULL_BAR(s), 0u));
       }
     }
     if (rank == 0) {
       // instruction descriptor (cute::UMMA::InstrDescriptor): D = s32, A = B = u8, both K-major, N = n_half,
-      // M = 128 (256 for the CTA pair)
-      // M = 128 (256 for the CTA pair); bit 2: sparse
-      const uint32_t idesc = (SP ? 4u : 0u) | (2u << 4) | ((uint32_t)(n_half >> 3) << 17) |
-                             ((uint32_t)((PAIR ? 2 * UG_ROWS : UG_ROWS) >> 4) << 24);
+      // M = 256 (the CTA pair)
+      const uint32_t idesc = (2u << 4) | ((uint32_t)(n_half >> 3) << 17) | ((uint32_t)(2 * UG_ROWS >> 4) << 24);
       // The whole warp runs this loop (convergent code keeps descriptors in uniform registers: with a single-lane
       // loop every tcgen05.mma needed five R2UR moves, ~150 dependent instructions per stage, and the issuing thread
       // itself limited the tensor pipe); only the tcgen05 instructions are predicated on one elected lane.  No
       // divisions, no clock reads, descriptors by addition.
-      const uint64_t ad0 = umma_desc<AKT>(smem_base);
+      const uint64_t ad0 = umma_desc<KT>(smem_base);
       const uint64_t bd00 = umma_desc<KT>(smem_base + A_BYTES);
-      const uint64_t bd10 = umma_desc<KT>(smem_base + A_BYTES + (uint32_t)(PAIR ? n_half >> 1 : n_half) * KT);
+      const uint64_t bd10 = umma_desc<KT>(smem_base + A_BYTES + (uint32_t)(n_half >> 1) * KT);
       const uint64_t dstep = (uint64_t)(STAGE >> 4);
       const uint32_t tm1 = tmem_base + (uint32_t)n_half;
       int s = 0;
@@ -575,46 +503,28 @@ __global__ void __launch_bounds__(UG_THREADS, 1) k_gram_umma(const __grid_consta
         int sn = s + 1;
         uint32_t phn = ph;
         if (sn == stages) { sn = 0; phn ^= 1u; }
-        if (SP) {
-          // one MMA = 64 logical columns: 32 bytes of the compressed A row, 64 bytes of every digit row, two metadata columns
-          if (elect_one()) {
-            const uint32_t e0 = tmem_base + (uint32_t)UG_SP_ACC_COLS + 4u * (uint32_t)s;
-#pragma unroll
-            for (int kk = 0; kk < KT / 64; ++kk) {
-              const uint32_t acc = (it > 0 || kk > 0) ? 1u : 0u;
-              umma_i8_sp<PAIR>(tmem_base, ad + 2 * kk, bd0 + 4 * kk, e0 + 2u * kk, idesc, acc);
-              umma_i8_sp<PAIR>(tm1, ad + 2 * kk, bd1 + 4 * kk, e0 + 2u * kk, idesc, acc);
-            }
-            if (PAIR) umma_commit_pair(EMPTY_BAR(s), MC ? 0xFu : 3u); else umma_commit(EMPTY_BAR(s));
-          }
-        } else if (elect_one()) {
+        if (elect_one()) {
 #pragma unroll
           for (int kk = 0; kk < KT / 32; ++kk) {
             const uint32_t acc = (it > 0 || kk > 0) ? 1u : 0u;
-            if (PAIR) {
-              umma_i8_pair(tmem_base, ad + 2 * kk, bd0 + 2 * kk, idesc, acc);
-              umma_i8_pair(tm1, ad + 2 * kk, bd1 + 2 * kk, idesc, acc);
-            } else {
-              umma_i8(tmem_base, ad + 2 * kk, bd0 + 2 * kk, idesc, acc);
-              umma_i8(tm1, ad + 2 * kk, bd1 + 2 * kk, idesc, acc);
-            }
+            umma_i8_pair(tmem_base, ad + 2 * kk, bd0 + 2 * kk, idesc, acc);
+            umma_i8_pair(tm1, ad + 2 * kk, bd1 + 2 * kk, idesc, acc);
           }
-          if (PAIR) umma_commit_pair(EMPTY_BAR(s), MC ? 0xFu : 3u); else umma_commit(EMPTY_BAR(s));
+          umma_commit_pair(EMPTY_BAR(s));
         }
         __syncwarp();
         if (it + 1 < ntile) mbar_wait(FULL_BAR(sn), phn);
         s = sn; ph = phn;
         soff = s == 0 ? 0 : soff + dstep;
       }
-      if (elect_one()) { if (PAIR) umma_commit_pair(ACCUM_BAR, 3u << lead); else umma_commit(ACCUM_BAR); }
+      if (elect_one()) umma_commit_pair(ACCUM_BAR);
     }
     __syncwarp();
   }
-  if (PAIR) cluster_sync_all(); else __syncthreads();      // nobody frees tensor memory the partner still reads
+  cluster_sync_all();                                      // nobody frees tensor memory the partner still reads
   if (warp == UG_EXP_WARPS + 1) {
     tc_fence_after();
-    if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
   }
 #undef FULL_BAR
 #undef EMPTY_BAR
@@ -682,27 +592,21 @@ static long long plan_workspace_bytes(const UmmaPlan& pl, long long ld) {
 
 long long umma_workspace_bytes(int K, int vb, long long ld) {
   long long m = 0;
-  for (int sums = 0; sums < 2; ++sums)
-    for (int pair = 0; pair < 4; ++pair) {          // (the multicast bit does not change the plan)
-      const long long b = plan_workspace_bytes(make_umma_plan(K, vb, sums, pair & 1, pair >> 1), ld);
-      m = b > m ? b : m;
-    }
+  for (int sums = 0; sums < 2; ++sums) {
+    const long long b = plan_workspace_bytes(make_umma_plan(K, vb, sums), ld);
+    m = b > m ? b : m;
+  }
   return m;
 }
 
 int launch_stats_gram_umma(const uint32_t* bits, int rows, int ld, int cols, const double* Xp, const double* Vp, int K,
-                           int polarity, int nseg, int kt, int pair, int sums, int max_stages, double* Gout, double* SVout,
-                           void* workspace, long long workspace_bytes, cudaStream_t st) {
+                           int polarity, int nseg, int kt, int sums, double* Gout, double* SVout, void* workspace,
+                           long long workspace_bytes, cudaStream_t st) {
   if (rows <= 0 || ld <= 0 || ld % 64 || nseg <= 0 || cols <= 0 || cols > ld) { set_error("stats_gram_umma: bad shape"); return -2; }
   if (kt != 64 && kt != 128) { set_error("stats_gram_umma: tile width must be 64 or 128"); return -2; }
   if ((long long)ld * 255 >= 2147483647ll) { set_error("stats_gram_umma: more than 8.4M columns would overflow the int32 accumulators"); return -2; }
   const int vb = Vp != nullptr;
-  const int sp = (pair >> 1) & 1;               // bit 1 of `pair`: the 2:4-sparse form (128-column stages)
-  const int mc = (pair >> 2) & 1;               // bit 2: clusters of two pairs, digit tiles multicast between them
-  pair &= 1;
-  if (mc && !pair) { set_error("stats_gram_umma: the multicast form needs CTA pairs"); return -2; }
-  if (sp && kt != 128) { set_error("stats_gram_umma: the sparse form needs tile width 128"); return -2; }
-  const UmmaPlan pl = make_umma_plan(K, vb, sums, pair, sp);
+  const UmmaPlan pl = make_umma_plan(K, vb, sums);
   if (workspace_bytes < plan_workspace_bytes(pl, ld)) { set_error("stats_gram_umma: workspace too small"); return -2; }
   EncodeTiledFn encode = get_encode_fn();
   if (!encode) { set_error("stats_gram_umma: cuTensorMapEncodeTiled not available"); return -3; }
@@ -735,7 +639,7 @@ int launch_stats_gram_umma(const uint32_t* bits, int rows, int ld, int cols, con
     const int nh = which ? pl.nh_last : pl.nh_full;
     const cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)pl.nch * UG_CHUNK_ROWS};
     const cuuint64_t gstr[1] = {(cuuint64_t)ld};
-    const cuuint32_t box[2] = {(cuuint32_t)kt, (cuuint32_t)(pair ? nh / 2 : nh)};
+    const cuuint32_t box[2] = {(cuuint32_t)kt, (cuuint32_t)(nh / 2)};
     const cuuint32_t estr[2] = {1, 1};
     const CUresult r = encode(&tmaps[which], CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, Bd, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                               kt == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
@@ -754,22 +658,17 @@ int launch_stats_gram_umma(const uint32_t* bits, int rows, int ld, int cols, con
   size_t smem = 0;
   for (int which = 0; which < 2; ++which) {
     const int nh = which ? pl.nh_last : pl.nh_full;
-    const int stage_bytes = (sp ? UG_ROWS / 2 : UG_ROWS) * kt + (pair ? nh : 2 * nh) * kt;
+    const int stage_bytes = UG_ROWS * kt + nh * kt;
     int stages = (227 * 1024 - 1024 - tail) / stage_bytes;
     if (stages > 16) stages = 16;
-    if (sp && stages > 8) stages = 8;                  // four metadata columns per stage in tensor-memory columns [480, 512)
-    if (max_stages > 0 && stages > max_stages) stages = max_stages;
     if (stages < 2) { set_error("stats_gram_umma: stage does not fit"); return -2; }
     a.stages_of[which] = stages;
     const size_t need = (size_t)stages * stage_bytes + tail + 1024;
     smem = need > smem ? need : smem;
   }
-  { const char* e = getenv("BNMTF_UMMA_DBG"); a.dbg = e ? atoi(e) : 0; }
   // > half of the SM's shared memory: one CTA per SM, so the 512-column tensor-memory allocation never waits
   if (smem < 116 * 1024) smem = 116 * 1024;
-  int rbs = (rows + UG_ROWS - 1) / UG_ROWS;
-  if (pair) rbs = (rbs + 1) / 2 * 2;                   // a padding CTA (no live rows) completes the last pair
-  if (mc) rbs = (rbs + 3) / 4 * 4;
+  const int rbs = (rows + 2 * UG_ROWS - 1) / (2 * UG_ROWS) * 2;     // a padding CTA (no live rows) completes the last pair
   dim3 grid(rbs, pl.nch, nseg);
   // the mask bits as a (rows x ld/32) uint32 tensor: windows of 128 rows x 16 words; rows / words past the end read as zero
   CUtensorMap tmap_bits = tmaps[0];
@@ -786,16 +685,13 @@ int launch_stats_gram_umma(const uint32_t* bits, int rows, int ld, int cols, con
     if (r != CUDA_SUCCESS) { set_error("stats_gram_umma: cuTensorMapEncodeTiled (mask) failed (%d)", (int)r); return -3; }
   }
   void (*kern)(const CUtensorMap, const CUtensorMap, const CUtensorMap, UmmaGramArgs) =
-      mc ? (sp ? k_gram_umma<128, true, true, true> : (kt == 128 ? k_gram_umma<128, true, false, true> : k_gram_umma<64, true, false, true>))
-      : sp ? (pair ? k_gram_umma<128, true, true, false> : k_gram_umma<128, false, true, false>)
-         : kt == 128 ? (pair ? k_gram_umma<128, true, false, false> : k_gram_umma<128, false, false, false>)
-                     : (pair ? k_gram_umma<64, true, false, false> : k_gram_umma<64, false, false, false>);
+      kt == 128 ? k_gram_umma<128> : k_gram_umma<64>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = dim3(UG_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = mc ? 4 : (pair ? 2 : 1); attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   const cudaError_t le = cudaLaunchKernelEx(&cfg, kern, tmaps[0], tmaps[1], tmap_bits, a);
   if (le != cudaSuccess) { set_error("stats_gram_umma: launch failed: %s", cudaGetErrorString(le)); cudaGetLastError(); return -1; }

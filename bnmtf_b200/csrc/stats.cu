@@ -220,160 +220,6 @@ __global__ void __launch_bounds__(256) k_stats_gram(const uint32_t* __restrict__
 // ---------------------------------------------------------------------------------------------------
 // k_gram_full: unmasked totals over all n factor rows, as per-CTA partials (deterministic two-stage sum).
 // ---------------------------------------------------------------------------------------------------
-// ---------------------------------------------------------------------------------------------------
-// k_gram_fixup: the share of the per-row masked Gram that the 2:4-sparse tcgen05 kernel (gram_umma.cu) leaves out -- the
-// third and fourth selected column of every aligned group of four (sparse_split: 0.7 % of the entries when 20 % are
-// selected) -- summed in fp64 into ONE more segment of the partial statistics.  A warp per row: the row's overflow
-// columns are compacted into a queue (eight mask words per lane and one warp scan per batch), then the queued factor
-// rows are gathered four k-steps at a time and contracted with DMMA exactly as k_stats_gram does; the variance sums
-// (VB) are plain additions.  `cols` clips the last mask word as the tcgen05 kernel does.
-// ---------------------------------------------------------------------------------------------------
-constexpr int FIX_WARPS = 4;
-constexpr int FIX_QCAP = 1024;
-template <int NT, bool VB>
-__global__ void __launch_bounds__(32 * FIX_WARPS) k_gram_fixup(const uint32_t* __restrict__ bits, int rows, int ld, int cols,
-                                                               const double* __restrict__ Xp, const double* __restrict__ Vp,
-                                                               int polarity, double* __restrict__ Gout, double* __restrict__ SVout) {
-  constexpr int KP = 8 * NT;
-  constexpr int NTP = NT * (NT + 1) / 2;
-  __shared__ uint16_t queue[FIX_WARPS][FIX_QCAP + 16];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, e = lane & 3;
-  const int row = blockIdx.x * FIX_WARPS + warp;
-  if (row >= rows) return;  // whole warp leaves together; only __syncwarp below
-  const int wpr = ld >> 5;
-  const uint32_t* mrow = bits + (size_t)row * wpr;
-  const uint32_t flip = polarity ? 0u : 0xffffffffu;
-  uint16_t* q = queue[warp];
-
-  double acc[NTP][2];
-#pragma unroll
-  for (int p = 0; p < NTP; ++p) acc[p][0] = acc[p][1] = 0.0;
-  double sv[NT];
-#pragma unroll
-  for (int n = 0; n < NT; ++n) sv[n] = 0.0;
-
-  int qn = 0;               // queued columns
-  size_t qbase = 0;         // column the queued 16-bit offsets are relative to
-  auto drain = [&]() {
-    // pad to whole groups of four k-steps with the dummy (all-zero) factor row `ld`
-    if (lane < 16) q[qn + lane] = 0xFFFFu;
-    __syncwarp();
-    for (int i = 0; i < qn; i += 16) {
-      double x[4][NT], v[4][NT];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const uint32_t off = q[i + 4 * u + e];
-        const size_t j = (off == 0xFFFFu) ? (size_t)ld : qbase + off;
-        const double* xr = Xp + j * KP + g;
-#pragma unroll
-        for (int n = 0; n < NT; ++n) x[u][n] = xr[8 * n];
-        if (VB) {
-          const double* vr = Vp + j * KP + g;
-#pragma unroll
-          for (int n = 0; n < NT; ++n) v[u][n] = vr[8 * n];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-#pragma unroll
-        for (int a = 0; a < NT; ++a)
-#pragma unroll
-          for (int b = a; b < NT; ++b) {
-            const int p = a * NT - a * (a - 1) / 2 + (b - a);
-            dmma884(acc[p][0], acc[p][1], x[u][a], x[u][b]);
-          }
-        if (VB) {
-#pragma unroll
-          for (int n = 0; n < NT; ++n) sv[n] += v[u][n];
-        }
-      }
-    }
-    __syncwarp();
-    qn = 0;
-  };
-
-  for (int wb = 0; wb < wpr; wb += 256) {
-    if ((size_t)wb * 32 - qbase >= 32768) { drain(); qbase = (size_t)wb * 32; }      // 16-bit offsets
-    uint32_t ov[8];
-    int cnt = 0;
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      const int w = wb + c * 32 + lane;
-      uint32_t m = w < wpr ? (mrow[w] ^ flip) : 0u;
-      const int jb = w * 32;
-      if (jb + 32 > cols) m = jb >= cols ? 0u : (m & ((1u << (cols - jb)) - 1u));
-      uint32_t v0, v1, meta;
-      ov[c] = sparse_split(m, v0, v1, meta);
-      cnt += __popc(ov[c]);
-    }
-    int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int t = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += t;
-    }
-    const int total = __shfl_sync(0xffffffffu, incl, 31);
-    if (qn + total > FIX_QCAP) drain();
-    if (total <= FIX_QCAP) {
-      int pos = qn + incl - cnt;
-#pragma unroll
-      for (int c = 0; c < 8; ++c) {
-        uint32_t m = ov[c];
-        const int cb = (int)((size_t)(wb + c * 32 + lane) * 32 - qbase);
-        while (m) {
-          const int b = __ffs(m) - 1;
-          m &= m - 1;
-          q[pos++] = (uint16_t)(cb + b);
-        }
-      }
-      qn += total;
-      __syncwarp();
-    } else {
-      // a batch that does not fit the queue (a densely selected row): one group of 32 words at a time (<= 512 columns)
-#pragma unroll 1
-      for (int c = 0; c < 8; ++c) {
-        const int cc = __popc(ov[c]);
-        int inc2 = cc;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int t = __shfl_up_sync(0xffffffffu, inc2, o);
-          if (lane >= o) inc2 += t;
-        }
-        const int tot2 = __shfl_sync(0xffffffffu, inc2, 31);
-        if (qn + tot2 > FIX_QCAP) drain();
-        int pos = qn + inc2 - cc;
-        uint32_t m = ov[c];
-        const int cb = (int)((size_t)(wb + c * 32 + lane) * 32 - qbase);
-        while (m) {
-          const int b = __ffs(m) - 1;
-          m &= m - 1;
-          q[pos++] = (uint16_t)(cb + b);
-        }
-        qn += tot2;
-        __syncwarp();
-      }
-    }
-  }
-  drain();
-
-  double* go = Gout + (size_t)row * (NTP * 64);
-#pragma unroll
-  for (int p = 0; p < NTP; ++p)
-    *reinterpret_cast<double2*>(go + p * 64 + g * 8 + 2 * e) = make_double2(acc[p][0], acc[p][1]);
-  if (VB) {
-#pragma unroll
-    for (int n = 0; n < NT; ++n) {
-      sv[n] += __shfl_xor_sync(0xffffffffu, sv[n], 1);
-      sv[n] += __shfl_xor_sync(0xffffffffu, sv[n], 2);
-    }
-    if (e == 0) {
-      double* so = SVout + (size_t)row * KP;
-#pragma unroll
-      for (int n = 0; n < NT; ++n) so[8 * n + g] = sv[n];
-    }
-  }
-}
-
 template <int NT, bool VB>
 __global__ void __launch_bounds__(256) k_gram_full(const double* __restrict__ Xp, const double* __restrict__ Vp, int n,
                                                   int K, int dummy_row, double* __restrict__ partial) {
@@ -485,28 +331,6 @@ int launch_stats_gram(const uint32_t* bits, int rows, int ld, const double* Xp, 
     BNMTF_DISPATCH_NT(nt, (k_stats_gram<NT, false><<<grid, 256, 0, st>>>(bits, rows, ld, seg_words, Xp, nullptr, polarity, K, Gout, nullptr, run_flag)));
   }
   return check_launch("stats_gram");
-}
-
-// the overflow share of the 2:4-sparse tcgen05 Gram kernel: ONE segment (rows records) at Gout / SVout
-int launch_stats_gram_fixup(const uint32_t* bits, int rows, int ld, int cols, const double* Xp, const double* Vp, int K,
-                            int polarity, double* Gout, double* SVout, cudaStream_t st) {
-  if (rows <= 0 || ld <= 0 || ld % 64 || cols <= 0 || cols > ld) { set_error("stats_gram_fixup: bad shape"); return -2; }
-  const int nt = tiles_for(K);
-  if (nt > 4) { set_error("stats_gram_fixup: K=%d > 31", K); return -2; }
-  const int wpr = ld / 32;
-  (void)wpr;
-  dim3 grid((rows + FIX_WARPS - 1) / FIX_WARPS, 1);
-  switch (nt) {
-    case 1: if (Vp) k_gram_fixup<1, true><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, Vp, polarity, Gout, SVout);
-            else k_gram_fixup<1, false><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, nullptr, polarity, Gout, nullptr); break;
-    case 2: if (Vp) k_gram_fixup<2, true><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, Vp, polarity, Gout, SVout);
-            else k_gram_fixup<2, false><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, nullptr, polarity, Gout, nullptr); break;
-    case 3: if (Vp) k_gram_fixup<3, true><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, Vp, polarity, Gout, SVout);
-            else k_gram_fixup<3, false><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, nullptr, polarity, Gout, nullptr); break;
-    default: if (Vp) k_gram_fixup<4, true><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, Vp, polarity, Gout, SVout);
-             else k_gram_fixup<4, false><<<grid, 32 * FIX_WARPS, 0, st>>>(bits, rows, ld, cols, Xp, nullptr, polarity, Gout, nullptr); break;
-  }
-  return check_launch("stats_gram_fixup");
 }
 
 // out: NTP*64 Gram tiles followed by KP variance sums.  scratch: >= kGramFullParts * (NTP*64+KP) doubles.

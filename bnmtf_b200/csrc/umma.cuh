@@ -144,15 +144,6 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap
       ::"r"(dst), "l"(map), "r"(x), "r"(y), "r"(cluster_bar)
       : "memory");
 }
-// the same, delivered to every CTA of `cta_mask` (same shared-memory offset); `bar_off` is this CTA's own barrier address
-// with the peer bit cleared: in every destination the bytes are credited to the barrier of ITS pair leader
-__device__ __forceinline__ void tma_load_2d_pair_mc(uint32_t dst, const CUtensorMap* map, int x, int y, uint32_t bar_off,
-                                                    uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], [%4], %5;"
-      ::"r"(dst), "l"(map), "r"(x), "r"(y), "r"(bar_off), "h"(cta_mask)
-      : "memory");
-}
 __device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
@@ -162,32 +153,10 @@ __device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t adesc, ui
       : "memory");
 }
 // arrive on the barrier at this shared-memory offset in both CTAs of the pair when the MMAs issued so far are done
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint32_t cta_mask = 3u) {
-  const uint16_t mask = (uint16_t)cta_mask;
+__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask)
+               ::"r"(bar), "h"((uint16_t)3u)
                : "memory");
-}
-
-// 2:4-sparse form: A compressed in shared memory, its metadata at tensor-memory address `tmem_e` (idesc bit 2 set);
-// one instruction covers K = 64 logical columns
-template <bool PAIR>
-__device__ __forceinline__ void umma_i8_sp(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t tmem_e, uint32_t idesc,
-                                           uint32_t accum) {
-  if (PAIR)
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.sp.cta_group::2.kind::i8 [%0], %1, %2, [%3], %4, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accum)
-        : "memory");
-  else
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.sp.cta_group::1.kind::i8 [%0], %1, %2, [%3], %4, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accum)
-        : "memory");
 }
 
 // contiguous global -> shared bulk copy (TMA engine, no tensor map), completion on an mbarrier

@@ -350,11 +350,6 @@ class BNMFEngine:
         assert self.rx in ("umma", "dmma") and (self.rx == "dmma" or self.K <= 32)
         self.metrics_mode = os.environ.get("BNMTF_METRICS", "stats" if self.gram == "umma" else "direct")
         self.guard = 1e-5
-        # 0: the two statistics kernels of a phase run back to back; 1/2 (experimental): the tcgen05 Gram kernel runs on a
-        # high-priority second stream beside the R-streaming kernel.  Measured on B200: no gain (the two kernels do not
-        # become co-resident: different shared-memory carveouts; forcing the same carveout slows the streaming kernel)
-        self.overlap = int(os.environ.get("BNMTF_OVERLAP", "0")) if self.gram == "umma" else 0
-        self.umma_stages = int(os.environ.get("BNMTF_UMMA_STAGES", "3" if self.overlap else "0"))
         # 1: replay the sweep as a CUDA graph (0: launch by launch).  Sharded runs are captured too when the exchange runs
         # over peer memory with our own barrier / all-reduce kernels (csrc/peer.cu) -- with NCCL collectives inside the
         # capture (round 1's BNMTF_GRAPH=2) the process group did not shut down cleanly
@@ -368,12 +363,6 @@ class BNMFEngine:
         # (profiles/r06_split_sweep.txt, short runs): 64 still best at K = 20 (132.5 vs 131.8 / 131.8 / 130.1 at 56 / 72 /
         # 80: with fewer SMs the R.X kernel outlasts the Gram), K = 10, 24 and 32 within 0.3 % of the values tried
         self.split = int(os.environ.get("BNMTF_SPLIT", "64" if self.K > 16 else ("80" if self.K > 8 else "96")))
-        # Gram kernel form (bit 0: CTA pairs, cta_group::2; bit 1: 2:4-sparse MMAs + fp64 fix-up segment; bit 2: clusters of
-        # two pairs with multicast digit tiles).  Measured at the headline shape (DESIGN.md section 4): the sparse kernel
-        # alone takes 1.15 ms against 1.62 ms, but the fix-up of the 0.7 % of entries it leaves out gathers 3-6 GB of factor
-        # rows from L2 (0.45-0.8 ms) and one more segment slows the solver, so the sweep is faster with the dense form.
-        self.umma_pair = int(os.environ.get("BNMTF_UMMA_PAIR", "1"))
-        self._fix_stream = None
         self._side = None
         self.m = MODE[mode]
         self.vb = mode == "vb"
@@ -434,19 +423,13 @@ class BNMFEngine:
             else:
                 nrx = max(1, min(ld // 128, -(-2664 // rb)))
             if self.gram == "umma":
-                # CTAs = row blocks x column chunks x segments; aim for ~10 waves of one CTA per SM
+                # CTAs = row blocks (rounded up to whole CTA pairs) x column chunks x segments; aim for ~10 waves of one
+                # CTA per SM
                 tile = 128 if ld >= 256 else 64
                 sums = K if (side == 1 and self.metrics_mode == "stats") else 0
-                self.umma_form = getattr(self, "umma_form", {})
-                form = self.umma_pair
-                if tile != 128 or K > 31:
-                    form &= ~2                       # the sparse form needs 128-column stages (and its fix-up K <= 31)
-                self.umma_form[side] = form
-                acc_cols = 480 if form & 2 else 512
-                nch = -(-(K * (K + 1) // 2 + (K if self.vb else 0) + sums) // (acc_cols // _lib.call("bnmtf_fixed_point_digits")))
+                nch = -(-(K * (K + 1) // 2 + (K if self.vb else 0) + sums) // (512 // _lib.call("bnmtf_fixed_point_digits")))
                 ktiles = -(-ld // tile)
-                ng = _pick_nseg(((rb + 1) // 2 * 2 if form & 1 else rb) * nch, ktiles,
-                                t_tile=(0.3 if form & 2 else 0.55) * tile / 128, t_fix=10.0)
+                ng = _pick_nseg((rb + 1) // 2 * 2 * nch, ktiles, t_tile=0.55 * tile / 128, t_fix=10.0)
                 self.umma_tile = getattr(self, "umma_tile", {})
                 self.umma_tile[side] = tile
             else:
@@ -456,9 +439,7 @@ class BNMFEngine:
             self.nseg[side] = (nrx, ng, nm)
         rI, rJ = max(1, self.loc[0][1]), max(1, self.loc[1][1])
         mrx = max(self.nseg[0][0] * rI, self.nseg[1][0] * rJ)
-        # (+1: the fix-up segment of the sparse Gram form)
-        self.gram_segs = {side: self.nseg[side][1] + (1 if self.gram == "umma" and self.umma_form[side] & 2 else 0) for side in (0, 1)}
-        mg = max(self.gram_segs[0] * rI, self.gram_segs[1] * rJ)
+        mg = max(self.nseg[0][1] * rI, self.nseg[1][1] * rJ)
         f64 = lambda *shape: torch.zeros(shape, dtype=torch.float64, device=dev)
         self.RXpart = f64(mrx, KP)
         self.Gpart = f64(mg, GL)
@@ -527,11 +508,11 @@ class BNMFEngine:
         if not self.range_guard or rows == 0:
             return
         nrx, ng, _ = self.nseg[side]
-        _lib.call("bnmtf_range_guard_f64", _ptr(self.Gpart), self.gram_segs[side], rows, _ptr(self.Gfull), self.polarity, self.K, other.n,
+        _lib.call("bnmtf_range_guard_f64", _ptr(self.Gpart), ng, rows, _ptr(self.Gfull), self.polarity, self.K, other.n,
                   self.ws_ptr, _ptr(self.range_flag), _ptr(self.range_trips), _stream())
         _lib.call("bnmtf_stats_gated_f64", _ptr(self.range_flag), _ptr(R), _ptr(bits), rows, ld, _ptr(other.Xp), _ptr(other.Vp),
-                  self.K, self.polarity, nrx, self.gram_segs[side], _ptr(self.RXpart) if need_rx else 0, _ptr(self.Gpart),
-                  _ptr(self.SVpart), _stream())       # (every segment the solver adds up is rewritten, the fix-up one included)
+                  self.K, self.polarity, nrx, ng, _ptr(self.RXpart) if need_rx else 0, _ptr(self.Gpart),
+                  _ptr(self.SVpart), _stream())
 
     def _stats_kernels(self, side, need_rx=True, sums=False, timers=None):
         """Layer-1 passes for one phase: statistics of this rank's rows of R (side 0) / R^T (side 1) w.r.t. the
@@ -546,7 +527,6 @@ class BNMFEngine:
         if self.polarity == 0:
             _lib.call("bnmtf_gram_full_f64", _ptr(other.Xp), _ptr(other.Vp), other.n, self.K, ld,
                       _ptr(self.Gfull), _ptr(self.gscratch), _stream())
-        rx = lambda: self._rx(side)
         if need_rx and self.split > 0 and self.rx == "umma" and self.gram == "umma":
             # SM split: the persistent, HBM-bound R.X kernel takes `split` SMs (high-priority stream, launched first),
             # the tensor-bound Gram kernel the rest; neither could share an SM's tensor memory with the other
@@ -572,26 +552,9 @@ class BNMFEngine:
                 timers.append(("stats_rx_in_sweep", tev[0], tev[1]))
                 timers.append(("stats_gram_in_sweep", tev[2], tev[3]))
             main.wait_event(self._ev[1])
-        elif need_rx and self.overlap:
-            # the Gram kernel goes to a high-priority stream: its one-per-SM, long-lived CTAs are placed as soon as
-            # a CTA of the streaming kernel retires, and the two then share every SM (tensor pipe | fp64 pipe + HBM)
-            if self._side is None:
-                self._side = torch.cuda.Stream(device=self.ds.device, priority=-1)
-                self._ev = [torch.cuda.Event(), torch.cuda.Event()]
-            main = torch.cuda.current_stream()
-            self._ev[0].record(main)
-            self._side.wait_event(self._ev[0])
-            if self.overlap == 2:
-                rx()
-            with torch.cuda.stream(self._side):
-                self._gram(side, sums)
-                self._ev[1].record(self._side)
-            if self.overlap != 2:
-                rx()
-            main.wait_event(self._ev[1])
         else:
             if need_rx:
-                rx()
+                self._rx(side)
             self._gram(side, sums)
 
     def _rx(self, side, max_ctas=0):
@@ -609,27 +572,9 @@ class BNMFEngine:
         me, other, R, bits, rows, ld, lo = self._sides(side)
         ng = self.nseg[side][1]
         if self.gram == "umma":
-            form = self.umma_form[side]
-            if form & 2:
-                # what the 2:4-sparse MMAs leave out (0.7 % of the entries at 20 % missing): summed in fp64 on a stream of
-                # its own beside the two tensor-core kernels, into one more segment of the partial statistics
-                if self._fix_stream is None:
-                    self._fix_stream = torch.cuda.Stream(device=self.ds.device)
-                    self._fix_ev = [torch.cuda.Event(), torch.cuda.Event()]
-                main = torch.cuda.current_stream()
-                self._fix_ev[0].record(main)
-                self._fix_stream.wait_event(self._fix_ev[0])
-                with torch.cuda.stream(self._fix_stream):
-                    _lib.call("bnmtf_stats_gram_fixup_f64", _ptr(bits), rows, ld, other.n, _ptr(other.Xp), _ptr(other.Vp), self.K,
-                              self.polarity, self.Gpart.data_ptr() + 8 * ng * rows * self.Gpart.shape[1],
-                              self.SVpart.data_ptr() + 8 * ng * rows * self.SVpart.shape[1] if self.vb else 0, _stream())
-                    self._fix_ev[1].record(self._fix_stream)
             _lib.call("bnmtf_stats_gram_umma_f64", _ptr(bits), rows, ld, other.n, _ptr(other.Xp), _ptr(other.Vp), self.K,
-                      self.polarity, ng, self.umma_tile[side], form, 1 if sums else 0, self.umma_stages,
-                      _ptr(self.Gpart),
-                      _ptr(self.SVpart), self.ws_ptr, self.ws_bytes, _stream())
-            if form & 2:
-                torch.cuda.current_stream().wait_event(self._fix_ev[1])
+                      self.polarity, ng, self.umma_tile[side], 1 if sums else 0, _ptr(self.Gpart), _ptr(self.SVpart),
+                      self.ws_ptr, self.ws_bytes, _stream())
         else:
             _lib.call("bnmtf_stats_gram_f64", _ptr(bits), rows, ld, _ptr(other.Xp), _ptr(other.Vp), self.K,
                       self.polarity, ng, _ptr(self.Gpart), _ptr(self.SVpart), _stream())
@@ -649,7 +594,7 @@ class BNMFEngine:
                                      device=self.ds.device)
         fused = gather and apply and me.peer is not None     # the kernel stores the finished rows into the peers' copies
         if rows > 0:
-            _lib.call("bnmf_row_solve_f64", self.m, rows, self.K, nrx, self.gram_segs[side] if self.gram == "umma" else ng, self.polarity,
+            _lib.call("bnmf_row_solve_f64", self.m, rows, self.K, nrx, ng, self.polarity,
                       _ptr(self.RXpart), _ptr(self.Gpart), _ptr(self.SVpart), _ptr(self.Gfull),
                       _ptr(me.fac, lo), _ptr(me.var, lo), _ptr(me.mu, lo), _ptr(me.tauf, lo), _ptr(me.lam, lo),
                       _ptr(self.scalars), order_ptr, n_order, 1 if apply else 0, float(minimum_TN),
@@ -1014,7 +959,7 @@ class SparseBNMFEngine(BNMFEngine):
         self.guard = 1e-5
         self.polarity = 1
         self.range_guard = False
-        self.split = self.overlap = 0
+        self.split = 0
         self.use_graph = int(os.environ.get("BNMTF_GRAPH", "1")) >= 1
         self._graph = self._graph_key = self._graph_seen = None
         self._small_c = 0               # never the single-kernel small path

@@ -112,19 +112,16 @@ int bnmtf_stats_gram_f64(const uint32_t* bits, int64_t rows, int64_t ld, const d
  * the products X_ja X_jb (and Var_jk) are cut into bnmtf_fixed_point_digits() exact 8-bit digits (6: a 48-bit
  * fixed-point value per column, by default) and multiplied with the 0/1 selection matrix of the rows, so the result is
  * the exactly summed, once-rounded value of the quantised products.  cols = number of valid columns (<= ld); tile = 64 or 128 (bytes of the column range staged
- * per pipeline stage); pair: bit 0 runs CTA pairs (cta_group::2: adjacent 128-row blocks share every MMA and each
- * CTA stages only half of the digit rows), bit 1 selects the 2:4-SPARSE form (tcgen05.mma.sp, tile 128 only): of every
- * aligned group of four columns only the first two selected ones are summed, and the caller adds the rest with
- * bnmtf_stats_gram_fixup_f64 as one more segment, bit 2 runs clusters of two pairs that multicast the digit tiles; sums != 0 also accumulates the masked column sums of X (slot (k, K) of the packed tiles,
- * as the ones-column of Xp does in bnmtf_stats_gram_f64; the selected-entry count always goes to slot (K, K));
- * max_stages > 0 caps the pipeline depth (shared memory left for kernels running concurrently on other streams);
+ * per pipeline stage).  The kernel runs as CTA pairs (cta_group::2: adjacent 128-row blocks share every MMA and each
+ * CTA stages only half of the digit rows).  sums != 0 also accumulates the masked column sums of X (slot (k, K) of the
+ * packed tiles, as the ones-column of Xp does in bnmtf_stats_gram_f64; the selected-entry count always goes to slot (K, K));
  * workspace: >= bnmtf_gram_umma_workspace_bytes(K, Vp != NULL, ld) bytes, 1024-byte aligned.
  * Only the entries (a, b < K), the slots above, and the first K entries of SVpart are written. */
 int64_t bnmtf_gram_umma_workspace_bytes(int K, int vb, int64_t ld);
 int bnmtf_stats_gram_umma_f64(const uint32_t* bits, int64_t rows, int64_t ld, int64_t cols, const double* Xp,
-                              const double* Vp /*or NULL*/, int K, int polarity, int nseg, int tile, int pair, int sums,
-                              int max_stages, double* Gpart, double* SVpart /*or NULL*/, void* workspace,
-                              int64_t workspace_bytes, void* stream);
+                              const double* Vp /*or NULL*/, int K, int polarity, int nseg, int tile, int sums,
+                              double* Gpart, double* SVpart /*or NULL*/, void* workspace, int64_t workspace_bytes,
+                              void* stream);
 /* Single-kernel sweeps for small two-factor problems (K <= 16, a few hundred rows and columns: the reference's toy and
  * GDSC matrices).  One thread-block cluster runs `sweeps` whole iterations of bnmf_gibbs_optimised.run /
  * bnmf_vb_optimised.run / nmf_icm.run (bnmf_gibbs_optimised.py:121-157, bnmf_vb_optimised.py:121-153, nmf_icm.py:114-149)
@@ -174,12 +171,6 @@ int bnmtf_csr_kmeans_distances_f64(const int64_t* rowptr, const int32_t* colidx,
  * `only` alone (only its rows of sums / counts are written).  2 <= d, 1 <= K <= 64. */
 int bnmtf_csr_kmeans_sums_f64(const int64_t* coordptr, const int32_t* point, const double* val, int64_t d,
                               const int32_t* assign, int K, int only, double* sums, double* counts, void* stream);
-/* The share the 2:4-sparse form leaves out (third and fourth selected column of every aligned group of four: 0.7 % of
- * the entries at 20 % missing), summed in fp64 (mma.sync.m8n8k4.f64 on gathered factor rows) into ONE segment: Gseg /
- * SVseg point at `rows` records laid out like a segment of Gpart / SVpart; pass nseg + 1 segments to the solver.  K <= 31. */
-int bnmtf_stats_gram_fixup_f64(const uint32_t* bits, int64_t rows, int64_t ld, int64_t cols, const double* Xp,
-                               const double* Vp /*or NULL*/, int K, int polarity, double* Gseg, double* SVseg /*or NULL*/,
-                               void* stream);
 /* Dynamic-range guard of the two tcgen05 statistics kernels, run after them on the same stream.  Both use one scale
  * per factor column, so a row whose observed set only meets entries far below a column's maximum gets statistics with
  * few significant bits.  flag <- 1 (and *trips += 1, if given) when for some row i and column k

@@ -111,7 +111,7 @@ def test_engine_picked_the_headline_variants(dataset):
     m = bnmf.bnmf_vb_optimised.from_dataset(dataset, K, PRI, seed=1)
     eng = m._engine()
     assert eng.gram == "umma" and eng.rx == "umma" and eng.metrics_mode == "stats" and eng.split == 64 and eng.use_graph
-    assert eng.umma_pair == 1 and eng.umma_tile == {0: 128, 1: 128}
+    assert eng.umma_tile == {0: 128, 1: 128}
     assert eng.nseg[1][0] >= 2 and eng.nseg[1][1] >= 2, eng.nseg          # column phase: several column segments
     assert dataset.partI.cnt() >= 24576                                    # row phase: thread-per-row solver
 

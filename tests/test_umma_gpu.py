@@ -44,7 +44,7 @@ def _tile_index(a, b, KP):
     return (ta * nt - ta * (ta - 1) // 2 + (tb - ta)) * 64 + (a % 8) * 8 + (b % 8)
 
 
-def _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums, stages=0, pair=0):
+def _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums):
     import torch
     from bnmtf_b200 import _lib
     from bnmtf_b200.engine import _ptr, _stream, gram_len
@@ -52,34 +52,33 @@ def _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums, stages=0, pair=
     wsb = _lib.call("bnmtf_gram_umma_workspace_bytes", K, vb, d["ld"])
     ws = torch.zeros(wsb + 1024, dtype=torch.uint8, device=d["dev"])
     wsp = (ws.data_ptr() + 1023) // 1024 * 1024
-    sparse = (pair >> 1) & 1         # 2:4-sparse form: the fix-up kernel adds what it leaves out as one more segment
-    nsg = nseg + sparse
-    G = torch.zeros((nsg * rows, GL), dtype=torch.float64, device=d["dev"])
-    S = torch.zeros((nsg * rows, d["KP"]), dtype=torch.float64, device=d["dev"]) if vb else None
+    G = torch.zeros((nseg * rows, GL), dtype=torch.float64, device=d["dev"])
+    S = torch.zeros((nseg * rows, d["KP"]), dtype=torch.float64, device=d["dev"]) if vb else None
     _lib.call("bnmtf_stats_gram_umma_f64", _ptr(d["bits"]), rows, d["ld"], cols, _ptr(d["Xp"]), _ptr(d["Vp"]) if vb else 0,
-              K, polarity, nseg, tile, pair, sums, stages, _ptr(G), _ptr(S), wsp, wsb, _stream())
-    if sparse:
-        _lib.call("bnmtf_stats_gram_fixup_f64", _ptr(d["bits"]), rows, d["ld"], cols, _ptr(d["Xp"]), _ptr(d["Vp"]) if vb else 0,
-                  K, polarity, G.data_ptr() + 8 * nseg * rows * GL, S.data_ptr() + 8 * nseg * rows * d["KP"] if vb else 0,
-                  _stream())
+              K, polarity, nseg, tile, sums, _ptr(G), _ptr(S), wsp, wsb, _stream())
     torch.cuda.synchronize()
-    G = G.view(nsg, rows, GL).sum(0).cpu().numpy()
-    S = S.view(nsg, rows, d["KP"]).sum(0).cpu().numpy() if vb else None
+    G = G.view(nseg, rows, GL).sum(0).cpu().numpy()
+    S = S.view(nseg, rows, d["KP"]).sum(0).cpu().numpy() if vb else None
     return G, S
 
 
-@pytest.mark.parametrize("pair", [0, 1])
 @pytest.mark.parametrize("rows,cols,K,vb,polarity,nseg,tile,sums", [
     (100, 80, 10, 0, 0, 1, 128, 0),      # config-1 shape
     (100, 80, 5, 1, 0, 1, 64, 1),        # config-2 shape, VB, with the column sums
     (129, 65, 5, 1, 1, 1, 64, 1),        # ragged rows/cols, observed-set polarity
+    (129, 65, 5, 1, 1, 1, 128, 1),
     (622, 138, 10, 1, 0, 1, 64, 1),      # GDSC shape (odd number of row blocks: a padding CTA completes the last pair)
+    (622, 138, 10, 1, 0, 1, 128, 1),
     (300, 1000, 20, 1, 0, 2, 64, 1),     # two column segments, four chunks
+    (300, 1000, 20, 1, 0, 2, 128, 1),    # VB column phase at K = 20
     (260, 700, 33, 0, 0, 3, 128, 0),     # K > 32: eight chunks
+    (700, 4100, 20, 0, 0, 3, 128, 0),    # 33 column tiles in three segments: the pipeline stages wrap around
+    (300, 4096, 12, 1, 0, 5, 64, 1),     # mask windows through TMA; odd segments start half a window in
+    (390, 2176, 12, 1, 1, 2, 128, 1),    # mask windows through TMA, observed-set polarity
 ])
-def test_gram_umma_matches_numpy(rows, cols, K, vb, polarity, nseg, tile, sums, pair):
+def test_gram_umma_matches_numpy(rows, cols, K, vb, polarity, nseg, tile, sums):
     d = _setup(rows, cols, K, seed=rows + cols + K)
-    G, S = _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums, pair=pair)
+    G, S = _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums)
     W = d["M"] if polarity else 1.0 - d["M"]
     X, KP = d["X"], d["KP"]
     for a in range(K):
@@ -99,55 +98,16 @@ def test_gram_umma_matches_numpy(rows, cols, K, vb, polarity, nseg, tile, sums, 
         np.testing.assert_allclose(S[:, :K], ref, rtol=1e-13, atol=1e-13 * np.abs(ref).max())
 
 
-@pytest.mark.parametrize("form", [3, 5, 7, 2])
-@pytest.mark.parametrize("rows,cols,K,vb,polarity,nseg,sums", [
-    (100, 80, 10, 0, 0, 1, 0),
-    (129, 65, 5, 1, 1, 1, 1),           # observed-set polarity: 80 % selected, most groups of four overflow
-    (622, 138, 10, 1, 0, 1, 1),
-    (300, 1000, 20, 1, 0, 2, 1),        # VB column phase at K = 20: four chunks in the sparse form
-    (700, 4100, 20, 0, 0, 3, 0),        # 33 stages: the mask windows and the metadata slots wrap around
-])
-def test_gram_umma_sparse_and_multicast_forms(rows, cols, K, vb, polarity, nseg, sums, form):
-    """`pair` bit 1: tcgen05.mma.sp on the 2:4 part + fp64 fix-up of the overflow columns; bit 2: clusters of two CTA pairs
-    with multicast digit tiles.  Same statistics as the dense form (bnmf_gibbs_optimised.py:167-177)."""
-    d = _setup(rows, cols, K, seed=rows + cols + K + form)
-    G, S = _gram_umma(d, rows, cols, K, vb, polarity, nseg, 128, sums, pair=form)
-    W = d["M"] if polarity else 1.0 - d["M"]
-    X, KP = d["X"], d["KP"]
-    for a in range(K):
-        for b in range(a, K):
-            ref = W @ (X[:, a] * X[:, b])
-            np.testing.assert_allclose(G[:, _tile_index(a, b, KP)], ref, rtol=1e-13, atol=1e-13 * np.abs(ref).max())
-    assert np.array_equal(G[:, _tile_index(K, K, KP)], W.sum(1))
-    if sums:
-        for k in range(K):
-            ref = W @ X[:, k]
-            np.testing.assert_allclose(G[:, _tile_index(k, K, KP)], ref, rtol=1e-13, atol=1e-13 * np.abs(ref).max())
-    if vb:
-        ref = W @ d["Var"]
-        np.testing.assert_allclose(S[:, :K], ref, rtol=1e-13, atol=1e-13 * np.abs(ref).max())
-
-
 def test_gram_umma_forms_agree_bit_for_bit(monkeypatch):
-    """Exact accumulation: the dense forms (single CTA, pairs, multicast clusters; mask words through TMA windows or loaded
-    directly) give identical bits on any data; on integer data the sparse form + fix-up does too."""
-    rows, cols, K = 390, 2100, 12        # ld = 2112 is not a multiple of 128: direct mask loads; 2176 columns would use TMA
+    """Exact accumulation: mask words through TMA windows or loaded directly give identical bits on any data."""
+    rows, cols, K = 390, 2100, 12        # ld = 2112 is not a multiple of 128: direct mask loads; 2176 columns use TMA
     for cols_ in (cols, 2176):
         d = _setup(rows, cols_, K, seed=77)
-        ref, _ = _gram_umma(d, rows, cols_, K, 1, 0, 2, 128, 1, pair=0)
-        for form in (1, 5):
-            G, _ = _gram_umma(d, rows, cols_, K, 1, 0, 2, 128, 1, pair=form)
-            assert np.array_equal(G, ref), (cols_, form)
+        ref, _ = _gram_umma(d, rows, cols_, K, 1, 0, 2, 128, 1)
         monkeypatch.setenv("BNMTF_GRAM_MASK_TMA", "0")
-        G, _ = _gram_umma(d, rows, cols_, K, 1, 0, 2, 128, 1, pair=1)
+        G, _ = _gram_umma(d, rows, cols_, K, 1, 0, 2, 128, 1)
         monkeypatch.delenv("BNMTF_GRAM_MASK_TMA")
         assert np.array_equal(G, ref), cols_
-    d = _setup(rows, 2176, K, seed=78, integer=True)
-    ref, Sref = _gram_umma(d, rows, 2176, K, 1, 0, 1, 128, 1, pair=1)
-    for form in (3, 7):
-        G, S = _gram_umma(d, rows, 2176, K, 1, 0, 1, 128, 1, pair=form)
-        idx = [_tile_index(a, b, d["KP"]) for a in range(K) for b in range(a, K)] + [_tile_index(k, K, d["KP"]) for k in range(K + 1)]
-        assert np.array_equal(G[:, idx], ref[:, idx]) and np.array_equal(S[:, :K], Sref[:, :K]), form
 
 
 def test_gram_umma_is_exact_on_integers():
@@ -155,8 +115,8 @@ def test_gram_umma_is_exact_on_integers():
     rows, cols, K = 200, 900, 12
     d = _setup(rows, cols, K, seed=5, integer=True)
     W = 1.0 - d["M"]
-    for nseg, tile, pair in ((1, 64, 0), (3, 128, 0), (2, 128, 1)):
-        G, S = _gram_umma(d, rows, cols, K, 1, 0, nseg, tile, 1, pair=pair)
+    for nseg, tile in ((1, 64), (3, 128), (2, 128)):
+        G, S = _gram_umma(d, rows, cols, K, 1, 0, nseg, tile, 1)
         for a in range(K):
             for b in range(a, K):
                 assert np.array_equal(G[:, _tile_index(a, b, d["KP"])], W @ (d["X"][:, a] * d["X"][:, b]))
@@ -244,7 +204,7 @@ def test_fixed_point_statistics_error_model():
     ld_ = np.longdouble
     W = 1.0 - d["M"]
     X = d["X"]
-    G, _ = _gram_umma(d, rows, cols, K, 0, 0, 1, 128, 0, pair=1)
+    G, _ = _gram_umma(d, rows, cols, K, 0, 0, 1, 128, 0)
     worst = 0.0
     for a, b in ((0, 0), (0, 1), (3, 17), (19, 19), (7, 12)):
         p = X[:, a] * X[:, b]

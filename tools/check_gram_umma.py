@@ -12,38 +12,30 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PAIR = int(os.environ.get("PAIR", "0"))
 sys.path.insert(0, ROOT)
 
-# rows, cols, K, vb, polarity, nseg, tile, signed, timing reps, sums, max_stages
+# rows, cols, K, vb, polarity, nseg, tile, signed, timing reps, sums
 CASES = [
-    (100, 80, 10, 0, 0, 1, 128, 0, 0, 0, 0),
-    (100, 80, 10, 0, 0, 1, 64, 0, 0, 1, 0),
-    (129, 65, 5, 1, 0, 1, 64, 0, 0, 1, 2),
-    (129, 65, 5, 1, 1, 1, 128, 0, 0, 0, 0),
-    (300, 1000, 20, 1, 0, 2, 64, 0, 0, 1, 3),
-    (300, 1000, 20, 0, 0, 3, 128, 1, 0, 1, 0),
-    (1000, 5000, 20, 1, 0, 1, 64, 1, 0, 0, 0),
-    (700, 3000, 33, 1, 0, 2, 128, 0, 0, 1, 0),
-    (65536, 32768, 20, 0, 0, 1, 128, 0, 3, 0, 0),
-    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0, 4),
-    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0, 3),
-    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0, 2),
-    (65536, 32768, 20, 0, 0, 1, 128, 0, 3, 0, 1),
-    (32768, 65536, 20, 0, 0, 2, 128, 0, 3, 1, 0),
-    (32768, 65536, 20, 1, 0, 2, 128, 0, 3, 1, 0),
-    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0, 0),     # 15: tile 64, as many stages as fit
-    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0, 6),
-    (65536, 32768, 20, 0, 0, 1, 128, 0, 3, 0, 3),
-    (65536, 32768, 20, 0, 0, 1, 128, 0, 3, 0, 2),
-    (65536, 32768, 20, 1, 0, 1, 128, 0, 3, 0, 0),    # 19: VB row phase
-    (8192, 32768, 20, 0, 0, 3, 128, 0, 3, 0, 0),     # 20: one rank of 8, row phase (Gibbs)
-    (4096, 65536, 20, 1, 0, 3, 128, 0, 3, 1, 0),     # 21: one rank of 8, column phase (VB, with the column sums)
-    (80, 100, 10, 1, 0, 1, 64, 0, 0, 1, 0),          # 22: the toy matrix's column phase (VB): two 64-column stages, eight slots
-    (80, 100, 10, 1, 0, 1, 64, 0, 0, 0, 0),
-    (80, 100, 10, 0, 0, 1, 64, 0, 0, 0, 0),
-    (80, 100, 10, 1, 0, 2, 64, 0, 0, 0, 0),          # 25: one stage per segment
-    (100, 80, 10, 1, 0, 2, 64, 0, 0, 1, 0),
+    (100, 80, 10, 0, 0, 1, 128, 0, 0, 0),
+    (100, 80, 10, 0, 0, 1, 64, 0, 0, 1),
+    (129, 65, 5, 1, 0, 1, 64, 0, 0, 1),
+    (129, 65, 5, 1, 1, 1, 128, 0, 0, 0),
+    (300, 1000, 20, 1, 0, 2, 64, 0, 0, 1),
+    (300, 1000, 20, 0, 0, 3, 128, 1, 0, 1),
+    (1000, 5000, 20, 1, 0, 1, 64, 1, 0, 0),
+    (700, 3000, 33, 1, 0, 2, 128, 0, 0, 1),
+    (65536, 32768, 20, 0, 0, 1, 128, 0, 3, 0),
+    (32768, 65536, 20, 0, 0, 2, 128, 0, 3, 1),
+    (32768, 65536, 20, 1, 0, 2, 128, 0, 3, 1),
+    (65536, 32768, 20, 0, 0, 1, 64, 0, 3, 0),        # 11: tile 64
+    (65536, 32768, 20, 1, 0, 1, 128, 0, 3, 0),       # 12: VB row phase
+    (8192, 32768, 20, 0, 0, 3, 128, 0, 3, 0),        # 13: one rank of 8, row phase (Gibbs)
+    (4096, 65536, 20, 1, 0, 3, 128, 0, 3, 1),        # 14: one rank of 8, column phase (VB, with the column sums)
+    (80, 100, 10, 1, 0, 1, 64, 0, 0, 1),             # 15: the toy matrix's column phase (VB): two 64-column stages, eight slots
+    (80, 100, 10, 1, 0, 1, 64, 0, 0, 0),
+    (80, 100, 10, 0, 0, 1, 64, 0, 0, 0),
+    (80, 100, 10, 1, 0, 2, 64, 0, 0, 0),             # 18: one stage per segment
+    (100, 80, 10, 1, 0, 2, 64, 0, 0, 1),
 ]
 
 
@@ -52,10 +44,7 @@ def run_case(idx):
     import torch
     from bnmtf_b200 import _lib
     from bnmtf_b200.engine import _ptr, _stream, ld_for, kp_for, gram_len
-    rows, cols, K, vb, pol, nseg, tile, signed, reps, sums, stages = CASES[idx]
-    sparse = (PAIR >> 1) & 1          # PAIR=2|3: the 2:4-sparse form (128-column stages only)
-    if sparse:
-        tile = 128
+    rows, cols, K, vb, pol, nseg, tile, signed, reps, sums = CASES[idx]
     if reps:
         reps = int(os.environ.get("REPS", reps))
     dev = torch.device("cuda:0")
@@ -86,36 +75,23 @@ def run_case(idx):
     wsb = _lib.call("bnmtf_gram_umma_workspace_bytes", K, vb, ld)
     ws = torch.zeros(wsb + 1024, dtype=torch.uint8, device=dev)
     wsp = (ws.data_ptr() + 1023) // 1024 * 1024
-    fixup = sparse and int(os.environ.get("FIXUP", "0"))
-    nsg = nseg + (1 if fixup else 0)
-    G1 = torch.full((nsg * rows, GL), float("nan"), dtype=torch.float64, device=dev)
-    S1 = torch.full((nsg * rows, KP), float("nan"), dtype=torch.float64, device=dev) if vb else None
+    G1 = torch.full((nseg * rows, GL), float("nan"), dtype=torch.float64, device=dev)
+    S1 = torch.full((nseg * rows, KP), float("nan"), dtype=torch.float64, device=dev) if vb else None
 
     def umma():
         _lib.call("bnmtf_stats_gram_umma_f64", _ptr(bits), rows, ld, cols, _ptr(Xp), _ptr(Vp) if vb else 0, K, pol, nseg,
-                  tile, PAIR, sums, stages, _ptr(G1), _ptr(S1), wsp, wsb, _stream())
-        if fixup:
-            _lib.call("bnmtf_stats_gram_fixup_f64", _ptr(bits), rows, ld, cols, _ptr(Xp), _ptr(Vp) if vb else 0, K, pol,
-                      G1.data_ptr() + 8 * nseg * rows * GL, S1.data_ptr() + 8 * nseg * rows * KP if vb else 0, _stream())
+                  tile, sums, _ptr(G1), _ptr(S1), wsp, wsb, _stream())
     umma()
     torch.cuda.synchronize()
     out = {"case": idx, "shape": [rows, cols, K], "vb": vb, "pol": pol, "nseg": nseg, "tile": tile, "signed": signed,
-           "sums": sums, "stages": stages}
+           "sums": sums}
     # reference on the first chunk of rows: W @ P in fp64
     nr = min(rows, chunk)
     W = M0[:nr] if pol == 1 else 1.0 - M0[:nr]
-    if sparse and not int(os.environ.get("FIXUP", "0")):
-        # the kernel alone keeps the first two selected columns of every aligned group of four
-        c4 = (cols + 3) // 4 * 4
-        Wp = torch.zeros((nr, c4), dtype=torch.float64, device=dev)
-        Wp[:, :cols] = W
-        g4 = Wp.view(nr, c4 // 4, 4)
-        W = (g4 * (g4.cumsum(2) <= 2)).reshape(nr, c4)[:, :cols].contiguous()
-        out["overflow_frac"] = float(1.0 - W.sum() / Wp.sum())
     ia, ib = np.triu_indices(K)
     P = X[:, ia] * X[:, ib]
     Gref = W @ P                                   # nr x ng
-    Gu = G1.view(nsg, rows, GL).nan_to_num(0.0).sum(0)[:nr]
+    Gu = G1.view(nseg, rows, GL).nan_to_num(0.0).sum(0)[:nr]
     NT = KP // 8
 
     def tile_index(a, b):
@@ -137,7 +113,7 @@ def run_case(idx):
     out["count_err"] = float((Gu[:, tile_index(K, K)] - W.sum(1)).abs().max())
     if vb:
         Sref = W @ Var
-        Su = S1.view(nsg, rows, KP).sum(0)[:nr, :K]
+        Su = S1.view(nseg, rows, KP).sum(0)[:nr, :K]
         out["sv_vs_ref"] = float(((Su - Sref).abs() / Sref.abs().max(0).values.clamp_min(1e-300)).max())
     if int(os.environ.get("STRESS", "0")):
         # exact integer accumulation: every call must give the same bits; report where repeated calls differ
