@@ -624,7 +624,11 @@ int launch_stats_gram_umma(const uint32_t* bits, int rows, int ld, int cols, con
     const size_t sm = (size_t)(vb ? 2 : 1) * K * 65 * sizeof(double);
     int nbm = (cols + 63) / 64;
     if (nbm > 296) nbm = 296;
+    // VB from K = 48 on stages more than the default 48 KB: without the opt-in the launch fails, the column maxima stay
+    // zero and every product above 1 saturates at the scale of a zero maximum
+    if (sm > 48 * 1024) cudaFuncSetAttribute(k_ug_colmax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     k_ug_colmax<<<nbm, 256, sm, st>>>(Xp, Vp, cols, KP, pl, colmax);
+    if (check_launch("stats_gram_umma column maxima")) return -1;
     k_ug_scales<<<(pl.nc + 127) / 128, 128, 0, st>>>(colmax, pl.nc, cscale, cexp);
     const size_t sq = (size_t)(vb ? 2 : 1) * K * 130 * sizeof(double) + (size_t)pl.nc * 4;
     if (sq > 48 * 1024) cudaFuncSetAttribute(k_ug_quantize, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sq);

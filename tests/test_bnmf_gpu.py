@@ -1,7 +1,14 @@
 """GPU parity of the two-factor models against the golden fixtures (generated from the reference itself) and
 against the CPU oracle on the same seeded inputs.  Everything here goes through the ctypes C ABI."""
+import os
+import re
+import sys
+
 import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from test_row_solve_gpu import auto_form, in_fresh_process, solver_kernel_pattern  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -229,49 +236,113 @@ def test_tn_moments_in_the_tail_follow_scipys_erfc():
 
 
 # ---- the row solvers: sub-warp (W lanes per row, the default below 24576 rows), thread per row (from 24576 rows on),
-# ---- warp per row (explicit orders) -- csrc/solve.cu::launch_row_solve; BNMTF_SOLVE forces one of them
+# ---- warp per row (explicit orders) -- csrc/solve.cu::launch_row_solve; BNMTF_SOLVE forces one of them.  These shapes
+# ---- would otherwise run as one single-kernel sweep (csrc/small.cu), which has no row solver: BNMTF_SMALL=0
 SOLVERS = ["warp", "lane", "sub4", "sub8", "sub16", "sub32"]
+
+
+GIBBS_SHAPES = [((300, 170), 7), ((2500, 96), 20), ((130, 2300), 31), ((37, 45), 3)]
+
+
+def gibbs_problem(shape, K):
+    rng = np.random.RandomState(5)
+    I, J = shape
+    R = rng.exponential(1.0, (I, K)) @ rng.exponential(1.0, (J, K)).T + rng.normal(size=(I, J))
+    M = (rng.rand(I, J) >= 0.25).astype(float)
+    return R, M, {"alpha": 1.0, "beta": 1.0, "lambdaU": 0.1, "lambdaV": 0.1}
+
+
+def icm_from_golden(models, g):
+    m = models.nmf_icm(g["R"], g["M"], int(g["K"]), priors2(g))
+    m.initialise("exp")
+    m.U, m.V = g["init_U"].copy(), g["init_V"].copy()
+    m.tau = (m.alpha_s() - 1.0) / m.beta_s()
+    return m
+
+
+_MODEL_PROBE = """
+import numpy as np
+import bnmtf_b200 as models
+from test_bnmf_gpu import GIBBS_SHAPES, SOLVERS, gibbs_problem, icm_from_golden, vb_from_golden
+golden = lambda name: dict(np.load(os.path.join(%r, name + ".npz")))
+os.environ["BNMTF_SMALL"] = "0"
+out = {}
+
+
+def first_sweep(m):
+    names = launched_kernels(lambda: m.run(1))
+    assert m._engine().small_cluster() == 0
+    return names
+for solver in SOLVERS + [""]:
+    os.environ["BNMTF_SOLVE"] = solver
+    if solver:
+        for name in ("toy_bnmf_vb", "gdsc_bnmf_vb"):
+            out["vb %%s %%s" %% (name, solver)] = first_sweep(vb_from_golden(models, golden(name)))
+        out["icm " + solver] = first_sweep(icm_from_golden(models, golden("toy_nmf_icm")))
+    for shape, K in GIBBS_SHAPES:
+        R, M, pri = gibbs_problem(shape, K)
+        m = models.bnmf_gibbs_optimised(R, M, K, pri, seed=3)
+        m.initialise("exp")
+        out["gibbs %%s %%s" %% (shape, solver)] = first_sweep(m)
+print(json.dumps(out))
+"""
+
+
+@pytest.fixture(scope="module")
+def sweep_kernels():
+    """Kernels of the first sweep (launched eagerly, not from a CUDA graph) of every forced-solver run below, with
+    BNMTF_SMALL=0, listed by the profiler in a fresh interpreter (test_row_solve_gpu.in_fresh_process)."""
+    return in_fresh_process(_MODEL_PROBE % os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+
+
+def assert_solver_ran(names, solver, K, rows=()):
+    """The per-phase sweep ran (no single-kernel sweep) and `solver` (empty: the launcher's choice for each phase's row
+    count) is among the kernels launched."""
+    assert not any("k_small" in n for n in names), sorted(set(names))
+    for form in ([solver] if solver else [auto_form(r, K) for r in rows]):
+        assert any(re.search(solver_kernel_pattern(form, K), n) for n in names), (form, sorted(set(names)))
 
 
 @pytest.mark.parametrize("solver", SOLVERS)
 @pytest.mark.parametrize("name", ["toy_bnmf_vb", "gdsc_bnmf_vb"])
-def test_every_solver_follows_the_golden_vb_trajectory(models, golden, name, solver, monkeypatch):
+def test_every_solver_follows_the_golden_vb_trajectory(models, golden, name, solver, monkeypatch, sweep_kernels):
     """The golden VB trajectories with each row-solver kernel forced, 1e-9 as above."""
     monkeypatch.setenv("BNMTF_SOLVE", solver)
+    monkeypatch.setenv("BNMTF_SMALL", "0")
     g = golden(name)
     m = vb_from_golden(models, g)
     m.run(int(g["its"]))
+    assert m._engine().small_cluster() == 0
     close(m.all_performances["MSE"], g["trace_MSE"], what="MSE trace")
     close(m.all_exp_tau, g["trace_exptau"], what="exptau trace")
     ok = np.isfinite(g["trace_elbo"])
     close(np.asarray(m.all_elbo)[ok], g["trace_elbo"][ok], what="ELBO trace")
     for k in ("expU", "varU", "muU", "tauU", "expV", "varV", "muV", "tauV"):
         close(getattr(m, k), g["final_" + k], what=k)
+    assert_solver_ran(sweep_kernels["vb %s %s" % (name, solver)], solver, int(g["K"]))
 
 
 @pytest.mark.parametrize("solver", SOLVERS)
-def test_every_solver_follows_the_golden_icm_trajectory(models, golden, solver, monkeypatch):
+def test_every_solver_follows_the_golden_icm_trajectory(models, golden, solver, monkeypatch, sweep_kernels):
     monkeypatch.setenv("BNMTF_SOLVE", solver)
+    monkeypatch.setenv("BNMTF_SMALL", "0")
     g = golden("toy_nmf_icm")
-    m = models.nmf_icm(g["R"], g["M"], int(g["K"]), priors2(g))
-    m.initialise("exp")
-    m.U, m.V = g["init_U"].copy(), g["init_V"].copy()
-    m.tau = (m.alpha_s() - 1.0) / m.beta_s()
+    m = icm_from_golden(models, g)
     m.run(int(g["its"]), minimum_TN=float(g["minimum_TN"]))
+    assert m._engine().small_cluster() == 0
     close(m.all_performances["MSE"], g["trace_MSE"]), close(m.all_tau, g["trace_tau"])
     close(m.U, g["final_U"]), close(m.V, g["final_V"])
+    assert_solver_ran(sweep_kernels["icm " + solver], solver, int(g["K"]))
 
 
-@pytest.mark.parametrize("shape,K", [((300, 170), 7), ((2500, 96), 20), ((130, 2300), 31), ((37, 45), 3)])
-def test_all_solvers_draw_the_same_gibbs_chain(models, shape, K, monkeypatch):
+@pytest.mark.parametrize("shape,K", GIBBS_SHAPES)
+def test_all_solvers_draw_the_same_gibbs_chain(models, shape, K, monkeypatch, sweep_kernels):
     """Same Philox counters, same statistics: the solvers differ only in the summation order of the K-term dot
     products, so a short Gibbs chain agrees to ~1e-10 between any two of them (a draw that lands on a branch boundary
-    of the sampler would show up as an O(1) difference).  Ragged row counts exercise the partial last warp."""
-    rng = np.random.RandomState(5)
-    I, J = shape
-    R = rng.exponential(1.0, (I, K)) @ rng.exponential(1.0, (J, K)).T + rng.normal(size=(I, J))
-    M = (rng.rand(I, J) >= 0.25).astype(float)
-    pri = {"alpha": 1.0, "beta": 1.0, "lambdaU": 0.1, "lambdaV": 0.1}
+    of the sampler would show up as an O(1) difference).  Ragged row counts exercise the partial last warp.  The
+    profiler confirms the kernel each run used."""
+    monkeypatch.setenv("BNMTF_SMALL", "0")
+    R, M, pri = gibbs_problem(shape, K)
     out = {}
     for solver in SOLVERS + [""]:
         if solver:
@@ -281,6 +352,8 @@ def test_all_solvers_draw_the_same_gibbs_chain(models, shape, K, monkeypatch):
         m = models.bnmf_gibbs_optimised(R, M, K, pri, seed=3)
         m.initialise("exp")
         m.run(4)
+        assert m._engine().small_cluster() == 0
+        assert_solver_ran(sweep_kernels["gibbs %s %s" % (shape, solver)], solver, K, rows=shape)
         out[solver] = (m.U.copy(), m.V.copy(), m.tau, list(m.all_performances["MSE"]))
     for solver in SOLVERS[1:] + [""]:
         for a, b in zip(out[solver], out["warp"]):
@@ -303,21 +376,31 @@ def test_uploaded_dataset_is_shared_between_models(models, golden):
     assert len(c.all_performances["MSE"]) == 3 and a._engine().ds is c._engine().ds
 
 
-@pytest.mark.parametrize("I,J,K,frac", [(23, 17, 4, 0.3), (40, 155, 7, 0.6), (513, 64, 20, 0.2), (64, 1030, 31, 0.45)])
+@pytest.mark.parametrize("I,J,K,frac", [(23, 17, 4, 0.3), (40, 155, 7, 0.6), (513, 64, 20, 0.2), (64, 1030, 31, 0.45),
+                                         (200, 700, 32, 0.3), (230, 650, 33, 0.6), (180, 600, 48, 0.4), (160, 560, 63, 0.55)])
 def test_vb_and_icm_against_the_oracle_on_fresh_inputs(models, I, J, K, frac):
     """Shapes, ranks and missing fractions the golden fixtures do not contain (ragged tiles, K = 31, 60 % missing, so
     both polarities of the Gram kernel): 8 VB sweeps and 8 ICM sweeps from a seeded random start against the CPU oracle
-    (itself checked against the live reference on such inputs by tests/test_oracle_vs_reference.py), 1e-9."""
+    (itself checked against the live reference on such inputs by tests/test_oracle_vs_reference.py), 1e-9.
+    K = 32 ... 63 is the dense production path above the sub-warp solvers: tcgen05 Gram statistics over several column
+    segments, the tcgen05 R.X kernel at 32 and the fp64 one above, the warp-per-row solver at 5 to 8 tiles with its
+    metric sums (mstat) feeding the training metrics, and predict() on a held-out mask through the masked-metrics
+    kernel with more than 8 k-steps."""
     from oracle import bnmtf_oracle as orc
     rng = np.random.RandomState(I + J)
     R = np.abs(rng.exponential(1.0, (I, K)) @ rng.exponential(1.0, (J, K)).T + rng.normal(size=(I, J)) + 3.0)
     M = (rng.rand(I, J) >= frac).astype(float)
     M[np.arange(I), rng.randint(0, J, I)] = 1.0
     M[rng.randint(0, I, J), np.arange(J)] = 1.0
+    M_test = (rng.rand(I, J) < 0.3).astype(float)
     pri = {"alpha": 2.0, "beta": 0.5, "lambdaU": 0.3, "lambdaV": 0.7}
     np.random.seed(4)
     m = models.bnmf_vb_optimised(R, M, K, pri)
     m.initialise("random")
+    eng = m._engine()
+    if K >= 32:
+        assert eng.gram == "umma" and eng.rx == ("umma" if K == 32 else "dmma") and eng.metrics_mode == "stats"
+        assert eng.nseg[0][0] > 1 and eng.nseg[0][1] > 1 and eng.small_cluster() == 0
     o = orc.OracleBNMF(R, M, K, pri, mode="vb")
     o.init_vb(m.muU.copy(), m.muV.copy())
     close(m.expU, o.U), close(m.exptau, o.exptau)
@@ -328,10 +411,26 @@ def test_vb_and_icm_against_the_oracle_on_fresh_inputs(models, I, J, K, frac):
     # factors: 1e-9, except the 64 x 1030 case, whose VB iteration doubles a perturbation every sweep: 3e-11 after one
     # sweep, 2e-8 after eight -- the same figures with the fp64 mma.sync statistics (BNMTF_GRAM=dmma BNMTF_RX=dmma) as
     # with the tcgen05 fixed-point ones and with either solver (measured in round 1: BNMTF_GRAM=dmma BNMTF_RX=dmma give the same 2e-8), i.e. the conditioning of that
-    # problem, not a property of a kernel.  Checked at 1e-7 there; its traces above still hold 1e-9
-    ftol = 1e-7 if min(I, J) < 100 and max(I, J) > 1000 else 1e-9
+    # problem, not a property of a kernel.  Checked at 1e-7 there; its traces above still hold 1e-9.  The K >= 32 cases
+    # grow faster still: in the oracle alone a 1e-14 relative change of the start moves the factors by 1e-11 .. 5e-11
+    # after one sweep and by 2e-10 .. 1e-7 after eight, so their factors are checked at 1e-9 after one sweep (below) and
+    # at 1e-6 after eight
+    ftol = 1e-7 if min(I, J) < 100 and max(I, J) > 1000 else (1e-6 if K >= 32 else 1e-9)
     close(m.expU, o.U, rtol=ftol, what="expU"), close(m.expV, o.V, rtol=ftol, what="expV")
     close(m.varU, o.varU, rtol=ftol, what="varU")
+    check_predict(m.predict(M_test), o, M_test, "predict")
+    if K >= 32:
+        np.random.seed(4)
+        m1 = models.bnmf_vb_optimised(R, M, K, pri)
+        m1.initialise("random")
+        o1 = orc.OracleBNMF(R, M, K, pri, mode="vb")
+        o1.init_vb(m1.muU.copy(), m1.muV.copy())
+        o1.sweep()
+        m1.run(1)
+        # (not the variances: the reference's TN variance amplifies the last bits of mu by up to 1e-13 x^4 in the tail,
+        # see bench.py's parity note)
+        close(m1.expU, o1.U, what="expU, one sweep"), close(m1.expV, o1.V, what="expV, one sweep")
+        close(m1.muV, o1.muV, what="muV, one sweep"), close(m1.tauV, o1.tauV, what="tauV, one sweep")
     np.random.seed(5)
     c = models.nmf_icm(R, M, K, pri)
     c.initialise("random")
@@ -341,3 +440,17 @@ def test_vb_and_icm_against_the_oracle_on_fresh_inputs(models, I, J, K, frac):
         oc.sweep(minimum_TN=0.05)
     c.run(8, minimum_TN=0.05)
     close(c.U, oc.U, what="ICM U"), close(c.V, oc.V, what="ICM V"), close(c.tau, oc.tau)
+    close(c.quality("BIC"), oc.quality("BIC"))
+    check_predict(c.predict(M_test), oc, M_test, "ICM predict")
+
+
+def check_predict(got, o, M_test, what):
+    """predict() on a held-out mask against the oracle: MSE and R^2 at 1e-9; Rp = cov / (sd_r sd_p) at 1e-9 times
+    max|p| / sd_p, its sensitivity to a relative change of the predictions (ICM can leave every factor entry at
+    minimum_TN: a constant prediction, sd_p ~ 1e-18, Rp rounding noise)."""
+    ref = o.predict(M_test)
+    P = (o.U @ o.V.T)[M_test > 0]
+    close(got["MSE"], ref["MSE"], what=what + " MSE"), close(got["R^2"], ref["R^2"], what=what + " R^2")
+    cond = float(np.abs(P).max() / max(P.std(), 1e-300))
+    if cond < 1e6:                                   # (else Rp is 0 / 0 up to rounding, NaN or +-inf on either side)
+        np.testing.assert_allclose(got["Rp"], ref["Rp"], rtol=RTOL, atol=RTOL * max(1.0, cond), err_msg=what + " Rp")

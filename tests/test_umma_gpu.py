@@ -1,8 +1,13 @@
 """tcgen05 statistics kernels (csrc/gram_umma.cu, csrc/rx_umma.cu) against numpy restatements of the sums they replace
 (the masked row sums of bnmf_gibbs_optimised.py:167-177 / bnmf_vb_optimised.py:189-195), against the fp64 mma.sync
 kernels, and -- through the model classes -- against each other over whole trajectories.  All through the C ABI."""
+import os
+import sys
+
 import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 pytestmark = pytest.mark.gpu
 
@@ -75,6 +80,10 @@ def _gram_umma(d, rows, cols, K, vb, polarity, nseg, tile, sums):
     (700, 4100, 20, 0, 0, 3, 128, 0),    # 33 column tiles in three segments: the pipeline stages wrap around
     (300, 4096, 12, 1, 0, 5, 64, 1),     # mask windows through TMA; odd segments start half a window in
     (390, 2176, 12, 1, 1, 2, 128, 1),    # mask windows through TMA, observed-set polarity
+    (260, 700, 48, 1, 0, 3, 128, 1),     # K = 48, 63: the widest packed tiles (7 and 8 per side), VB, both polarities
+    (200, 520, 48, 1, 1, 2, 64, 1),
+    (200, 520, 63, 1, 0, 2, 128, 1),
+    (150, 700, 63, 1, 1, 3, 128, 1),
 ])
 def test_gram_umma_matches_numpy(rows, cols, K, vb, polarity, nseg, tile, sums):
     d = _setup(rows, cols, K, seed=rows + cols + K)
@@ -233,26 +242,58 @@ def test_fixed_point_statistics_error_model():
     assert float(np.max(err / scale)) < (1e-14 if T == 47 else 1e-15)
 
 
-@pytest.mark.parametrize("mode", ["vb", "icm"])
-def test_engine_paths_agree_over_a_trajectory(mode, monkeypatch):
-    """tcgen05 statistics + statistics-based metrics vs fp64 mma.sync statistics + direct metrics: same trajectory."""
-    import bnmtf_b200
+PATHS = (("umma", {"BNMTF_GRAM": "umma", "BNMTF_RX": "umma", "BNMTF_METRICS": "stats"}),
+         ("dmma", {"BNMTF_GRAM": "dmma", "BNMTF_RX": "dmma", "BNMTF_METRICS": "direct"}))
+
+
+def trajectory_problem():
     rng = np.random.RandomState(3)
     I, J, K = 300, 220, 6
     R = rng.exponential(1.0, (I, K)) @ rng.exponential(1.0, (J, K)).T + rng.normal(size=(I, J))
     M = (rng.rand(I, J) < 0.8).astype(float)
-    pri = {"alpha": 1.0, "beta": 1.0, "lambdaU": 0.1, "lambdaV": 0.1}
+    return R, M, K, {"alpha": 1.0, "beta": 1.0, "lambdaU": 0.1, "lambdaV": 0.1}
+
+
+_PATH_PROBE = """
+import bnmtf_b200
+from test_umma_gpu import PATHS, trajectory_problem
+os.environ["BNMTF_SMALL"] = "0"
+out = {}
+for mode in ("vb", "icm"):
+    for name, env in PATHS:
+        os.environ.update(env)
+        R, M, K, pri = trajectory_problem()
+        m = (bnmtf_b200.bnmf_vb_optimised if mode == "vb" else bnmtf_b200.nmf_icm)(R, M, K, pri)
+        m.initialise("exp")
+        out[mode + " " + name] = launched_kernels(lambda: m.run(1))
+print(json.dumps(out))
+"""
+
+
+@pytest.mark.parametrize("mode", ["vb", "icm"])
+def test_engine_paths_agree_over_a_trajectory(mode, monkeypatch):
+    """tcgen05 statistics + statistics-based metrics vs fp64 mma.sync statistics + direct metrics: same trajectory.
+    BNMTF_SMALL=0: at this size the whole run would otherwise be one single-kernel sweep, which uses neither; the
+    profiler (in a fresh interpreter) confirms which Gram kernel the first sweep of each path launches."""
+    import bnmtf_b200
+    from test_row_solve_gpu import in_fresh_process
+    monkeypatch.setenv("BNMTF_SMALL", "0")
+    R, M, K, pri = trajectory_problem()
     runs = {}
-    for name, env in (("umma", {"BNMTF_GRAM": "umma", "BNMTF_RX": "umma", "BNMTF_METRICS": "stats"}),
-                      ("dmma", {"BNMTF_GRAM": "dmma", "BNMTF_RX": "dmma", "BNMTF_METRICS": "direct"})):
+    kernels = in_fresh_process(_PATH_PROBE)
+    for name, env in PATHS:
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         cls = bnmtf_b200.bnmf_vb_optimised if mode == "vb" else bnmtf_b200.nmf_icm
         m = cls(R, M, K, pri)
         m.initialise("exp")
         m.run(15)
-        assert m._engine().gram == name
+        assert m._engine().gram == name and m._engine().small_cluster() == 0
         runs[name] = m
+        names = kernels[mode + " " + name]
+        assert not any("k_small" in n for n in names)
+        assert any("k_gram_umma" in n for n in names) == (name == "umma")
+        assert any("k_stats_gram" in n for n in names)     # dmma: the statistics; umma: the range guard's gated pass
     a, b = runs["umma"], runs["dmma"]
     Ua, Ub = (a.expU, b.expU) if mode == "vb" else (a.U, b.U)
     np.testing.assert_allclose(Ua, Ub, rtol=1e-9, atol=1e-11)
@@ -262,8 +303,10 @@ def test_engine_paths_agree_over_a_trajectory(mode, monkeypatch):
 
 def test_metrics_guard_switches_to_the_direct_pass(monkeypatch):
     """A (numerically) exact fit: sum e^2 = sum r^2 - 2 sum rp + sum p^2 cancels completely, the device flag routes the
-    sweep to the direct pass, and the MSE stays accurate."""
+    sweep to the direct pass, and the MSE stays accurate.  BNMTF_SMALL=0: the single-kernel sweep this size would
+    otherwise get has no such guard."""
     import bnmtf_b200
+    monkeypatch.setenv("BNMTF_SMALL", "0")
     rng = np.random.RandomState(4)
     I, J, K = 120, 90, 3
     U0, V0 = rng.exponential(1.0, (I, K)) + 0.5, rng.exponential(1.0, (J, K)) + 0.5
@@ -277,6 +320,10 @@ def test_metrics_guard_switches_to_the_direct_pass(monkeypatch):
         m.initialise("exp")
         m.U, m.V, m.tau = U0.copy(), V0.copy(), 1.0
         m.run(3)
+        eng = m._engine()
+        assert eng.small_cluster() == 0 and eng.metrics_mode == name
+        if name == "stats":
+            assert int(eng.flag.item()) == 1              # the guard tripped: the direct pass replaced the sums
         out[name] = np.array(m.all_performances["MSE"])
     assert out["direct"][-1] < 1e-12
     np.testing.assert_allclose(out["stats"], out["direct"], rtol=1e-6, atol=1e-20)
